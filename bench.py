@@ -23,6 +23,12 @@ configuration the north-star HBM-roofline target is stated on.
 `roofline`: dominant kernel of the step (largest total device time in a profiled pass of the same step):
             algorithmic bytes of its launches / their CUDA-event duration, against MEASURED_PEAKS.json.
 `cpu_baseline`: the oracle (a single-threaded port of the reference path) timed on a bounded sample.
+
+--dump-outputs DIR writes what the timed `value` path returned in the last pass of its last step, so that two builds can
+be compared output for output (the inputs depend only on the arguments):
+  DIR/counts_rank<r>.npy   float64 (frames, 2): sequence index of every frame of rank r, points the chain returned for it
+  DIR/frame<f>.npy         float32 (points, 7): x, y, z, r, g, b, tile of the chain's result for frame f, for a fixed
+                           seeded sample of DUMP_FRAMES frames (rows subsampled with a seed if the files would exceed 64 MB)
 """
 from __future__ import annotations
 
@@ -41,6 +47,7 @@ os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "32")
 
 REPO = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, REPO)
+sys.dont_write_bytecode = True   # the tree may be read-only: the bench writes nothing into it
 
 POINTS_PER_FRAME = int(os.environ.get("BENCH_POINTS", 1000 * 1000))   # BENCH_POINTS: diagnostic only (host-bound or GPU-bound?)
 VOXEL = 0.01
@@ -50,6 +57,8 @@ PASSES = 8                   # passes over the sequence per step
 WORKERS = 30                 # host threads (one CUDA stream each) feeding one GPU; divides the rank's share of the 240 frames at 1, 2 and 4 GPUs
                              # (scripts/ab_value.py on one B200, 16 host cores: 15 threads 8.2-8.5, 24 threads 8.3-8.6, 32 threads 8.6-8.7 Gpoints/s)
 HBM_FALLBACK_GBS = 6650.0    # B200_PROFILING.md fallback when MEASURED_PEAKS.json is absent
+DUMP_FRAMES = 32             # --dump-outputs: frames written in full (of the rank's share of the sequence)
+DUMP_BYTES = 64 << 20        # --dump-outputs: at most this much in all
 
 
 def log(*a):
@@ -141,6 +150,8 @@ class Worker(threading.Thread):
         self.out_points = 0
         self.mid_points = 0
         self.d2h_bytes = 0
+        self.last_counts = {}     # frame -> points returned in the last pass (--dump-outputs)
+        self.kept = {}            # frame -> result cloud of the last pass, for the frames state["keep"] names
 
     def frame_chain(self, pc):
         stage = os.environ.get("BENCH_STAGE", "")   # diagnostic only: time one stage of the chain
@@ -174,10 +185,18 @@ class Worker(threading.Thread):
                 lib.cwipc_cuda_timer_start(timer)
                 # K steps back to back: a worker starts its share of step s+1 as soon as it has finished its share of
                 # step s (frames are independent), the timed region is bracketed once, around all K steps
-                for f in [f for _ in range(st["nsteps"] * st["passes"]) for f in mine]:
+                order = [f for _ in range(st["nsteps"] * st["passes"]) for f in mine]
+                last_pass = len(order) - len(mine) if mode == "resident" and st["keep"] is not None else len(order)
+                for i, f in enumerate(order):
                     if mode == "resident":
                         o = self.frame_chain(st["device_frames"][f])
-                        self.out_points += o.count()
+                        m = o.count()
+                        self.out_points += m
+                        if i >= last_pass:
+                            self.last_counts[f] = m
+                            if f in st["keep"]:
+                                self.kept[f] = o     # read back after the timed region
+                                continue
                         o.free()
                     else:  # e2e: pinned host -> device -> filters -> pinned host
                         err = ctypes.c_char_p()
@@ -225,6 +244,26 @@ def run_steps(workers, barrier, state, lib, mode, nsteps, passes=None):
             lib.cwipc_cuda_timer_destroy(t)
         w.timers = []
     return ms
+
+
+def dump_outputs(out_dir, workers, rank, world):
+    """--dump-outputs (see the module docstring): frame j of this rank is frame rank + j * world of the sequence."""
+    counts = {j: m for w in workers for j, m in w.last_counts.items()}
+    kept = {j: o for w in workers for j, o in w.kept.items()}
+    for w in workers:
+        w.kept = {}
+    np.save(os.path.join(out_dir, f"counts_rank{rank}.npy"),
+            np.array([(rank + j * world, counts[j]) for j in sorted(counts)], np.float64).reshape(-1, 2))
+    # 7 float32 per point; every rank's files together stay within DUMP_BYTES (headers and the counts included)
+    max_rows = (DUMP_BYTES // world - 16 * len(counts) - 4096 * (len(kept) + 1)) // (7 * 4 * max(1, len(kept)))
+    for j in sorted(kept):
+        f = rank + j * world
+        pts = kept[j].get_numpy_array()
+        kept[j].free()
+        if len(pts) > max_rows:
+            pts = pts[np.sort(np.random.default_rng(f).choice(len(pts), max_rows, replace=False))]
+        cols = np.stack([pts[c].astype(np.float32) for c in ("x", "y", "z", "r", "g", "b", "tile")], axis=1)
+        np.save(os.path.join(out_dir, f"frame{f:03d}.npy"), cols)
 
 
 def dist_setup(args):
@@ -492,7 +531,8 @@ def run_ours(args):
         state_mid = []
     nworkers = args.workers
     host_out = [lib.cwipc_cuda_host_alloc(POINTS_PER_FRAME * 16) for _ in range(nworkers)]
-    state = {"frames": frames, "device_frames": device_frames, "host_ptrs": host_ptrs, "host_out": host_out, "cellsize": cellsize, "stop": False, "mode": "resident", "mid_frames": state_mid}
+    state = {"frames": frames, "device_frames": device_frames, "host_ptrs": host_ptrs, "host_out": host_out, "cellsize": cellsize, "stop": False, "mode": "resident", "mid_frames": state_mid,
+             "keep": None}
     barrier = threading.Barrier(nworkers + 1)
     workers = [Worker(w, nworkers, dev, cw, lib, barrier, state) for w in range(nworkers)]
     for w in workers:
@@ -507,12 +547,15 @@ def run_ours(args):
     cw.cuda_synchronize()
     dist_barrier(dist, torch)
 
+    if args.dump_outputs:
+        state["keep"] = set(np.random.default_rng(0).choice(nframes, min(DUMP_FRAMES, nframes), replace=False).tolist())
     sampler.armed.set()
     launches0 = cw.cuda_kernel_launches()
     resident_ms = run_steps(workers, barrier, state, lib, "resident", args.steps)
     launches = cw.cuda_kernel_launches() - launches0
     out_points = sum(w.out_points for w in workers) // args.steps      # per step
     mid_points = sum(w.mid_points for w in workers) // args.steps
+    state["keep"] = None
     dist_barrier(dist, torch)
     e2e_ms = run_steps(workers, barrier, state, lib, "e2e", args.steps)
     d2h_bytes = sum(w.d2h_bytes for w in workers)
@@ -524,6 +567,8 @@ def run_ours(args):
     run_steps(workers, barrier, state, lib, "e2e_pageable", 1, passes=1)     # warm-up: every thread's staging ring gets allocated here
     pageable_ms = run_steps(workers, barrier, state, lib, "e2e_pageable", 1, passes=1)
     dist_barrier(dist, torch)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, workers, rank, world)
 
     # ---- roofline: the same frames once more on ONE stream with events around every launch, so that the
     # per-kernel durations are not inflated by the other streams' kernels sharing the SMs ----
@@ -696,7 +741,15 @@ def main():
     ap.add_argument("--passes", type=int, default=PASSES, help="diagnostics: passes over the sequence per step (the contract value is 8)")
     ap.add_argument("--workers", type=int, default=0, help="host threads per GPU (0 = choose from the core count)")
     ap.add_argument("--cpu-frames", type=int, default=24)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path returned in its last step to DIR/*.npy (float32/float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of our arm (--impl ours)")
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
     PASSES = max(1, args.passes)
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":

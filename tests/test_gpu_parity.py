@@ -657,7 +657,7 @@ def test_two_devices_in_one_process(cw):
     (ADVICE r01: the event pool used to be process-global)."""
     import threading
     if cw.cuda_device_count() < 2:
-        pytest.skip("needs two GPUs (gpurun --gpus 2)")
+        pytest.skip("needs two GPUs")
     clouds = [synthetic.camera_cloud(50000 + 1000 * i, seed=60 + i) for i in range(4)]
 
     def chain(p):

@@ -77,7 +77,7 @@ def test_slabs_with_an_empty_part(cw, orc, tmp_path):
 
 def test_slabs_nccl_one_gpu_per_rank(cw, orc, tmp_path):
     if cw.cuda_device_count() < 2:
-        pytest.skip("needs two GPUs (run with gpurun --gpus 2)")
+        pytest.skip("needs two GPUs")
     world = min(cw.cuda_device_count(), 4)
     parts = make_parts(200000, world, seed=31)
     args = dict(voxelsize=0.005, k=30, mul=1.0, cellsize=0.002)
@@ -114,7 +114,7 @@ def test_library_slabs_over_nccl(cw, orc, voxelsize, tmp_path):
     tilefilter of the partitioned cloud against the single-GPU calls and the oracle.  Needs >= 2 GPUs."""
     from parity_helpers import per_tile_check
     if cw.cuda_device_count() < 2:
-        pytest.skip("needs two GPUs (run with gpurun --gpus 2)")
+        pytest.skip("needs two GPUs")
     world = min(cw.cuda_device_count(), 4)
     parts = make_parts(200000, world, seed=31)
     args = dict(voxelsize=voxelsize, k=30, mul=1.0, cellsize=0.002)
@@ -156,7 +156,7 @@ def test_library_slabs_clean_synthetic_cloud_over_nccl(cw, orc, tmp_path):
     two coordinate planes, whole rings lie exactly on leaf faces, and the single-GPU call takes the fused pass while the
     slabs take the planned one -- the records must still be the same, bit for bit."""
     if cw.cuda_device_count() < 2:
-        pytest.skip("needs two GPUs (run with gpurun --gpus 2)")
+        pytest.skip("needs two GPUs")
     world = min(cw.cuda_device_count(), 4)
     pts = synthetic.simulate_cameras(synthetic.synthetic_cloud(640000), 4)
     edges = numpy.quantile(pts["x"], numpy.linspace(0, 1, world + 1))
