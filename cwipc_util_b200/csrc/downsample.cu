@@ -29,6 +29,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 
 #include "device_utils.cuh"
 #include "kernels.hpp"
@@ -1506,14 +1507,14 @@ void table_size(size_t n, bool full, size_t &claim_limit, size_t &capacity) {
 } // namespace
 
 namespace {
-DownsampleResult downsample_impl(const StoragePtr &in, float cellsize, bool octree_split, const OctreeBox *external, uint64_t total_points, int dev, cudaStream_t s) {
-    DownsampleResult result;
-    const size_t n = in->count;
+// pts[0..n) -> voxels.  `dest(v)` is called once, when the voxel count v is known, and returns room for them.
+DownsampleRange downsample_impl(const cwipc_point *pts, size_t n, float cellsize, bool octree_split, const OctreeBox *external, uint64_t total_points,
+                                const std::function<cwipc_point *(size_t)> &dest, int dev, cudaStream_t s) {
+    DownsampleRange result;
     if (n == 0) {
         if (octree_split) {
             // no octree leaves: an empty, non-NULL cloud (python/test_cwipc_util.py:589-594)
-            result.out = std::make_shared<Storage>(dev, 0, s);
-            result.out->mark_ready();
+            (void)dest(0);
         } else {
             result.failed = true; // ref: src/cwipc_filters.cpp:58-62
             result.error = "VoxelGrid filter produced empty pointcloud";
@@ -1557,7 +1558,7 @@ DownsampleResult downsample_impl(const StoragePtr &in, float cellsize, bool octr
             if (!external) {
                 OctreeSeed none;
                 memset(&none, 0, sizeof(none));
-                ob = measure_box(in->d_pts, n, cellsize, octree_split, none, dev, s);
+                ob = measure_box(pts, n, cellsize, octree_split, none, dev, s);
             }
             plan = derive_plan(ob, n, cellsize, octree_split);
             have_plan = true;
@@ -1579,7 +1580,7 @@ DownsampleResult downsample_impl(const StoragePtr &in, float cellsize, bool octr
             Scratch chunk_bbox(fused ? (size_t)ntiles * 6 * sizeof(float) : 0, s), box(sizeof(OctreeBox), s);
             StreamArgs args;
             memset(&args, 0, sizeof(args));
-            args.pts = in->d_pts;
+            args.pts = pts;
             args.n = (uint32_t)n;
             args.ntiles = ntiles;
             args.cs = cellsize;
@@ -1702,7 +1703,7 @@ DownsampleResult downsample_impl(const StoragePtr &in, float cellsize, bool octr
                                                                                                  depth, words.as<uint64_t>(), header);
             });
             const uint64_t *sorted = radix_sort_u64(words.as<uint64_t>(), other.as<uint64_t>(), v, cbits, cbits + keybits, dev, s);
-            auto out = std::make_shared<Storage>(dev, v, s);
+            cwipc_point *dst = dest(v);
             EmitGeom geom;
             memset(&geom, 0, sizeof(geom));
             geom.mode = fused ? VS_FUSED : (octree_split ? VS_TABLES : VS_LINEAR);
@@ -1715,17 +1716,15 @@ DownsampleResult downsample_impl(const StoragePtr &in, float cellsize, bool octr
             }
             launch("voxel_emit_kernel", s, 16 * v, [&] {
                 voxel_emit_kernel<<<(unsigned)std::max<size_t>(1, div_up(v, 256)), 256, 0, s>>>(sorted, (uint32_t)v, (uint32_t)((1ull << cbits) - 1ull), list_keys.as<uint64_t>(),
-                                                                                                list_slots.as<uint32_t>(), table, geom, cellsize, inv_scale, out->d_pts, header);
+                                                                                                list_slots.as<uint32_t>(), table, geom, cellsize, inv_scale, dst, header);
             });
-            out->count = v;
+            result.count = v;
             // centroids lie inside the input's bounding box: hand it on so that a following filter need not recompute it
-            out->has_bounds = true;
+            result.has_bounds = true;
             for (int a = 0; a < 3; a++) {
-                out->bounds_min[a] = plan.gmin[a];
-                out->bounds_max[a] = plan.gmax[a];
+                result.bounds_min[a] = plan.gmin[a];
+                result.bounds_max[a] = plan.gmax[a];
             }
-            out->mark_ready();
-            result.out = out;
             return result;
         } catch (...) {
             thread_zeroed_invalidate(dev);
@@ -1740,10 +1739,37 @@ OctreeSeed no_seed() {
     memset(&none, 0, sizeof(none));
     return none;
 }
+
+// a new cloud of exactly the voxels
+DownsampleResult downsample_to_cloud(const StoragePtr &in, float cellsize, bool octree_split, const OctreeBox *external, uint64_t total_points, int dev, cudaStream_t s) {
+    StoragePtr out;
+    const DownsampleRange r = downsample_impl(in->d_pts, in->count, cellsize, octree_split, external, total_points, [&](size_t v) {
+        out = std::make_shared<Storage>(dev, v, s);
+        return out->d_pts;
+    }, dev, s);
+    DownsampleResult result;
+    if (r.failed) {
+        result.failed = true;
+        result.error = r.error;
+        return result;
+    }
+    out->count = r.count;
+    out->has_bounds = r.has_bounds;
+    memcpy(out->bounds_min, r.bounds_min, sizeof(out->bounds_min));
+    memcpy(out->bounds_max, r.bounds_max, sizeof(out->bounds_max));
+    out->mark_ready();
+    result.out = out;
+    return result;
+}
 } // namespace
 
 DownsampleResult downsample_points(const StoragePtr &in, float cellsize, bool octree_split, int dev, cudaStream_t s) {
-    return downsample_impl(in, cellsize, octree_split, nullptr, 0, dev, s);
+    return downsample_to_cloud(in, cellsize, octree_split, nullptr, 0, dev, s);
+}
+
+// the scale of the centroid sums comes from n, as for a cloud of these n points
+DownsampleRange downsample_range(const cwipc_point *pts, size_t n, float cellsize, bool octree_split, cwipc_point *dst, int dev, cudaStream_t s) {
+    return downsample_impl(pts, n, cellsize, octree_split, nullptr, 0, [dst](size_t) { return dst; }, dev, s);
 }
 
 // Partitioned clouds: the octree box and the bounding box of the WHOLE cloud are supplied by the caller.
@@ -1763,7 +1789,7 @@ DownsampleResult downsample_points_planned(const StoragePtr &in, float cellsize,
         r.error = "planned downsample needs the octree state of the whole cloud";
         return r;
     }
-    return downsample_impl(in, cellsize, octree_split, &ob, state.points, dev, s);
+    return downsample_to_cloud(in, cellsize, octree_split, &ob, state.points, dev, s);
 }
 
 // Continue the octree bounding-box replay over this cloud's points; also returns its bounding box.

@@ -186,6 +186,92 @@ cwipc_pointcloud *cwipc_downsample(cwipc_pointcloud *pc, float voxelsize) {
     });
 }
 
+// cwipc_downsample of every tile group on its own, the results one after another:
+// join(downsample(tilefilter(pc, t1)), downsample(tilefilter(pc, t2)), ...) over the distinct tile values in first-appearance
+// order, tile 0 meaning "every point" as cwipc_tilefilter(pc, 0) does.  Every group is downsampled exactly as cwipc_downsample
+// downsamples the cloud tilefilter(pc, t) (its points in input order; the centroid scale from the group's own count).
+// ref: python/cwipc/registration/util.py:170-182, src/cwipc_filters.cpp:239-256
+cwipc_pointcloud *cwipc_cuda_downsample_pertile(cwipc_pointcloud *pc, float voxelsize) {
+    if (pc == nullptr) return nullptr;
+    const bool octree_split = !(voxelsize < 0);
+    float cellsize = octree_split ? voxelsize : -voxelsize;
+    return guarded<cwipc_pointcloud *>("cwipc_cuda_downsample_pertile", nullptr, [&]() -> cwipc_pointcloud * {
+        if (pc->cellsize() >= cellsize) cellsize = pc->cellsize();
+        StoragePtr in = storage_of(pc, "cwipc_cuda_downsample_pertile");
+        if (!in) return nullptr;
+        const int dev = in->dev;
+        const size_t n = in->count;
+        DeviceGuard g(dev);
+        cudaStream_t s = thread_stream(dev);
+        in->acquire_for_read(s);
+        StoragePtr out;
+        std::string error;
+        try {
+            std::vector<size_t> counts;
+            const std::vector<int> tiles = tiles_in_first_appearance_order(in->d_pts, n, s, &counts);
+            if (tiles.size() <= 1) { // the whole cloud is the only group (or there is none)
+                DownsampleResult r = downsample_points(in, cellsize, octree_split, dev, s);
+                out = r.out;
+                if (r.failed || !out) error = (tiles.empty() ? std::string() : "tile " + std::to_string(tiles[0]) + ": ") + (r.error.empty() ? std::string("downsample failed") : r.error);
+            } else {
+                // the non-zero groups side by side in one buffer; the tile-0 group is the input itself
+                std::vector<int> split;
+                size_t nsplit = 0;
+                for (size_t i = 0; i < tiles.size(); i++) {
+                    if (tiles[i] == 0) continue;
+                    split.push_back(tiles[i]);
+                    nsplit += counts[i];
+                }
+                Scratch grouped(nsplit * sizeof(cwipc_point), s);
+                split_by_tile(in->d_pts, n, split, nsplit, grouped.as<cwipc_point>(), dev, s);
+                // a group keeps at most all of its points: room for the sum of the group sizes
+                const bool has_zero = split.size() < tiles.size();
+                out = std::make_shared<Storage>(dev, has_zero ? n + nsplit : n, s);
+                size_t total = 0, offset = 0;
+                bool first = true;
+                for (size_t i = 0; i < tiles.size(); i++) {
+                    const cwipc_point *src = in->d_pts;
+                    size_t cnt = n;
+                    if (tiles[i] != 0) {
+                        src = grouped.as<cwipc_point>() + offset;
+                        cnt = counts[i];
+                        offset += cnt;
+                    }
+                    const DownsampleRange r = downsample_range(src, cnt, cellsize, octree_split, out->d_pts + total, dev, s);
+                    if (r.failed) {
+                        error = "tile " + std::to_string(tiles[i]) + ": " + r.error;
+                        out.reset();
+                        break;
+                    }
+                    total += r.count;
+                    // a box that holds every group's centroids
+                    for (int a = 0; a < 3; a++) {
+                        out->bounds_min[a] = first ? r.bounds_min[a] : std::min(out->bounds_min[a], r.bounds_min[a]);
+                        out->bounds_max[a] = first ? r.bounds_max[a] : std::max(out->bounds_max[a], r.bounds_max[a]);
+                    }
+                    first = false;
+                }
+                if (out) {
+                    out->count = total;
+                    out->has_bounds = true;
+                    out->mark_ready();
+                }
+            }
+        } catch (...) {
+            in->release_after_read(s);
+            throw;
+        }
+        in->release_after_read(s);
+        if (!out) {
+            log(CWIPC_LOG_LEVEL_ERROR, "cwipc_cuda_downsample_pertile", error);
+            return nullptr;
+        }
+        auto *rv = new DevicePointcloud(out, pc->timestamp(), 0.f);
+        rv->_set_cellsize(cellsize);
+        return rv;
+    });
+}
+
 // Statistical outlier removal, whole cloud or once per distinct tile value (first-appearance order,
 // tile 0 meaning "every point" exactly as cwipc_tilefilter(pc, 0) does).  ref: src/cwipc_filters.cpp:181-278
 cwipc_pointcloud *cwipc_remove_outliers(cwipc_pointcloud *pc, int kNeighbors, float stddevMulThresh, bool perTile) {

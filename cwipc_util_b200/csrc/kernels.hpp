@@ -31,7 +31,11 @@ void colormap_points(const cwipc_point *in, size_t n, cwipc_point *out, uint32_t
 // min over i>=1 of |p_i - p_0| (float), 0 when n < 2.  ref: src/cwipc_util.cpp:173-204
 float min_distance_to_first(const cwipc_point *in, size_t n, cudaStream_t s);
 // distinct tile values in first-appearance order. ref: src/cwipc_filters.cpp:239-249
-std::vector<int> tiles_in_first_appearance_order(const cwipc_point *in, size_t n, cudaStream_t s);
+// counts (nullable) receives the number of points of each, in the same order (same pass, same read-back).
+std::vector<int> tiles_in_first_appearance_order(const cwipc_point *in, size_t n, cudaStream_t s, std::vector<size_t> *counts = nullptr);
+// Stable split by tile value: the points of tiles[0], then those of tiles[1], ..., each group in input order, into out.
+// `tiles` are distinct and non-zero; points of other values are left out.  nkept = the number of points written.
+void split_by_tile(const cwipc_point *in, size_t n, const std::vector<int> &tiles, size_t nkept, cwipc_point *out, int dev, cudaStream_t s);
 
 // The reference's synthetic cloud (src/cwipc_synthetic.cpp:182-222) generated in HBM: side x side points, row hi at height
 // hi * dh, column ai at angle ai * da.  d_radius[hi] (float), d_sin[ai] / d_cos[ai] (double) are the host's own libm values
@@ -47,6 +51,16 @@ struct DownsampleResult {
 // cellsize > 0 already resolved against the cloud's own cellsize.  octree_split selects the
 // reference's positive-size path (per-octree-leaf grids) vs the single global grid.
 DownsampleResult downsample_points(const StoragePtr &in, float cellsize, bool octree_split, int dev, cudaStream_t s);
+// The same downsample of pts[0..n), written to dst (room for n points) instead of a new cloud: the voxels come out exactly as
+// downsample_points gives them for a cloud of these n points.  Returns their number and the input's bounding box.
+struct DownsampleRange {
+    bool failed = false;
+    std::string error;
+    size_t count = 0;
+    bool has_bounds = false; // false when n == 0
+    float bounds_min[3] = {0, 0, 0}, bounds_max[3] = {0, 0, 0};
+};
+DownsampleRange downsample_range(const cwipc_point *pts, size_t n, float cellsize, bool octree_split, cwipc_point *dst, int dev, cudaStream_t s);
 // Octree bounding box of pcl::octree::OctreePointCloud after inserting points in order (a cloud partitioned
 // over several GPUs is replayed part by part, the state travelling from rank to rank).
 struct OctreeState {
@@ -94,6 +108,8 @@ double outlier_threshold(double sum, double sq, double n, float stddev_mul);
 // interval (x_lo, x_hi); kth2 == nullptr marks every query.  Returns their number (synchronises the stream).
 size_t mark_open_queries(const cwipc_point *pts, const float *kth2, size_t nquery, float x_lo, float x_hi, uint32_t *open_idx, int dev, cudaStream_t s);
 void gather_points(const cwipc_point *pts, const uint32_t *idx, size_t n, cwipc_point *out, cudaStream_t s);
+// the same with the indices in the low 32 bits of 64-bit words
+void gather_points(const cwipc_point *pts, const uint64_t *words, size_t n, cwipc_point *out, cudaStream_t s);
 void scatter_floats(const float *values, const uint32_t *idx, size_t n, float *out, cudaStream_t s);
 
 // ---- runtime.cu ----------------------------------------------------------------------------

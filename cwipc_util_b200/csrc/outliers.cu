@@ -1579,9 +1579,10 @@ __global__ void __launch_bounds__(256) mark_open_kernel(const cwipc_point *__res
     first = __shfl_sync(FULL_MASK, first, __ffs(m) - 1);
     if (open) open_idx[first + __popc(m & lanemask_lt())] = i;
 }
-__global__ void __launch_bounds__(256) gather_points_kernel(const cwipc_point *__restrict__ pts, const uint32_t *__restrict__ idx, uint32_t n, cwipc_point *__restrict__ out) {
+template <class Index> // uint32_t, or uint64_t words with the index in their low 32 bits
+__global__ void __launch_bounds__(256) gather_points_kernel(const cwipc_point *__restrict__ pts, const Index *__restrict__ idx, uint32_t n, cwipc_point *__restrict__ out) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) st_point(out, i, ld_point(pts, idx[i]));
+    if (i < n) st_point(out, i, ld_point(pts, (uint32_t)idx[i]));
 }
 __global__ void __launch_bounds__(256) gather_floats_kernel(const float *__restrict__ values, const uint32_t *__restrict__ idx, uint32_t n, float *__restrict__ out) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -1610,6 +1611,11 @@ size_t mark_open_queries(const cwipc_point *pts, const float *kth2, size_t nquer
 void gather_points(const cwipc_point *pts, const uint32_t *idx, size_t n, cwipc_point *out, cudaStream_t s) {
     if (n == 0) return;
     launch("gather_points_kernel", s, 36 * n, [&] { gather_points_kernel<<<(unsigned)div_up(n, 256), 256, 0, s>>>(pts, idx, (uint32_t)n, out); });
+}
+
+void gather_points(const cwipc_point *pts, const uint64_t *words, size_t n, cwipc_point *out, cudaStream_t s) {
+    if (n == 0) return;
+    launch("gather_points_kernel", s, 40 * n, [&] { gather_points_kernel<<<(unsigned)div_up(n, 256), 256, 0, s>>>(pts, words, (uint32_t)n, out); });
 }
 
 void gather_floats(const float *values, const uint32_t *idx, size_t n, float *out, cudaStream_t s) {

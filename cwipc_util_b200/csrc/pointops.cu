@@ -1,4 +1,5 @@
-// pointops.cu -- stable single-pass compaction (tilefilter / crop / outlier mask) and per-point maps.
+// pointops.cu -- stable single-pass compaction (tilefilter / crop / outlier mask), per-point maps, and the tile listing and
+// stable split by tile of the per-tile filters.
 //
 // ref: src/cwipc_filters.cpp:281-306 (tilefilter), :308-331 (tilemap), :333-360 (crop),
 //      :362-386 (colormap); src/cwipc_util.cpp:173-204 (cellsize heuristic).
@@ -8,6 +9,7 @@
 // (the reference's loops are sequential push_backs).  Algorithmic bytes: 16*N read + 16*M written.
 #include "device_utils.cuh"
 #include "kernels.hpp"
+#include "radix_sort.hpp"
 
 #include <algorithm>
 #include <cstring>
@@ -214,18 +216,46 @@ __global__ void __launch_bounds__(256) min_dist2_kernel(const cwipc_point *__res
     if (lane_id() == 0) atomicMin(result_bits, __float_as_uint(best));
 }
 
-__global__ void __launch_bounds__(256) first_tile_kernel(const cwipc_point *__restrict__ in, uint32_t n, uint32_t *__restrict__ first_index) {
+// first index of every tile value and, when `counts` is not null, its number of points (one atomic per value and warp)
+__global__ void __launch_bounds__(256) first_tile_kernel(const cwipc_point *__restrict__ in, uint32_t n, uint32_t *__restrict__ first_index, uint32_t *__restrict__ counts) {
     __shared__ uint32_t s_first[256];
+    __shared__ uint32_t s_count[256];
     s_first[threadIdx.x] = 0xffffffffu;
+    s_count[threadIdx.x] = 0;
     __syncthreads();
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-        const Point16 p = ld_point_stream(in, i);
-        const uint32_t t = pt_tile(p);
-        if (s_first[t] > i) atomicMin(&s_first[t], i);
+    // the loop bound is uniform over the block, so that every lane of a warp takes part in the match
+    for (uint32_t i0 = blockIdx.x * blockDim.x; i0 < n; i0 += gridDim.x * blockDim.x) {
+        const uint32_t i = i0 + threadIdx.x;
+        uint32_t t = 256; // no point
+        if (i < n) {
+            t = pt_tile(ld_point_stream(in, i));
+            if (s_first[t] > i) atomicMin(&s_first[t], i);
+        }
+        if (counts) {
+            const unsigned peers = __match_any_sync(FULL_MASK, t);
+            if (t < 256 && lane_id() == (unsigned)(__ffs(peers) - 1)) atomicAdd(&s_count[t], (uint32_t)__popc(peers));
+        }
     }
     __syncthreads();
     const uint32_t v = s_first[threadIdx.x];
-    if (v != 0xffffffffu) atomicMin(&first_index[threadIdx.x], v);
+    if (v != 0xffffffffu) {
+        atomicMin(&first_index[threadIdx.x], v);
+        if (counts) atomicAdd(&counts[threadIdx.x], s_count[threadIdx.x]);
+    }
+}
+
+// rank of every tile value in a split (points of values outside the split get a rank above every group's)
+struct TileRanks {
+    uint8_t r[256];
+};
+
+// sort word of point i: [rank of its tile | i]
+__global__ void __launch_bounds__(256) tile_split_words_kernel(const cwipc_point *__restrict__ in, uint32_t n, TileRanks ranks, uint64_t *__restrict__ words) {
+    __shared__ uint8_t s_rank[256];
+    s_rank[threadIdx.x] = ranks.r[threadIdx.x];
+    __syncthreads();
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+        words[i] = ((uint64_t)s_rank[pt_tile(ld_point_stream(in, i))] << 32) | i;
 }
 
 unsigned grid_for(size_t n, int threads, int dev, int blocks_per_sm) {
@@ -292,22 +322,48 @@ float min_distance_to_first(const cwipc_point *in, size_t n, cudaStream_t s) {
     return sqrtf(d2);
 }
 
-std::vector<int> tiles_in_first_appearance_order(const cwipc_point *in, size_t n, cudaStream_t s) {
+std::vector<int> tiles_in_first_appearance_order(const cwipc_point *in, size_t n, cudaStream_t s, std::vector<size_t> *counts) {
     std::vector<int> tiles;
+    if (counts) counts->clear();
     if (n == 0) return tiles;
-    Scratch scratch(256 * sizeof(uint32_t), s);
+    // [first index x 256 | count x 256]
+    const size_t words = counts ? 512 : 256;
+    Scratch scratch(words * sizeof(uint32_t), s);
     CWCU_CHECK(cudaMemsetAsync(scratch.p, 0xff, 256 * sizeof(uint32_t), s));
+    if (counts) CWCU_CHECK(cudaMemsetAsync(scratch.as<uint32_t>() + 256, 0, 256 * sizeof(uint32_t), s));
     const unsigned grid = grid_for(n, 256, device_of_stream_guard(), 4);
-    launch("first_tile_kernel", s, 16 * (size_t)n, [&] { first_tile_kernel<<<grid, 256, 0, s>>>(in, (uint32_t)n, scratch.as<uint32_t>()); });
-    uint32_t *h = static_cast<uint32_t *>(thread_pinned(256 * sizeof(uint32_t)));
-    CWCU_CHECK(cudaMemcpyAsync(h, scratch.p, 256 * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    launch("first_tile_kernel", s, 16 * (size_t)n, [&] {
+        first_tile_kernel<<<grid, 256, 0, s>>>(in, (uint32_t)n, scratch.as<uint32_t>(), counts ? scratch.as<uint32_t>() + 256 : nullptr);
+    });
+    uint32_t *h = static_cast<uint32_t *>(thread_pinned(words * sizeof(uint32_t)));
+    CWCU_CHECK(cudaMemcpyAsync(h, scratch.p, words * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
     stream_sync(s);
     std::vector<std::pair<uint32_t, int>> found;
     for (int t = 0; t < 256; t++)
         if (h[t] != 0xffffffffu) found.emplace_back(h[t], t);
     std::sort(found.begin(), found.end());
-    for (auto &f : found) tiles.push_back(f.second);
+    for (auto &f : found) {
+        tiles.push_back(f.second);
+        if (counts) counts->push_back(h[256 + f.second]);
+    }
     return tiles;
+}
+
+// One radix pass on [rank | index] words keeps input order inside every group; the gather then reads each group's points
+// in order.
+void split_by_tile(const cwipc_point *in, size_t n, const std::vector<int> &tiles, size_t nkept, cwipc_point *out, int dev, cudaStream_t s) {
+    if (nkept == 0) return;
+    TileRanks ranks;
+    const uint8_t none = (uint8_t)tiles.size(); // <= 255: tile 0 is never among them
+    memset(ranks.r, none, sizeof(ranks.r));
+    for (size_t g = 0; g < tiles.size(); g++) ranks.r[tiles[g]] = (uint8_t)g;
+    Scratch a(n * sizeof(uint64_t), s), b(n * sizeof(uint64_t), s);
+    const unsigned grid = grid_for(n, 256, dev, 8);
+    launch("tile_split_words_kernel", s, 24 * n, [&] { tile_split_words_kernel<<<grid, 256, 0, s>>>(in, (uint32_t)n, ranks, a.as<uint64_t>()); });
+    int bits = 1;
+    while ((1u << bits) <= none) bits++;
+    const uint64_t *sorted = radix_sort_u64(a.as<uint64_t>(), b.as<uint64_t>(), n, 32, 32 + bits, dev, s);
+    gather_points(in, sorted, nkept, out, s);
 }
 
 // ---- L2 flush (bench hygiene) --------------------------------------------------------------

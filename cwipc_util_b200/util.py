@@ -25,7 +25,7 @@ __all__ = [
     "cwipc_read", "cwipc_write", "cwipc_read_debugdump", "cwipc_write_debugdump",
     "cwipc_from_points", "cwipc_from_numpy_array", "cwipc_from_numpy_matrix", "cwipc_from_packet", "cwipc_synthetic",
     "cwipc_downsample", "cwipc_remove_outliers", "cwipc_tilefilter", "cwipc_tilemap", "cwipc_colormap", "cwipc_crop",
-    "cwipc_join", "cwipc_join_multi", "cwipc_tilefilter_masked",
+    "cwipc_join", "cwipc_join_multi", "cwipc_tilefilter_masked", "cwipc_downsample_pertile",
     "cuda_device_count", "cuda_set_device", "cuda_synchronize", "cuda_kernel_launches",
 ]
 
@@ -143,6 +143,7 @@ def cwipc_util_dll_load(libname: Optional[str] = None) -> ctypes.CDLL:
         "cwipc_remove_outliers": ([cwipc_pointcloud_p, ctypes.c_int, ctypes.c_float, ctypes.c_bool], cwipc_pointcloud_p),
         "cwipc_tilefilter": ([cwipc_pointcloud_p, ctypes.c_int], cwipc_pointcloud_p),
         "cwipc_cuda_tilefilter_masked": ([cwipc_pointcloud_p, ctypes.c_int], cwipc_pointcloud_p),
+        "cwipc_cuda_downsample_pertile": ([cwipc_pointcloud_p, ctypes.c_float], cwipc_pointcloud_p),
         "cwipc_tilemap": ([cwipc_pointcloud_p, ctypes.c_char_p], cwipc_pointcloud_p),
         "cwipc_colormap": ([cwipc_pointcloud_p, ctypes.c_uint32, ctypes.c_uint32], cwipc_pointcloud_p),
         "cwipc_crop": ([cwipc_pointcloud_p, ctypes.POINTER(ctypes.c_float)], cwipc_pointcloud_p),
@@ -453,6 +454,12 @@ def cwipc_tilefilter(pc: cwipc_pointcloud_wrapper, tile: int) -> cwipc_pointclou
 def cwipc_tilefilter_masked(pc: cwipc_pointcloud_wrapper, mask: int) -> cwipc_pointcloud_wrapper:
     """(tile & mask) != 0 -- ref: python/cwipc/registration/util.py:98-112, here one kernel instead of a host round trip."""
     return cwipc_pointcloud_wrapper(cwipc_util_dll_load().cwipc_cuda_tilefilter_masked(pc.as_cwipc_p(), mask))
+
+
+def cwipc_downsample_pertile(pc: cwipc_pointcloud_wrapper, voxelsize: float) -> cwipc_pointcloud_wrapper:
+    """cwipc_downsample of every tile (camera) on its own, the results joined in first-appearance order of the tile values:
+    python/cwipc/registration/util.py:170-182 (tilefilter -> downsample per tile, then join) as one library call."""
+    return cwipc_pointcloud_wrapper(cwipc_util_dll_load().cwipc_cuda_downsample_pertile(pc.as_cwipc_p(), voxelsize))
 
 
 def cwipc_tilemap(pc: cwipc_pointcloud_wrapper, mapping: Union[List[int], dict, bytes]) -> cwipc_pointcloud_wrapper:

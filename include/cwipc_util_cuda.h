@@ -312,6 +312,14 @@ _CWIPC_UTIL_EXPORT int cwipc_cuda_pointcloud_device(cwipc_pointcloud *pc);
 _CWIPC_UTIL_EXPORT const void *cwipc_cuda_pointcloud_device_ptr(cwipc_pointcloud *pc);
 /* cwipc_tilefilter variant used by python/cwipc/registration/util.py:98-112: keep (tile & mask) != 0. */
 _CWIPC_UTIL_EXPORT cwipc_pointcloud *cwipc_cuda_tilefilter_masked(cwipc_pointcloud *pc, int mask);
+/* cwipc_downsample of each camera's points on their own, in one call: the same records, in the same order, as
+ *   join(downsample(tilefilter(pc, t1), voxelsize), downsample(tilefilter(pc, t2), voxelsize), ...)
+ * over the distinct tile values t1, t2, ... in first-appearance order (src/cwipc_filters.cpp:239-256), tile 0 standing for
+ * every point as in cwipc_tilefilter.  This is what python/cwipc/registration/util.py:170-182 (cwipc_downsample_pertile)
+ * builds from those filters, so that no voxel mixes the points of two cameras.  voxelsize as in cwipc_downsample (negative:
+ * one grid); the result has the input's timestamp and the effective cell size.  Empty input: as cwipc_downsample.  NULL,
+ * with an ERROR log naming the tile value, when a group cannot be downsampled. */
+_CWIPC_UTIL_EXPORT cwipc_pointcloud *cwipc_cuda_downsample_pertile(cwipc_pointcloud *pc, float voxelsize);
 /* Per-point mean k-neighbour distance of cwipc_remove_outliers' first pass, copied to host
  * (dist[count]); returns count or -1.  Diagnostic hook used by the parity tests. */
 _CWIPC_UTIL_EXPORT int cwipc_cuda_knn_mean_distances(cwipc_pointcloud *pc, int kNeighbors, float *dist, size_t ndist);
