@@ -8,14 +8,16 @@
 //     own voxel grid, so a voxel cut by a leaf face is emitted once per leaf.  Output order = leaves in
 //     depth-first (Morton, x most significant) order, voxels inside a leaf by (z, y, x);
 //   * negative voxelsize: one grid over the whole cloud, output ordered by (z, y, x);
-//   * per voxel: xyz = mean, rgb = (uint)(float sum / n) (truncation), tile = OR of the tiles.
+//   * per voxel: xyz = mean, rgb = (uint)(float sum / n) (truncation), tile = OR of the tiles.  Here the colour is the exact
+//     floor(sum / n): the reference's result wherever its float sum is exact (every channel sum below 2^24).
 //
 // Pipeline (one stream; N points in, V voxels out):
 //   voxel_stream_kernel   16 B/pt read   ONE pass over the points.  Warps stream 256-point tiles into shared memory
 //                                        (cp.async, double buffered, 128-byte-row swizzle); every lane walks 8
 //                                        CONSECUTIVE points and merges runs of equal (leaf, voxel) in registers, the
 //                                        lanes' partial runs are joined by a segmented shuffle scan, and only whole
-//                                        runs reach the voxel hash table in L2 (one probe + five RED per run).  In
+//                                        runs reach the voxel hash table in L2 (one probe + 5 RED per run, 7 for clouds
+//                                        over 16.8 M points).  In
 //                                        octree mode the same pass computes the 256-point chunk boxes, the block that
 //                                        finishes last replays PCL's sequential octree-box growth from them, and keys
 //                                        are taken relative to the first point (the leaf PARTITION depends on p0 and
@@ -500,20 +502,20 @@ __global__ void __launch_bounds__(256) voxel_keygen_kernel(const cwipc_point *__
 }
 
 // ---- the voxel hash table ---------------------------------------------------------------------------------
-// Every voxel owns one 64-byte slot (two L2 sectors): key, fixed-point coordinate sums RELATIVE to the voxel's own
-// origin, colour sums, point count, tile OR and the voxel's integer coordinates.  Sums are integers, so the result
-// does not depend on the order in which runs arrive (deterministic), and the origin-relative offsets of float
-// coordinates are exact in double, so the centroid is the correctly rounded mean whatever the cloud's extent.
+// Every voxel owns one 64-byte slot (two L2 sectors): key, tile OR, point count, fixed-point coordinate sums RELATIVE to
+// the voxel's own origin and colour sums.  Sums are integers, so the result does not depend on the order in which runs
+// arrive (deterministic), and the origin-relative offsets of float coordinates are exact in double, so the centroid is
+// the correctly rounded mean whatever the cloud's extent.  A voxel of n points sums up to 255 n per colour channel,
+// which passes 2^32 from n = 16 843 010 on: calls with more points than that use the WIDE layout, in which every colour
+// sum has 64 bits of its own (two more RED per run, measurably slower, hence not the default).
 struct __align__(64) VoxelSlot {
     unsigned long long keyp1;      // key + 1; 0 = empty                       } one 16-byte probe
     uint32_t tile;                 // OR of the tile bytes                      }
-    float vx;                      // voxel coordinate floorf(x * inv), x axis  }
-    unsigned long long sx, sy;     // two's-complement fixed-point sums of (x - vx * cellsize) * 2^shift
-    unsigned long long sz;
-    unsigned long long rg;         // sum r | sum g << 32
-    unsigned long long bn;         // sum b | count << 32
-    float vy, vz;
+    uint32_t count;                // wide layout: points                       }
+    unsigned long long sx, sy, sz; // two's-complement fixed-point sums of (x - voxel origin) * 2^shift
+    unsigned long long c[3];       // colour sums.  Narrow: sum r | sum g << 32, sum b | count << 32.  Wide: sum r, sum g, sum b
 };
+constexpr uint32_t VS_NARROW_MAX_POINTS = 16843009; // 255 * 16843009 = 2^32 - 1: the largest call whose 32-bit colour sums cannot overflow
 static_assert(sizeof(VoxelSlot) == 64, "one slot per 64 bytes");
 
 struct TableHeader { // first 64 bytes of the zeroed workspace (layout of the whole head: runtime.hpp, ZW_HEADER_BYTES)
@@ -623,6 +625,7 @@ __device__ __forceinline__ Run queue_load(const uint4 *q, uint32_t pos) {
 // ---- explicit state spaces: the table is global memory and the queue is shared memory, whatever the compiler can prove
 // (through a pointer in a struct it falls back to generic ATOM / LD, which wait for their result) ----
 __device__ __forceinline__ void red_add_u64(void *gaddr, unsigned long long v) { asm volatile("red.global.add.u64 [%0], %1;" ::"l"(gaddr), "l"(v) : "memory"); }
+__device__ __forceinline__ void red_add_u32(void *gaddr, uint32_t v) { asm volatile("red.global.add.u32 [%0], %1;" ::"l"(gaddr), "r"(v) : "memory"); }
 __device__ __forceinline__ void red_or_u32(void *gaddr, uint32_t v) { asm volatile("red.global.or.b32 [%0], %1;" ::"l"(gaddr), "r"(v) : "memory"); }
 __device__ __forceinline__ unsigned long long atom_cas_u64(void *gaddr, unsigned long long cmp, unsigned long long val) {
     unsigned long long old;
@@ -648,7 +651,8 @@ struct DrainCtx { // by value: a reference to the kernel's parameter block would
     uint32_t slot_mask, claim_limit;
 };
 
-// one queued run: find or claim its slot (the first probe `h` is already in flight), add the sums
+// one queued run: find or claim its slot (the first probe `h` is already in flight), add the sums (WIDE: slot layout)
+template <bool WIDE>
 __device__ __forceinline__ void flush_run(const DrainCtx &c, bool active, uint64_t key, uint32_t slot, uint4 h, const uint4 &q0, const uint4 &q1, const uint4 &q2, bool &claimed,
                                           bool &lost, uint32_t &slot_out) {
     claimed = false;
@@ -683,8 +687,15 @@ __device__ __forceinline__ void flush_run(const DrainCtx &c, bool active, uint64
     red_add_u64(&sl->sx, ((unsigned long long)q0.w << 32) | q0.z);
     red_add_u64(&sl->sy, ((unsigned long long)q1.y << 32) | q1.x);
     red_add_u64(&sl->sz, ((unsigned long long)q1.w << 32) | q1.z);
-    red_add_u64(&sl->rg, (unsigned long long)(q2.x & 0xffffu) | ((unsigned long long)(q2.y & 0xffffu) << 32));
-    red_add_u64(&sl->bn, (unsigned long long)(q2.x >> 16) | ((unsigned long long)(q2.y >> 16) << 32));
+    if constexpr (WIDE) {
+        red_add_u64(&sl->c[0], q2.x & 0xffffu);
+        red_add_u64(&sl->c[1], q2.y & 0xffffu);
+        red_add_u64(&sl->c[2], q2.x >> 16);
+        red_add_u32(&sl->count, q2.y >> 16);
+    } else {
+        red_add_u64(&sl->c[0], (unsigned long long)(q2.x & 0xffffu) | ((unsigned long long)(q2.y & 0xffffu) << 32));
+        red_add_u64(&sl->c[1], (unsigned long long)(q2.x >> 16) | ((unsigned long long)(q2.y >> 16) << 32));
+    }
     const uint32_t tl = q2.z >> 24;
     if ((seen_tile & tl) != tl) red_or_u32(&sl->tile, tl);
 }
@@ -693,6 +704,7 @@ __device__ __forceinline__ void flush_run(const DrainCtx &c, bool active, uint64
 // (claim with a 64-bit CAS when the slot is empty, linear probing), then fire-and-forget L2 reductions (RED).  Claims are
 // appended to the voxel list with one counter update per warp and pass.
 // `seen` is the largest claim count this warp has seen so far (returned by its own counter updates): no extra load.
+template <bool WIDE>
 __device__ __noinline__ uint32_t drain_queue(uint32_t qaddr, uint32_t qn, DrainCtx c, unsigned lane, uint32_t seen) {
     __syncwarp();
     // more voxels than the table was sized for: stop claiming (the host repeats the call with a full-size table)
@@ -728,8 +740,8 @@ __device__ __noinline__ uint32_t drain_queue(uint32_t qaddr, uint32_t qn, DrainC
             b2 = lds_v4(qaddr + r1 * (16 * VS_REC) + 32);
         }
         bool cla, clb, losta, lostb;
-        flush_run(c, act0, keya, slota, ha, a0, a1, a2, cla, losta, slota);
-        flush_run(c, act1, keyb, slotb, hb, b0, b1, b2, clb, lostb, slotb);
+        flush_run<WIDE>(c, act0, keya, slota, ha, a0, a1, a2, cla, losta, slota);
+        flush_run<WIDE>(c, act1, keyb, slotb, hb, b0, b1, b2, clb, lostb, slotb);
         if (__any_sync(FULL_MASK, losta || lostb)) {
             if (losta || lostb) red_or_u32(&c.header->pad[5], VS_FLAG_OVERFLOW);
         }
@@ -863,7 +875,8 @@ __device__ __forceinline__ void lookup_leaf(const KeyTables *tab, float cx, floa
     *out = ls;
 }
 
-template <int MODE, bool DBG = false> // DBG: per-phase time accounting of the tile loop (diagnostics build of the fused pass only)
+// WIDE: slot layout (VoxelSlot); DBG: per-phase time accounting of the tile loop (diagnostics build of the fused pass only)
+template <int MODE, bool WIDE, bool DBG = false>
 __global__ void __launch_bounds__(VS_THREADS, 2) voxel_stream_kernel(const __grid_constant__ StreamArgs a, const __grid_constant__ KeyTables g_tab) {
     extern __shared__ __align__(128) unsigned char vs_smem_raw[];
     WarpStage *stages = reinterpret_cast<WarpStage *>(vs_smem_raw);
@@ -930,7 +943,7 @@ __global__ void __launch_bounds__(VS_THREADS, 2) voxel_stream_kernel(const __gri
         dctx.claim_limit = a.claim_limit;
         unsigned long long t0 = 0;
         if (DBG) t0 = now_ns();
-        seen_claims = drain_queue(qaddr, count, dctx, lane, seen_claims);
+        seen_claims = drain_queue<WIDE>(qaddr, count, dctx, lane, seen_claims);
         if (DBG && lane == 0) s_acc[warp][3] += now_ns() - t0;
     };
 
@@ -1260,24 +1273,33 @@ __device__ __forceinline__ void voxel_of_key(uint64_t key, const EmitGeom &g, fl
     }
 }
 
-// mean xyz (exact sum, one rounding), truncated float colour average as pcl::CentroidPoint, OR of tiles
+// mean xyz (exact sum, one rounding), colour floor(sum / n) (pcl::CentroidPoint's truncated float average wherever its
+// float sum is exact), OR of tiles
+template <bool WIDE>
 __device__ __forceinline__ Point16 finalize_voxel(const VoxelSlot &s, const float v[3], float cs, double inv_scale) {
     Point16 o;
-    const unsigned long long cnt = s.bn >> 32;
+    const uint32_t cnt = WIDE ? s.count : (uint32_t)(s.c[1] >> 32);
     const double dn = (double)cnt;
     o.x = (float)((double)__fmul_rn(v[0], cs) + ((double)(long long)s.sx * inv_scale) / dn);
     o.y = (float)((double)__fmul_rn(v[1], cs) + ((double)(long long)s.sy * inv_scale) / dn);
     o.z = (float)((double)__fmul_rn(v[2], cs) + ((double)(long long)s.sz * inv_scale) / dn);
-    const float fn = (float)cnt;
-    const uint32_t r = (uint32_t)__fdiv_rn((float)(s.rg & 0xffffffffull), fn) & 0xffu;
-    const uint32_t g = (uint32_t)__fdiv_rn((float)(s.rg >> 32), fn) & 0xffu;
-    const uint32_t b = (uint32_t)__fdiv_rn((float)(s.bn & 0xffffffffull), fn) & 0xffu;
+    uint32_t r, g, b; // floor(sum / n) <= 255
+    if constexpr (WIDE) {
+        r = (uint32_t)(s.c[0] / cnt);
+        g = (uint32_t)(s.c[1] / cnt);
+        b = (uint32_t)(s.c[2] / cnt);
+    } else {
+        r = (uint32_t)s.c[0] / cnt;
+        g = (uint32_t)(s.c[0] >> 32) / cnt;
+        b = (uint32_t)s.c[1] / cnt;
+    }
     o.rgbt = r | (g << 8) | (b << 16) | ((s.tile & 0xffu) << 24);
     return o;
 }
 
 // One output point per sorted list entry; the slot is read once and cleared, so the table is all zero
 // again when the kernel ends (no memset between calls).
+template <bool WIDE>
 __global__ void __launch_bounds__(256) voxel_emit_kernel(const uint64_t *__restrict__ sorted, uint32_t v, uint32_t cmask, const uint64_t *__restrict__ list_keys,
                                                           const uint32_t *__restrict__ list_slots, VoxelSlot *__restrict__ table, EmitGeom geom, float cs, double inv_scale,
                                                           cwipc_point *__restrict__ out, TableHeader *__restrict__ header) {
@@ -1302,7 +1324,7 @@ __global__ void __launch_bounds__(256) voxel_emit_kernel(const uint64_t *__restr
     raw[3] = zero;
     float vox[3];
     voxel_of_key(list_keys[c], geom, vox);
-    st_point(out, j, finalize_voxel(u.s, vox, cs, inv_scale));
+    st_point(out, j, finalize_voxel<WIDE>(u.s, vox, cs, inv_scale));
 }
 
 // a pass that failed half way: clear the claimed slots (the list knows them) and the header words
@@ -1472,28 +1494,28 @@ unsigned stream_grid(size_t n, int dev) {
 
 constexpr size_t VS_SMEM_BYTES = sizeof(WarpStage) * VS_WARPS + sizeof(KeyTables);
 
-template <int MODE>
+template <int MODE, bool WIDE>
 void launch_stream(const StreamArgs &args, const KeyTables &tab, int dev, cudaStream_t s) {
     static std::once_flag once[64];
     std::call_once(once[dev & 63], [&] {
-        CWCU_CHECK(cudaFuncSetAttribute(voxel_stream_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)VS_SMEM_BYTES));
+        CWCU_CHECK(cudaFuncSetAttribute(voxel_stream_kernel<MODE, WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)VS_SMEM_BYTES));
     });
     // two blocks of 106 KB per SM need the largest carve-out ($CWIPC_CUDA_DS_CARVEOUT, $CWIPC_CUDA_DS_BLOCKS_PER_SM: tuning only)
     static const int carveout = [] { const char *e = getenv("CWIPC_CUDA_DS_CARVEOUT"); return e && *e ? atoi(e) : (int)cudaSharedmemCarveoutMaxShared; }();
     static const size_t blocks_per_sm = [] { const char *e = getenv("CWIPC_CUDA_DS_BLOCKS_PER_SM"); return (size_t)std::max(1, std::min(2, e && *e ? atoi(e) : 2)); }();
-    tune_kernel(voxel_stream_kernel<MODE>, carveout, true);
+    tune_kernel(voxel_stream_kernel<MODE, WIDE>, carveout, true);
     // persistent warps: two blocks of eight warps per SM, every warp takes tiles gw, gw + nw, ...
     static const size_t tiles_per_warp = [] { const char *e = getenv("CWIPC_CUDA_DS_TILES_PER_WARP"); return (size_t)std::max(1, e && *e ? atoi(e) : 1); }(); // tuning only
     const unsigned grid = (unsigned)std::max<size_t>(1, std::min(div_up((size_t)args.ntiles, (size_t)VS_WARPS * tiles_per_warp), (size_t)sm_count(dev) * blocks_per_sm));
     if constexpr (MODE == VS_FUSED) {
         if (args.dbg) { // $CWIPC_CUDA_DEBUG_STREAM: the build with per-phase time accounting
-            CWCU_CHECK(cudaFuncSetAttribute(voxel_stream_kernel<MODE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)VS_SMEM_BYTES));
-            tune_kernel(voxel_stream_kernel<MODE, true>, carveout, true);
-            launch("voxel_stream_kernel", s, 16 * (size_t)args.n, [&] { voxel_stream_kernel<MODE, true><<<grid, VS_THREADS, VS_SMEM_BYTES, s>>>(args, tab); });
+            CWCU_CHECK(cudaFuncSetAttribute(voxel_stream_kernel<MODE, WIDE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)VS_SMEM_BYTES));
+            tune_kernel(voxel_stream_kernel<MODE, WIDE, true>, carveout, true);
+            launch("voxel_stream_kernel", s, 16 * (size_t)args.n, [&] { voxel_stream_kernel<MODE, WIDE, true><<<grid, VS_THREADS, VS_SMEM_BYTES, s>>>(args, tab); });
             return;
         }
     }
-    launch("voxel_stream_kernel", s, 16 * (size_t)args.n, [&] { voxel_stream_kernel<MODE><<<grid, VS_THREADS, VS_SMEM_BYTES, s>>>(args, tab); });
+    launch("voxel_stream_kernel", s, 16 * (size_t)args.n, [&] { voxel_stream_kernel<MODE, WIDE><<<grid, VS_THREADS, VS_SMEM_BYTES, s>>>(args, tab); });
 }
 
 // hash table size: room for n / 4 voxels (at most half full) when the cloud is large -- a downsample that keeps more than a
@@ -1547,6 +1569,7 @@ DownsampleRange downsample_impl(const cwipc_point *pts, size_t n, float cellsize
     const bool force_small = force && !strcmp(force, "smalltable");
     bool fused = octree_split && external == nullptr && !force_twopass;
     bool full_table = false;
+    const bool wide = n > VS_NARROW_MAX_POINTS; // slot layout (VoxelSlot)
     OctreeBox ob;
     memset(&ob, 0, sizeof(ob));
     Plan plan;
@@ -1609,7 +1632,7 @@ DownsampleRange downsample_impl(const cwipc_point *pts, size_t n, float cellsize
                     CWCU_CHECK(cudaMemsetAsync(dbg.p, 0xff, sizeof(unsigned long long), s));
                     args.dbg = dbg.as<unsigned long long>();
                 }
-                launch_stream<VS_FUSED>(args, plan.tables, dev, s);
+                wide ? launch_stream<VS_FUSED, true>(args, plan.tables, dev, s) : launch_stream<VS_FUSED, false>(args, plan.tables, dev, s);
                 if (debug_stream) {
                     unsigned long long h[16];
                     CWCU_CHECK(cudaMemcpyAsync(h, dbg.p, sizeof(h), cudaMemcpyDeviceToHost, s));
@@ -1622,7 +1645,7 @@ DownsampleRange downsample_impl(const cwipc_point *pts, size_t n, float cellsize
                 }
             } else {
                 args.kp = plan.kp;
-                if (!octree_split) launch_stream<VS_LINEAR>(args, plan.tables, dev, s);
+                if (!octree_split) wide ? launch_stream<VS_LINEAR, true>(args, plan.tables, dev, s) : launch_stream<VS_LINEAR, false>(args, plan.tables, dev, s);
                 else {
                     if (!plan.use_tables || force_generic) { // no usable tables: empty ones send every run through the generic path
                         memset(&plan.tables, 0, sizeof(plan.tables));
@@ -1630,7 +1653,7 @@ DownsampleRange downsample_impl(const cwipc_point *pts, size_t n, float cellsize
                             for (int m = 0; m <= KT_LEAVES; m++) plan.tables.thr[a][m] = m == 0 ? INFINITY : -INFINITY;
                         plan.tables.inv_res_f = 0.f;
                     }
-                    launch_stream<VS_TABLES>(args, plan.tables, dev, s);
+                    wide ? launch_stream<VS_TABLES, true>(args, plan.tables, dev, s) : launch_stream<VS_TABLES, false>(args, plan.tables, dev, s);
                 }
             }
             // one round trip: voxel count, flags, and (fused pass) the boxes
@@ -1697,7 +1720,7 @@ DownsampleRange downsample_impl(const cwipc_point *pts, size_t n, float cellsize
             }
             Scratch words(v * sizeof(uint64_t), s), other(v * sizeof(uint64_t), s);
             tune_kernel(voxel_words_kernel, CHAIN_CARVEOUT);
-            tune_kernel(voxel_emit_kernel, CHAIN_CARVEOUT);
+            tune_kernel(wide ? voxel_emit_kernel<true> : voxel_emit_kernel<false>, CHAIN_CARVEOUT);
             launch("voxel_words_kernel", s, 16 * v, [&] {
                 voxel_words_kernel<<<(unsigned)std::max<size_t>(1, div_up(v, 256)), 256, 0, s>>>(list_keys.as<uint64_t>(), (uint32_t)v, cbits, fused ? 1 : 0, ob.shift[0], ob.shift[1], ob.shift[2],
                                                                                                  depth, words.as<uint64_t>(), header);
@@ -1715,8 +1738,8 @@ DownsampleRange downsample_impl(const cwipc_point *pts, size_t n, float cellsize
                 geom.div[a] = std::max(1, plan.kp.div[a]);
             }
             launch("voxel_emit_kernel", s, 16 * v, [&] {
-                voxel_emit_kernel<<<(unsigned)std::max<size_t>(1, div_up(v, 256)), 256, 0, s>>>(sorted, (uint32_t)v, (uint32_t)((1ull << cbits) - 1ull), list_keys.as<uint64_t>(),
-                                                                                                list_slots.as<uint32_t>(), table, geom, cellsize, inv_scale, dst, header);
+                (wide ? voxel_emit_kernel<true> : voxel_emit_kernel<false>)<<<(unsigned)std::max<size_t>(1, div_up(v, 256)), 256, 0, s>>>(
+                    sorted, (uint32_t)v, (uint32_t)((1ull << cbits) - 1ull), list_keys.as<uint64_t>(), list_slots.as<uint32_t>(), table, geom, cellsize, inv_scale, dst, header);
             });
             result.count = v;
             // centroids lie inside the input's bounding box: hand it on so that a following filter need not recompute it

@@ -92,11 +92,51 @@ def assert_points_close(got, want, cs, counts=None):
     assert np.array_equal(got["tile"], want["tile"])
 
 
-def assert_exact_means(got, pts, ranks, counts, cs):
+def exact_voxels(pts, ranks, nvox=None):
+    """Plain reference of a voxel downsample, given each point's voxel rank (its output position): the point count
+    (int64), the float64 mean of x, y, z, the int64 sums of r, g, b, the colours as sum // count, and the OR of the
+    tiles."""
+    nvox = int(ranks.max()) + 1 if nvox is None else nvox
+    ranks = np.asarray(ranks, np.int64)
+    ref = {"count": np.bincount(ranks, minlength=nvox).astype(np.int64)}
+    assert np.all(ref["count"] > 0), "a voxel rank without points"
+    for a in "xyz":
+        ref[a] = np.bincount(ranks, weights=pts[a].astype(np.float64), minlength=nvox) / ref["count"]
+    for c in "rgb":  # float64 sums of integers below 2^53 are exact
+        s = np.bincount(ranks, weights=pts[c].astype(np.float64), minlength=nvox).astype(np.int64)
+        ref["sum_" + c] = s
+        ref[c] = s // ref["count"]
+    tile = np.zeros(nvox, np.uint8)
+    for b in range(8):
+        tile |= (np.bincount(ranks, weights=(pts["tile"] >> b) & 1, minlength=nvox) > 0).astype(np.uint8) << b
+    ref["tile"] = tile
+    return ref
+
+
+def assert_exact_means(got, pts, ranks, counts, cs, want=None):
     """The library's centroids are sums in exact integer arithmetic (offsets from the voxel's origin in 2^-46-ish fixed
     point), rounded once: equal to the float64 mean of the voxel's points to within one float32 ulp -- the ulp taken at
-    max(|coordinate|, cellsize / 1024), since next to a coordinate plane a float32 resolves more than the fixed point does."""
+    max(|coordinate|, cellsize / 1024), since next to a coordinate plane a float32 resolves more than the fixed point does.
+    Colours are the exact integer means floor(sum / count) and tiles the OR of the voxel's tiles, both bit for bit.  With
+    `want` (the oracle's output, pcl::CentroidPoint's float running sum) the colours must also equal the oracle's wherever
+    the voxel's channel sum is below 2^24, where that float sum is exact.  `counts` (or None) are the expected counts."""
+    ref = exact_voxels(pts, ranks, len(got) if counts is None else len(counts))
+    assert len(got) == len(ref["count"]), f"{len(got)} voxels, the reference has {len(ref['count'])}"
+    if counts is not None:
+        assert np.array_equal(ref["count"], counts)
+    errors = []
+
+    def report(what, bad, got_v, want_v):
+        if len(bad):
+            v = bad[0]
+            errors.append(f"{what}: {len(bad)} voxels differ, first voxel {v} ({ref['count'][v]} points): got {got_v[v]!r}, want {want_v[v]!r}")
+
+    for c in "rgb":
+        report(f"{c} != floor(sum / count)", np.flatnonzero(got[c].astype(np.int64) != ref[c]), got[c], ref[c])
+        if want is not None:
+            report(f"{c} != oracle where sum < 2^24", np.flatnonzero((ref["sum_" + c] < (1 << 24)) & (got[c] != want[c])), got[c], want[c])
+    report("tile != OR of the tiles", np.flatnonzero(got["tile"] != ref["tile"]), got["tile"], ref["tile"])
     for a in "xyz":
-        exact = np.bincount(ranks, weights=pts[a].astype(np.float64), minlength=len(got)) / counts
-        ulp = np.spacing(np.maximum(np.abs(exact), cs / 1024.0).astype(np.float32)).astype(np.float64)
-        assert np.all(np.abs(got[a].astype(np.float64) - exact) <= ulp), a
+        ulp = np.spacing(np.maximum(np.abs(ref[a]), cs / 1024.0).astype(np.float32)).astype(np.float64)
+        report(f"{a} more than one float32 ulp from the exact mean", np.flatnonzero(~(np.abs(got[a].astype(np.float64) - ref[a]) <= ulp)), got[a], ref[a])
+    assert not errors, "; ".join(errors)
