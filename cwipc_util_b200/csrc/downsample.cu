@@ -1796,7 +1796,7 @@ DownsampleRange downsample_range(const cwipc_point *pts, size_t n, float cellsiz
 }
 
 // Partitioned clouds: the octree box and the bounding box of the WHOLE cloud are supplied by the caller.
-DownsampleResult downsample_points_planned(const StoragePtr &in, float cellsize, bool octree_split, const OctreeState &state, const float bounds[6], int dev, cudaStream_t s) {
+DownsampleResult downsample_points_planned(const StoragePtr &in, float cellsize, bool octree_split, const cwipc_cuda_octree_state &state, const float bounds[6], int dev, cudaStream_t s) {
     OctreeBox ob;
     memset(&ob, 0, sizeof(ob));
     for (int a = 0; a < 3; a++) {
@@ -1816,7 +1816,7 @@ DownsampleResult downsample_points_planned(const StoragePtr &in, float cellsize,
 }
 
 // Continue the octree bounding-box replay over this cloud's points; also returns its bounding box.
-void octree_replay(const cwipc_point *in, size_t n, float cellsize, OctreeState &state, float bounds[6], int dev, cudaStream_t s) {
+void octree_replay(const cwipc_point *in, size_t n, float cellsize, cwipc_cuda_octree_state &state, float bounds[6], int dev, cudaStream_t s) {
     for (int a = 0; a < 3; a++) {
         bounds[a] = INFINITY;
         bounds[3 + a] = -INFINITY;

@@ -62,17 +62,11 @@ struct DownsampleRange {
 };
 DownsampleRange downsample_range(const cwipc_point *pts, size_t n, float cellsize, bool octree_split, cwipc_point *dst, int dev, cudaStream_t s);
 // Octree bounding box of pcl::octree::OctreePointCloud after inserting points in order (a cloud partitioned
-// over several GPUs is replayed part by part, the state travelling from rank to rank).
-struct OctreeState {
-    double min[3] = {0, 0, 0}, max[3] = {0, 0, 0};
-    int depth = 0;
-    int valid = 0;
-    // points inserted so far; the whole cloud's count fixes the fixed-point scale of the centroid sums, so every part of
-    // a partitioned cloud rounds exactly as the one-GPU call does
-    uint64_t points = 0;
-};
-void octree_replay(const cwipc_point *in, size_t n, float cellsize, OctreeState &state, float bounds[6], int dev, cudaStream_t s);
-DownsampleResult downsample_points_planned(const StoragePtr &in, float cellsize, bool octree_split, const OctreeState &state, const float bounds[6], int dev, cudaStream_t s);
+// over several GPUs is replayed part by part, the state travelling from rank to rank).  A state that starts a replay is
+// all zero.
+void octree_replay(const cwipc_point *in, size_t n, float cellsize, cwipc_cuda_octree_state &state, float bounds[6], int dev, cudaStream_t s);
+DownsampleResult downsample_points_planned(const StoragePtr &in, float cellsize, bool octree_split, const cwipc_cuda_octree_state &state, const float bounds[6], int dev,
+                                           cudaStream_t s);
 // global bounding box of in[0..n), n > 0 (synchronises the stream)
 void global_bbox(const cwipc_point *in, size_t n, float gmin[3], float gmax[3], int dev, cudaStream_t s);
 // diagnostic: sort keys (without the index bits) per input point, to host

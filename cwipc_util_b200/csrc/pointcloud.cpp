@@ -90,10 +90,8 @@ void DevicePointcloud::_set_cellsize(float cellsize) {
         cellsize = guarded<float>("cwipc_util", 0.f, [&] {
             DeviceGuard g(st->dev);
             cudaStream_t s = thread_stream(st->dev);
-            st->acquire_for_read(s);
-            float d = min_distance_to_first(st->d_pts, st->count, s);
-            st->release_after_read(s);
-            return d;
+            ReadLease lease(*st, s);
+            return min_distance_to_first(st->d_pts, st->count, s);
         });
     }
     m_cellsize = cellsize;
@@ -130,9 +128,8 @@ int DevicePointcloud::copy_uncompressed(struct cwipc_point *pointbuf, size_t siz
     return guarded<int>("cwipc_util", -1, [&] {
         DeviceGuard g(st->dev);
         cudaStream_t s = thread_stream(st->dev);
-        st->acquire_for_read(s);
+        ReadLease lease(*st, s);
         copy_to_host(pointbuf, st->d_pts, need, s); // returns when pointbuf is complete
-        st->release_after_read(s);
         return (int)st->count;
     });
 }

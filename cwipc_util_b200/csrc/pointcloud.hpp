@@ -83,4 +83,28 @@ R guarded(const char *module, R fallback, F &&body) {
     return fallback;
 }
 
+// The shape of every entry point that reads a cloud: NULL -> `fallback` (silent, as the reference's filters); the cloud's
+// storage (`fallback` when it cannot be had); its device, the calling thread's stream there and a ReadLease on the
+// storage for the whole of `body(in, dev, stream)`; any exception -> an ERROR log naming `who` and `fallback`.
+template <class R, class Body>
+R read_entry(const char *who, cwipc_pointcloud *pc, R fallback, Body &&body) {
+    if (pc == nullptr) return fallback;
+    return guarded<R>(who, fallback, [&]() -> R {
+        StoragePtr in = storage_of(pc, who);
+        if (!in) return fallback;
+        DeviceGuard g(in->dev);
+        cudaStream_t s = thread_stream(in->dev);
+        ReadLease lease(*in, s);
+        return body(in, in->dev, s);
+    });
+}
+
+// A filter result: a new cloud holding `out`, with the given timestamp and cellsize (cellsize < 0: estimated from the
+// points, as cwipc_pointcloud::_set_cellsize does).
+inline cwipc_pointcloud *new_result(StoragePtr out, uint64_t timestamp, float cellsize) {
+    auto *rv = new DevicePointcloud(std::move(out), timestamp, 0.f);
+    rv->_set_cellsize(cellsize);
+    return rv;
+}
+
 } // namespace cwcu

@@ -670,6 +670,16 @@ void Storage::release_after_read(cudaStream_t s) {
     readers.push_back(Reader{s, e, sdev});
 }
 
+ReadLease::~ReadLease() {
+    try {
+        m_st.release_after_read(m_s);
+    } catch (const CudaError &e) {
+        log(CWIPC_LOG_LEVEL_ERROR, "cwipc_util", "cannot record a reader of a pointcloud: " + e.what);
+    } catch (const std::exception &e) {
+        log(CWIPC_LOG_LEVEL_ERROR, "cwipc_util", std::string("cannot record a reader of a pointcloud: ") + e.what());
+    }
+}
+
 // ------------------------------------------------------------------------------------------
 // launch accounting / profiling
 // ------------------------------------------------------------------------------------------

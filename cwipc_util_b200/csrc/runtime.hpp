@@ -151,10 +151,29 @@ struct Storage {
     Storage &operator=(const Storage &) = delete;
 
     void mark_ready();                    // record `ready` on home (call after the producing work is queued)
+
+private:
+    friend class ReadLease;
     void acquire_for_read(cudaStream_t s); // make `s` wait until contents are valid
     void release_after_read(cudaStream_t s); // note that work queued so far on `s` reads this storage
 };
 using StoragePtr = std::shared_ptr<Storage>;
+
+// `s` reads `st` for the scope: the constructor makes `s` wait until the contents are valid, the destructor notes that
+// the work queued on `s` so far reads them, so that the storage's free on its home stream waits for that work on every
+// way out of the scope.  Hold it inside the DeviceGuard of `s`'s device, and hold `st` longer than the lease.  The
+// destructor does not throw: a failure to record the reader (a broken CUDA context) is logged as an ERROR.
+class ReadLease {
+public:
+    ReadLease(Storage &st, cudaStream_t s) : m_st(st), m_s(s) { m_st.acquire_for_read(m_s); }
+    ~ReadLease();
+    ReadLease(const ReadLease &) = delete;
+    ReadLease &operator=(const ReadLease &) = delete;
+
+private:
+    Storage &m_st;
+    cudaStream_t m_s;
+};
 
 // ---- launch accounting / profiling ----
 extern std::atomic<uint64_t> g_kernel_launches;

@@ -236,18 +236,18 @@ StoragePtr slab_downsample_storage(const StoragePtr &in, float voxelsize, float 
     //    usually contains the whole cloud's bounding box after the first part or two: rank r replays its part and
     //    broadcasts the state; as soon as the box contains the global bounding box no later point can move it, and the
     //    chain stops (every rank takes the same decision from the same data).
-    OctreeState state;
+    cwipc_cuda_octree_state state{};
     if (octree) {
-        Scratch wire(sizeof(OctreeState), s);
+        Scratch wire(sizeof(state), s);
         for (int q = 0; q < G; q++) {
             if (q == r) {
                 float ignored[6];
                 octree_replay(in->d_pts, n, cs, state, ignored, dev, s);
-                CWCU_CHECK(cudaMemcpyAsync(wire.p, &state, sizeof(OctreeState), cudaMemcpyHostToDevice, s));
+                CWCU_CHECK(cudaMemcpyAsync(wire.p, &state, sizeof(state), cudaMemcpyHostToDevice, s));
             }
             if (G > 1) {
-                NCCL_CHECK(nccl().Broadcast(wire.p, wire.p, sizeof(OctreeState), NCCL_UINT8, q, c->comm, s));
-                CWCU_CHECK(cudaMemcpyAsync(&state, wire.p, sizeof(OctreeState), cudaMemcpyDeviceToHost, s));
+                NCCL_CHECK(nccl().Broadcast(wire.p, wire.p, sizeof(state), NCCL_UINT8, q, c->comm, s));
+                CWCU_CHECK(cudaMemcpyAsync(&state, wire.p, sizeof(state), cudaMemcpyDeviceToHost, s));
             }
             stream_sync(s);
             bool covers = state.valid != 0;
@@ -452,27 +452,10 @@ size_t slab_sor_group(const cwipc_point *pts, size_t n, cwipc_point *out, int k,
     return compact_points(pts, n, out, p, dev, s);
 }
 
-template <class Body>
-cwipc_pointcloud *slab_filter(const char *who, cwipc_pointcloud *pc, cwipc_cuda_comm *comm, Body &&body) {
-    if (pc == nullptr || comm == nullptr) return nullptr;
-    return guarded<cwipc_pointcloud *>(who, nullptr, [&]() -> cwipc_pointcloud * {
-        if (comm->size > 1 && !nccl().error.empty()) throw CudaError{cudaErrorUnknown, nccl().error};
-        StoragePtr in = storage_of(pc, who);
-        if (!in) return nullptr;
-        if (in->dev != comm->dev) throw CudaError{cudaErrorInvalidDevice, "the cloud lives on another device than the communicator"};
-        DeviceGuard g(in->dev);
-        cudaStream_t s = thread_stream(in->dev);
-        in->acquire_for_read(s);
-        cwipc_pointcloud *rv = nullptr;
-        try {
-            rv = body(in, in->dev, s);
-        } catch (...) {
-            in->release_after_read(s);
-            throw;
-        }
-        in->release_after_read(s);
-        return rv;
-    });
+// what every collective entry point needs of its communicator, for a cloud on `dev`
+void check_comm(const cwipc_cuda_comm *comm, int dev) {
+    if (comm->size > 1 && !nccl().error.empty()) throw CudaError{cudaErrorUnknown, nccl().error};
+    if (dev != comm->dev) throw CudaError{cudaErrorInvalidDevice, "the cloud lives on another device than the communicator"};
 }
 
 } // namespace
@@ -534,12 +517,12 @@ int cwipc_cuda_comm_size(cwipc_cuda_comm *comm) { return comm ? comm->size : -1;
 
 // cwipc_downsample of the cloud whose parts are the ranks' `pc` (rank order); this rank's part of the result
 cwipc_pointcloud *cwipc_cuda_slab_downsample(cwipc_pointcloud *pc, float voxelsize, cwipc_cuda_comm *comm) {
-    return slab_filter("cwipc_cuda_slab_downsample", pc, comm, [&](const StoragePtr &in, int dev, cudaStream_t s) -> cwipc_pointcloud * {
+    if (comm == nullptr) return nullptr;
+    return read_entry<cwipc_pointcloud *>("cwipc_cuda_slab_downsample", pc, nullptr, [&](const StoragePtr &in, int dev, cudaStream_t s) -> cwipc_pointcloud * {
+        check_comm(comm, dev);
         float cs = 0.f;
         StoragePtr out = slab_downsample_storage(in, voxelsize, pc->cellsize(), comm, &cs, dev, s);
-        auto *rv = new DevicePointcloud(out, pc->timestamp(), 0.f);
-        rv->_set_cellsize(cs);
-        return rv;
+        return new_result(out, pc->timestamp(), cs);
     });
 }
 
@@ -547,7 +530,9 @@ cwipc_pointcloud *cwipc_cuda_slab_downsample(cwipc_pointcloud *pc, float voxelsi
 // of first appearance in the WHOLE cloud (tile 0 = every point), this rank's pieces concatenated in that order.
 // halo <= 0: chosen from the cellsize metadata.  ref: src/cwipc_filters.cpp:181-278
 cwipc_pointcloud *cwipc_cuda_slab_remove_outliers(cwipc_pointcloud *pc, int kNeighbors, float stddevMulThresh, bool perTile, float halo, cwipc_cuda_comm *comm) {
-    return slab_filter("cwipc_cuda_slab_remove_outliers", pc, comm, [&](const StoragePtr &in, int dev, cudaStream_t s) -> cwipc_pointcloud * {
+    if (comm == nullptr) return nullptr;
+    return read_entry<cwipc_pointcloud *>("cwipc_cuda_slab_remove_outliers", pc, nullptr, [&](const StoragePtr &in, int dev, cudaStream_t s) -> cwipc_pointcloud * {
+        check_comm(comm, dev);
         const size_t n = in->count;
         const float spacing = pc->cellsize();
         if (kNeighbors > 511) throw CudaError{cudaErrorInvalidValue, "remove_outliers: kNeighbors > 511 is not supported by libcwipc_util_cuda"};
@@ -591,16 +576,16 @@ cwipc_pointcloud *cwipc_cuda_slab_remove_outliers(cwipc_pointcloud *pc, int kNei
             out->count = total;
         }
         out->mark_ready();
-        auto *rv = new DevicePointcloud(out, pc->timestamp(), 0.f);
-        rv->_set_cellsize(pc->cellsize());
-        return rv;
+        return new_result(out, pc->timestamp(), pc->cellsize());
     });
 }
 
 // cwipc_tilefilter of the partitioned cloud: this rank's piece, and where it sits in the whole result (all-gather of the
 // counts).  ref: src/cwipc_filters.cpp:281-306
 cwipc_pointcloud *cwipc_cuda_slab_tilefilter(cwipc_pointcloud *pc, int tile, cwipc_cuda_comm *comm, uint64_t *global_offset, uint64_t *global_count) {
-    return slab_filter("cwipc_cuda_slab_tilefilter", pc, comm, [&](const StoragePtr &in, int dev, cudaStream_t s) -> cwipc_pointcloud * {
+    if (comm == nullptr) return nullptr;
+    return read_entry<cwipc_pointcloud *>("cwipc_cuda_slab_tilefilter", pc, nullptr, [&](const StoragePtr &, int dev, cudaStream_t s) -> cwipc_pointcloud * {
+        check_comm(comm, dev);
         cwipc_pointcloud *rv = cwipc_tilefilter(pc, tile);
         if (!rv) return nullptr;
         double mine = (double)rv->count();
@@ -612,7 +597,6 @@ cwipc_pointcloud *cwipc_cuda_slab_tilefilter(cwipc_pointcloud *pc, int tile, cwi
         }
         if (global_offset) *global_offset = off;
         if (global_count) *global_count = tot;
-        (void)dev;
         return rv;
     });
 }
