@@ -3,6 +3,7 @@
 // kernels in pointops.cu / downsample.cu / outliers.cu.
 // ref: src/cwipc_filters.cpp:30-418
 #include <algorithm>
+#include <cmath>
 #include <cstring>
 
 #include "kernels.hpp"
@@ -55,6 +56,28 @@ StoragePtr compact_to_new(const StoragePtr &in, const Predicate &pred, int dev, 
     inherit_bounds(*out, *in);
     out->mark_ready();
     return out;
+}
+
+// cwipc_cuda_transform's arguments checked, and the matrix slot of every tile value: slot[v] = i for tiles[i] == v, else the
+// tile-0 entry's slot when there is one.  A bad argument throws (-> NULL and one ERROR log).
+void transform_slots(const double *matrices, const uint8_t *tiles, int n, uint16_t slot[256]) {
+    auto bad = [](const std::string &what) { throw CudaError{cudaErrorInvalidValue, what}; };
+    if (n < 1) bad("n must be at least 1");
+    if (matrices == nullptr || tiles == nullptr) bad("matrices and tiles must not be NULL");
+    std::fill(slot, slot + 256, TRANSFORM_NONE);
+    for (int i = 0; i < n; i++) { // a repeat is met by i == 256 at the latest
+        if (slot[tiles[i]] != TRANSFORM_NONE) bad("tile value " + std::to_string(tiles[i]) + " is listed twice");
+        slot[tiles[i]] = (uint16_t)i;
+    }
+    for (int i = 0; i < n; i++) {
+        const double *m = matrices + 16 * i;
+        for (int k = 0; k < 16; k++)
+            if (!std::isfinite(m[k])) bad("matrix " + std::to_string(i) + " has a non-finite entry");
+        if (!(m[12] == 0.0 && m[13] == 0.0 && m[14] == 0.0 && m[15] == 1.0)) bad("the last row of matrix " + std::to_string(i) + " is not (0, 0, 0, 1)");
+    }
+    if (slot[0] != TRANSFORM_NONE)
+        for (int v = 1; v < 256; v++)
+            if (slot[v] == TRANSFORM_NONE) slot[v] = slot[0];
 }
 
 } // namespace
@@ -115,6 +138,21 @@ cwipc_pointcloud *cwipc_colormap(cwipc_pointcloud *pc, uint32_t clearBits, uint3
         auto out = std::make_shared<Storage>(dev, in->count, s);
         out->count = in->count;
         colormap_points(in->d_pts, in->count, out->d_pts, clearBits, setBits, s);
+        out->mark_ready();
+        return out;
+    });
+}
+
+// Every point moved by the 4x4 matrix of its tile value (see include/cwipc_util_cuda.h).  One kernel, no host wait.  The
+// result has no known box: the input's does not bound the moved points, and a stale box would mislead the kNN grid of
+// cwipc_remove_outliers.
+cwipc_pointcloud *cwipc_cuda_transform(cwipc_pointcloud *pc, const double *matrices, const uint8_t *tiles, int n) {
+    return unary_filter("cwipc_cuda_transform", pc, [&](const StoragePtr &in, int dev, cudaStream_t s) -> StoragePtr {
+        uint16_t slot[256];
+        transform_slots(matrices, tiles, n, slot);
+        auto out = std::make_shared<Storage>(dev, in->count, s);
+        out->count = in->count;
+        transform_points(in->d_pts, in->count, out->d_pts, matrices, slot, n, dev, s);
         out->mark_ready();
         return out;
     });

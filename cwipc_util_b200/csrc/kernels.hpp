@@ -27,6 +27,10 @@ void compact_tile_group_chained(const cwipc_point *in, size_t n, cwipc_point *ou
                                 uint32_t *d_total, cudaStream_t s);
 
 void tilemap_points(const cwipc_point *in, size_t n, cwipc_point *out, const uint8_t map[256], cudaStream_t s);
+// cwipc_cuda_transform: out[i] = in[i] with x, y, z moved by matrices[slot[tile]] (nmat row-major 4x4 doubles, affine),
+// or copied when slot[tile] == TRANSFORM_NONE.  1 <= nmat <= 256.  One kernel, no host wait.
+constexpr uint16_t TRANSFORM_NONE = 0xffff; // 16-bit slots: 256 matrices and "none"
+void transform_points(const cwipc_point *in, size_t n, cwipc_point *out, const double *matrices, const uint16_t slot[256], int nmat, int dev, cudaStream_t s);
 void colormap_points(const cwipc_point *in, size_t n, cwipc_point *out, uint32_t clearBits, uint32_t setBits, cudaStream_t s);
 // min over i>=1 of |p_i - p_0| (float), 0 when n < 2.  ref: src/cwipc_util.cpp:173-204
 float min_distance_to_first(const cwipc_point *in, size_t n, cudaStream_t s);

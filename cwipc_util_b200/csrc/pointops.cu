@@ -1,5 +1,5 @@
-// pointops.cu -- stable single-pass compaction (tilefilter / crop / outlier mask), per-point maps, and the tile listing and
-// stable split by tile of the per-tile filters.
+// pointops.cu -- stable single-pass compaction (tilefilter / crop / outlier mask), per-point maps (tilemap, colormap, the
+// per-tile affine transform), and the tile listing and stable split by tile of the per-tile filters.
 //
 // ref: src/cwipc_filters.cpp:281-306 (tilefilter), :308-331 (tilemap), :333-360 (crop),
 //      :362-386 (colormap); src/cwipc_util.cpp:173-204 (cellsize heuristic).
@@ -258,6 +258,62 @@ __global__ void __launch_bounds__(256) tile_split_words_kernel(const cwipc_point
         words[i] = ((uint64_t)s_rank[pt_tile(ld_point_stream(in, i))] << 32) | i;
 }
 
+constexpr int TR_THREADS = 256;
+constexpr int TR_ITEMS = 4; // points in flight per thread
+constexpr int TR_TILE = TR_THREADS * TR_ITEMS;
+
+// cwipc_cuda_transform's table, passed by value as a __grid_constant__ kernel parameter: no device buffer to fill and no
+// copy to wait for.  m[i] holds rows 0..2 of matrix i; slot[v] is the matrix of tile value v.  A launch costs more the
+// larger its parameters are (on a B200, 25 KB took 14 us more host time per launch than 2 KB), so calls with up to 16
+// matrices (the whole cloud, or one per camera) take the kernel instantiated for 16.
+template <int NMAX>
+struct TransformTable {
+    double m[NMAX][12];
+    uint16_t slot[256];
+    uint32_t nmat;
+};
+static_assert(sizeof(TransformTable<256>) <= 32764, "kernel parameters are limited to 32764 bytes (CUDA 12.1 and later)");
+
+// Every point whose tile value has a slot is moved by that slot's 3x4 rows, in double, in a fixed order with no FMA:
+// out = (float)(((m0*x + m1*y) + m2*z) + m3).  The block copies the slot map and the matrices from parameter space to
+// shared memory once: lanes of one warp read different matrices where tiles interleave, and such reads of the constant
+// bank would serialise.
+template <int NMAX>
+__global__ void __launch_bounds__(TR_THREADS) transform_kernel(const cwipc_point *__restrict__ in, uint32_t n, cwipc_point *__restrict__ out,
+                                                                const __grid_constant__ TransformTable<NMAX> table) {
+    extern __shared__ double s_m[]; // table.nmat * 12
+    __shared__ uint16_t s_slot[256];
+    s_slot[threadIdx.x] = table.slot[threadIdx.x];
+    for (uint32_t k = threadIdx.x; k < table.nmat * 12u; k += TR_THREADS) s_m[k] = table.m[k / 12][k % 12];
+    __syncthreads();
+    for (uint32_t t0 = blockIdx.x * TR_TILE; t0 < n; t0 += gridDim.x * TR_TILE) {
+        Point16 p[TR_ITEMS];
+#pragma unroll
+        for (int i = 0; i < TR_ITEMS; i++) {
+            const uint32_t idx = t0 + i * TR_THREADS + threadIdx.x;
+            if (idx < n) p[i] = ld_point_stream(in, idx);
+        }
+#pragma unroll
+        for (int i = 0; i < TR_ITEMS; i++) {
+            const uint32_t idx = t0 + i * TR_THREADS + threadIdx.x;
+            if (idx >= n) continue;
+            const uint32_t slot = s_slot[pt_tile(p[i])];
+            if (slot != TRANSFORM_NONE) {
+                const double *m = s_m + slot * 12;
+                const double x = p[i].x, y = p[i].y, z = p[i].z;
+                float r[3];
+#pragma unroll
+                for (int a = 0; a < 3; a++)
+                    r[a] = __double2float_rn(__dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(m[4 * a], x), __dmul_rn(m[4 * a + 1], y)), __dmul_rn(m[4 * a + 2], z)), m[4 * a + 3]));
+                p[i].x = r[0];
+                p[i].y = r[1];
+                p[i].z = r[2];
+            }
+            st_point(out, idx, p[i]);
+        }
+    }
+}
+
 unsigned grid_for(size_t n, int threads, int dev, int blocks_per_sm) {
     const size_t want = div_up(n, (size_t)threads);
     const size_t cap = (size_t)sm_count(dev) * blocks_per_sm;
@@ -305,6 +361,23 @@ void colormap_points(const cwipc_point *in, size_t n, cwipc_point *out, uint32_t
     if (n == 0) return;
     const unsigned grid = grid_for(n, 256, device_of_stream_guard(), 8);
     launch("colormap_kernel", s, 32 * (size_t)n, [&] { colormap_kernel<<<grid, 256, 0, s>>>(in, (uint32_t)n, out, clearBits, setBits); });
+}
+
+template <int NMAX>
+static void launch_transform(const cwipc_point *in, size_t n, cwipc_point *out, const double *matrices, const uint16_t slot[256], int nmat, int dev, cudaStream_t s) {
+    TransformTable<NMAX> table{};
+    for (int i = 0; i < nmat; i++) memcpy(table.m[i], matrices + 16 * i, sizeof(table.m[i]));
+    memcpy(table.slot, slot, sizeof(table.slot));
+    table.nmat = (uint32_t)nmat;
+    const unsigned grid = grid_for(n, TR_TILE, dev, 4);
+    const size_t smem = (size_t)nmat * sizeof(table.m[0]);
+    launch("transform_kernel", s, 32 * n, [&] { transform_kernel<NMAX><<<grid, TR_THREADS, smem, s>>>(in, (uint32_t)n, out, table); });
+}
+
+void transform_points(const cwipc_point *in, size_t n, cwipc_point *out, const double *matrices, const uint16_t slot[256], int nmat, int dev, cudaStream_t s) {
+    if (n == 0) return;
+    if (nmat <= 16) launch_transform<16>(in, n, out, matrices, slot, nmat, dev, s);
+    else launch_transform<256>(in, n, out, matrices, slot, nmat, dev, s);
 }
 
 float min_distance_to_first(const cwipc_point *in, size_t n, cudaStream_t s) {

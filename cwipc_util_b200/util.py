@@ -13,6 +13,7 @@ from __future__ import annotations
 
 import ctypes
 import os
+from collections.abc import Mapping
 from typing import Any, Iterable, List, Optional, Sequence, Union
 
 import numpy
@@ -25,7 +26,7 @@ __all__ = [
     "cwipc_read", "cwipc_write", "cwipc_read_debugdump", "cwipc_write_debugdump",
     "cwipc_from_points", "cwipc_from_numpy_array", "cwipc_from_numpy_matrix", "cwipc_from_packet", "cwipc_synthetic",
     "cwipc_downsample", "cwipc_remove_outliers", "cwipc_tilefilter", "cwipc_tilemap", "cwipc_colormap", "cwipc_crop",
-    "cwipc_join", "cwipc_join_multi", "cwipc_tilefilter_masked", "cwipc_downsample_pertile",
+    "cwipc_join", "cwipc_join_multi", "cwipc_tilefilter_masked", "cwipc_downsample_pertile", "cwipc_transform",
     "cuda_device_count", "cuda_set_device", "cuda_synchronize", "cuda_kernel_launches",
 ]
 
@@ -144,6 +145,7 @@ def cwipc_util_dll_load(libname: Optional[str] = None) -> ctypes.CDLL:
         "cwipc_tilefilter": ([cwipc_pointcloud_p, ctypes.c_int], cwipc_pointcloud_p),
         "cwipc_cuda_tilefilter_masked": ([cwipc_pointcloud_p, ctypes.c_int], cwipc_pointcloud_p),
         "cwipc_cuda_downsample_pertile": ([cwipc_pointcloud_p, ctypes.c_float], cwipc_pointcloud_p),
+        "cwipc_cuda_transform": ([cwipc_pointcloud_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int], cwipc_pointcloud_p),
         "cwipc_tilemap": ([cwipc_pointcloud_p, ctypes.c_char_p], cwipc_pointcloud_p),
         "cwipc_colormap": ([cwipc_pointcloud_p, ctypes.c_uint32, ctypes.c_uint32], cwipc_pointcloud_p),
         "cwipc_crop": ([cwipc_pointcloud_p, ctypes.POINTER(ctypes.c_float)], cwipc_pointcloud_p),
@@ -460,6 +462,28 @@ def cwipc_downsample_pertile(pc: cwipc_pointcloud_wrapper, voxelsize: float) -> 
     """cwipc_downsample of every tile (camera) on its own, the results joined in first-appearance order of the tile values:
     python/cwipc/registration/util.py:170-182 (tilefilter -> downsample per tile, then join) as one library call."""
     return cwipc_pointcloud_wrapper(cwipc_util_dll_load().cwipc_cuda_downsample_pertile(pc.as_cwipc_p(), voxelsize))
+
+
+def cwipc_transform(pc: cwipc_pointcloud_wrapper, matrices: Any) -> cwipc_pointcloud_wrapper:
+    """Every point moved by a 4x4 matrix on the device (cwipc_cuda_transform in include/cwipc_util_cuda.h): `matrices` is
+    one (4, 4) array-like for the whole cloud, or a mapping {tile value: (4, 4) array-like}, where tile 0 applies to every
+    value without an entry of its own and the points of other values are copied unchanged.  This replaces the round trip
+    get_numpy_matrix -> numpy -> cwipc_from_numpy_matrix.  A matrix of another shape raises ValueError before the library
+    is called; the library checks the rest (NULL and one ERROR log)."""
+    if isinstance(matrices, Mapping):
+        tiles, ms = list(matrices.keys()), list(matrices.values())
+    else:
+        tiles, ms = [0], [matrices]
+    table = numpy.zeros((len(ms), 4, 4), numpy.float64)
+    for i, m in enumerate(ms):
+        a = numpy.asarray(m, dtype=numpy.float64)
+        if a.shape != (4, 4):
+            raise ValueError(f"cwipc_transform: a matrix must have shape (4, 4), not {a.shape}")
+        table[i] = a
+    if not all(0 <= int(t) <= 255 for t in tiles):
+        raise ValueError("cwipc_transform: tile values are 0..255")
+    t = numpy.array([int(v) for v in tiles], numpy.uint8)
+    return cwipc_pointcloud_wrapper(cwipc_util_dll_load().cwipc_cuda_transform(pc.as_cwipc_p(), table.ctypes.data, t.ctypes.data, len(ms)))
 
 
 def cwipc_tilemap(pc: cwipc_pointcloud_wrapper, mapping: Union[List[int], dict, bytes]) -> cwipc_pointcloud_wrapper:

@@ -320,6 +320,24 @@ _CWIPC_UTIL_EXPORT cwipc_pointcloud *cwipc_cuda_tilefilter_masked(cwipc_pointclo
  * one grid); the result has the input's timestamp and the effective cell size.  Empty input: as cwipc_downsample.  NULL,
  * with an ERROR log naming the tile value, when a group cannot be downsampled. */
 _CWIPC_UTIL_EXPORT cwipc_pointcloud *cwipc_cuda_downsample_pertile(cwipc_pointcloud *pc, float voxelsize);
+/* Each point moved by the 4x4 matrix of its tile value.  matrices: n row-major 4x4 doubles; tiles: n tile values.
+ * A point whose tile value equals tiles[i] becomes M_i * (x, y, z, 1); the entry with tile value 0, if any, applies to every
+ * point whose value has no entry of its own (tile 0 standing for the whole cloud, as in cwipc_tilefilter); every other point
+ * is copied unchanged.  Order, colours and tile bytes are kept; the result has the input's timestamp and cellsize.
+ *   Whole cloud: n = 1, tiles = {0}.
+ *   Matching is by the exact tile value, as in cwipc_tilefilter, not by bits.  After cwipc_downsample a voxel's tile is the
+ *   OR of its cameras' tiles: such a voxel moves only if that exact OR value has an entry, or if there is a tile-0 entry.
+ *   Arithmetic: each output coordinate is (float)(((m[r][0]*x + m[r][1]*y) + m[r][2]*z) + m[r][3]), with x, y, z
+ *   promoted to double, every product and sum rounded to double (no fused multiply-add) and the result rounded to the
+ *   nearest float.  numpy float64 elementwise arithmetic in the same order gives the same bits.  So an identity matrix
+ *   returns a listed point bit for bit, except that -0.0 becomes +0.0 (the final + 0.0); unlisted points are copied verbatim.
+ *   Errors: n < 1, NULL matrices or tiles, a tile value listed twice (so also n > 256), a non-finite entry, or a last row
+ *   other than exactly (0, 0, 0, 1) (only affine maps; singular ones are accepted) give NULL and one ERROR log naming
+ *   cwipc_cuda_transform; the input stays usable.  NULL pc: NULL, silently, before any argument check.  An empty cloud
+ *   gives an empty cloud.
+ *   The cellsize is the input's even when a matrix scales the cloud (set it with _set_cellsize where that matters).  No
+ *   metadata is carried over.  The result carries no bounding box: the input's does not bound the moved points. */
+_CWIPC_UTIL_EXPORT cwipc_pointcloud *cwipc_cuda_transform(cwipc_pointcloud *pc, const double *matrices, const uint8_t *tiles, int n);
 /* Per-point mean k-neighbour distance of cwipc_remove_outliers' first pass, copied to host
  * (dist[count]); returns count or -1.  Diagnostic hook used by the parity tests. */
 _CWIPC_UTIL_EXPORT int cwipc_cuda_knn_mean_distances(cwipc_pointcloud *pc, int kNeighbors, float *dist, size_t ndist);
