@@ -36,6 +36,7 @@ SOURCES = [
     "logging.cpp",
     "pointcloud.cpp",
     "filters.cpp",
+    "icp.cpp",
     "slab.cpp",
     "abi.cpp",
     "synthetic.cpp",

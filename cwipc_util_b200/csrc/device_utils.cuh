@@ -47,6 +47,13 @@ __device__ __forceinline__ void st_point(cwipc_point *base, size_t i, const Poin
     *(reinterpret_cast<Point16 *>(base) + i) = p;
 }
 
+// One output coordinate of an affine map, the arithmetic cwipc_cuda_transform and cwipc_cuda_icp state:
+// (float)(((m[0]*x + m[1]*y) + m[2]*z) + m[3]) in double, every product and sum rounded on its own (never fused), the
+// result rounded to the nearest float.  m: one row of a row-major 4x4.
+__device__ __forceinline__ float affine_row(const double *m, double x, double y, double z) {
+    return __double2float_rn(__dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(m[0], x), __dmul_rn(m[1], y)), __dmul_rn(m[2], z)), m[3]));
+}
+
 __device__ __forceinline__ unsigned lane_id() { return threadIdx.x & 31u; }
 __device__ __forceinline__ unsigned lanemask_lt() {
     unsigned m;

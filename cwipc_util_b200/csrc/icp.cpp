@@ -1,0 +1,180 @@
+// icp.cpp -- cwipc_cuda_icp: point-to-point ICP of one device-resident cloud against another, the fine step of multi-camera
+// registration (python/cwipc/registration/: open3d's registration_icp with TransformationEstimationPointToPoint).  The
+// correspondences and their sums come from the target's search index in outliers.cu (IcpMatcher); the host solves the
+// 3x3 rigid motion from those ~20 numbers per iteration and runs the loop.
+#include <cmath>
+#include <cstring>
+
+#include "kernels.hpp"
+#include "pointcloud.hpp"
+
+using namespace cwcu;
+
+namespace {
+
+[[noreturn]] void bad(const std::string &what) { throw CudaError{cudaErrorInvalidValue, what}; }
+
+// Horn's closed-form absolute orientation with unit quaternions (J. Opt. Soc. Am. A 4(4):629-642, 1987): of all rotations,
+// the one that maximises sum (R a_i) . b_i over centred pairs (a_i, b_i) is given by the eigenvector of the largest
+// eigenvalue of a symmetric 4x4 matrix built from S = sum a_i b_i^T.  The eigenvector is found by cyclic Jacobi rotations
+// in double.  The result is always a proper rotation (det +1), also for degenerate (collinear, coincident) pairs.
+void horn_rotation(const double S[3][3], double R[3][3]) {
+    const double xx = S[0][0], xy = S[0][1], xz = S[0][2], yx = S[1][0], yy = S[1][1], yz = S[1][2], zx = S[2][0], zy = S[2][1], zz = S[2][2];
+    double N[4][4] = {{xx + yy + zz, yz - zy, zx - xz, xy - yx},
+                      {yz - zy, xx - yy - zz, xy + yx, zx + xz},
+                      {zx - xz, xy + yx, -xx + yy - zz, yz + zy},
+                      {xy - yx, zx + xz, yz + zy, -xx - yy + zz}};
+    double V[4][4] = {{1, 0, 0, 0}, {0, 1, 0, 0}, {0, 0, 1, 0}, {0, 0, 0, 1}};
+    for (int sweep = 0; sweep < 50; sweep++) {
+        double off = 0.0;
+        for (int p = 0; p < 4; p++)
+            for (int q = p + 1; q < 4; q++) off += N[p][q] * N[p][q];
+        if (off == 0.0) break;
+        for (int p = 0; p < 4; p++) {
+            for (int q = p + 1; q < 4; q++) {
+                const double g = 100.0 * std::fabs(N[p][q]);
+                if (sweep > 3 && std::fabs(N[p][p]) + g == std::fabs(N[p][p]) && std::fabs(N[q][q]) + g == std::fabs(N[q][q])) {
+                    N[p][q] = N[q][p] = 0.0; // below the rounding of both diagonal entries
+                    continue;
+                }
+                if (N[p][q] == 0.0) continue;
+                const double theta = (N[q][q] - N[p][p]) / (2.0 * N[p][q]);
+                const double t = (theta >= 0.0 ? 1.0 : -1.0) / (std::fabs(theta) + std::sqrt(theta * theta + 1.0));
+                const double c = 1.0 / std::sqrt(t * t + 1.0), s = t * c;
+                for (int k = 0; k < 4; k++) { // N <- N P, then P^T N, V <- V P
+                    const double a = N[k][p], b = N[k][q];
+                    N[k][p] = c * a - s * b;
+                    N[k][q] = s * a + c * b;
+                }
+                for (int k = 0; k < 4; k++) {
+                    const double a = N[p][k], b = N[q][k];
+                    N[p][k] = c * a - s * b;
+                    N[q][k] = s * a + c * b;
+                }
+                for (int k = 0; k < 4; k++) {
+                    const double a = V[k][p], b = V[k][q];
+                    V[k][p] = c * a - s * b;
+                    V[k][q] = s * a + c * b;
+                }
+            }
+        }
+    }
+    int best = 0;
+    for (int k = 1; k < 4; k++)
+        if (N[k][k] > N[best][best]) best = k;
+    double w = V[0][best], x = V[1][best], y = V[2][best], z = V[3][best];
+    const double norm = std::sqrt(w * w + x * x + y * y + z * z);
+    w /= norm, x /= norm, y /= norm, z /= norm;
+    R[0][0] = w * w + x * x - y * y - z * z, R[0][1] = 2.0 * (x * y - w * z), R[0][2] = 2.0 * (x * z + w * y);
+    R[1][0] = 2.0 * (y * x + w * z), R[1][1] = w * w - x * x + y * y - z * z, R[1][2] = 2.0 * (y * z - w * x);
+    R[2][0] = 2.0 * (z * x - w * y), R[2][1] = 2.0 * (z * y + w * x), R[2][2] = w * w - x * x - y * y + z * z;
+}
+
+// The rigid motion (row-major 4x4) that minimises sum |R p' + t - q|^2 over the correspondences whose sums (relative to
+// `origin`, layout of IcpMatcher::evaluate) are given.  sums[0] >= 3.
+void rigid_motion(const double sums[ICP_NSUMS], const double origin[3], double dT[16]) {
+    const double n = sums[0];
+    const double *sp = sums + 2, *sq = sums + 5;
+    double S[3][3], R[3][3];
+    for (int a = 0; a < 3; a++)
+        for (int b = 0; b < 3; b++) S[a][b] = sums[8 + 3 * a + b] - sp[a] * sq[b] / n; // the cross-covariance of the centred pairs
+    horn_rotation(S, R);
+    // t = mean q - R mean p', both back in the cloud's own coordinates
+    double mp[3], mq[3];
+    for (int a = 0; a < 3; a++) {
+        mp[a] = sp[a] / n + origin[a];
+        mq[a] = sq[a] / n + origin[a];
+    }
+    memset(dT, 0, 16 * sizeof(double));
+    for (int r = 0; r < 3; r++) {
+        for (int c = 0; c < 3; c++) dT[4 * r + c] = R[r][c];
+        dT[4 * r + 3] = mq[r] - (R[r][0] * mp[0] + R[r][1] * mp[1] + R[r][2] * mp[2]);
+    }
+    dT[15] = 1.0;
+}
+
+void compose(const double a[16], const double b[16], double out[16]) { // out = a * b (row-major 4x4)
+    double r[16];
+    for (int i = 0; i < 4; i++)
+        for (int j = 0; j < 4; j++) r[4 * i + j] = a[4 * i] * b[j] + a[4 * i + 1] * b[4 + j] + a[4 * i + 2] * b[8 + j] + a[4 * i + 3] * b[12 + j];
+    memcpy(out, r, sizeof(r));
+}
+
+struct Evaluation {
+    int32_t correspondences = 0;
+    double fitness = 0.0, rmse = 0.0;
+};
+
+Evaluation summarize(const double sums[ICP_NSUMS], size_t nsource) {
+    Evaluation e;
+    e.correspondences = (int32_t)sums[0];
+    if (e.correspondences > 0) {
+        e.fitness = sums[0] / (double)nsource;
+        e.rmse = std::sqrt(sums[1] / sums[0]);
+    }
+    return e;
+}
+
+} // namespace
+
+extern "C" {
+
+// The loop of open3d's RegistrationICP with point-to-point estimation (see include/cwipc_util_cuda.h for every rule).
+int cwipc_cuda_icp(cwipc_pointcloud *source, cwipc_pointcloud *target, const double init[16], double max_correspondence_distance, int max_iterations,
+                   double relative_fitness, double relative_rmse, struct cwipc_cuda_icp_result *result) {
+    if (target == nullptr) return -1;
+    return read_entry<int>("cwipc_cuda_icp", source, -1, [&](const StoragePtr &src, int dev, cudaStream_t s) -> int {
+        if (!(std::isfinite(max_correspondence_distance) && max_correspondence_distance > 0.0)) bad("max_correspondence_distance must be finite and > 0");
+        if (max_iterations < 0) bad("max_iterations must be >= 0");
+        if (!(std::isfinite(relative_fitness) && relative_fitness >= 0.0 && std::isfinite(relative_rmse) && relative_rmse >= 0.0))
+            bad("relative_fitness and relative_rmse must be finite and >= 0");
+        double T[16] = {1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1};
+        if (init) {
+            for (int k = 0; k < 16; k++)
+                if (!std::isfinite(init[k])) bad("init has a non-finite entry");
+            if (!(init[12] == 0.0 && init[13] == 0.0 && init[14] == 0.0 && init[15] == 1.0)) bad("the last row of init is not (0, 0, 0, 1)");
+            memcpy(T, init, sizeof(T));
+        }
+        if (result == nullptr) bad("result must not be NULL");
+        StoragePtr tgt = storage_of(target, "cwipc_cuda_icp");
+        if (!tgt) return -1;
+        if (tgt->dev != dev) bad("source and target live on different devices (" + std::to_string(dev) + " and " + std::to_string(tgt->dev) + ")");
+        ReadLease lease_t(*tgt, s);
+
+        Evaluation e;
+        int iterations = 0;
+        const size_t ns = src->count;
+        if (ns > 0 && tgt->count > 0) {
+            float box[6];
+            if (tgt->has_bounds) {
+                memcpy(box, tgt->bounds_min, 3 * sizeof(float));
+                memcpy(box + 3, tgt->bounds_max, 3 * sizeof(float));
+            }
+            IcpMatcher matcher(tgt->d_pts, tgt->count, target->cellsize(), tgt->has_bounds ? box : nullptr, dev, s);
+            const float limit = (float)(max_correspondence_distance * max_correspondence_distance);
+            double sums[ICP_NSUMS];
+            matcher.evaluate(src->d_pts, ns, T, limit, true, sums);
+            if (sums[17] != 0.0) bad("the source or the target contains non-finite coordinates");
+            e = summarize(sums, ns);
+            while (iterations < max_iterations && e.correspondences >= 3) {
+                double dT[16];
+                rigid_motion(sums, matcher.origin(), dT);
+                compose(dT, T, T);
+                // the composed motion is applied to the original points (open3d moves its moved copy again: its rounding adds up)
+                matcher.evaluate(src->d_pts, ns, T, limit, false, sums);
+                const Evaluation prev = e;
+                e = summarize(sums, ns);
+                iterations++;
+                if (std::fabs(prev.fitness - e.fitness) < relative_fitness && std::fabs(prev.rmse - e.rmse) < relative_rmse) break;
+            }
+        }
+        memcpy(result->matrix, T, sizeof(T));
+        result->fitness = e.fitness;
+        result->inlier_rmse = e.rmse;
+        result->iterations = iterations;
+        result->correspondences = e.correspondences;
+        return 0;
+    });
+}
+
+} // extern "C"

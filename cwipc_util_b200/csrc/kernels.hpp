@@ -110,6 +110,26 @@ void gather_points(const cwipc_point *pts, const uint32_t *idx, size_t n, cwipc_
 void gather_points(const cwipc_point *pts, const uint64_t *words, size_t n, cwipc_point *out, cudaStream_t s);
 void scatter_floats(const float *values, const uint32_t *idx, size_t n, float *out, cudaStream_t s);
 
+// cwipc_cuda_icp's correspondences: the search index of a target cloud (built once, k = 1), and the evaluation of a motion of
+// a source cloud against it.  sums, in double, relative to origin() (the centre of the target's box), over the pairs
+// (p' = motion * p, its nearest target point q) with float d2 <= limit, ties to the smaller target index:
+//   [0] count, [1] sum d2, [2..4] sum p', [5..7] sum q, [8..16] sum p'_a q_b (row-major a, b),
+//   [17] with check_finite: the number of points of either cloud with a non-finite coordinate (else 0).
+// One search kernel, one reduction kernel and one read-back per evaluation; the same bits on every run.
+constexpr int ICP_NSUMS = 18;
+class IcpMatcher {
+public:
+    // nt > 0; bounds (min xyz, max xyz, nullable): a box known to hold every target point
+    IcpMatcher(const cwipc_point *target, size_t nt, float hint_spacing, const float *bounds, int dev, cudaStream_t s);
+    ~IcpMatcher();
+    const double *origin() const;
+    void evaluate(const cwipc_point *source, size_t ns, const double motion[16], float limit, bool check_finite, double sums[ICP_NSUMS]);
+
+private:
+    struct Impl;
+    std::unique_ptr<Impl> m;
+};
+
 // ---- runtime.cu ----------------------------------------------------------------------------
 void flush_l2(int dev, cudaStream_t s);
 

@@ -1474,6 +1474,188 @@ void check_k(int k, size_t n) {
     (void)n;
 }
 
+// ---- ICP correspondences (cwipc_cuda_icp): the nearest target point of every moved source point ----------------------
+constexpr int ICP_WARPS = 2;
+constexpr int ICP_THREADS = ICP_WARPS * 32;
+constexpr int ICP_BLOCKS_PER_SM = 8;
+
+struct IcpParams {
+    double m[12];      // rows 0..2 of the current source -> target motion
+    double origin[3];  // the sums are taken relative to this point (the centre of the target's box)
+    float limit;       // (float)(max_correspondence_distance^2): a pair counts iff d2 <= limit
+    float slack;       // how far a point may lie outside the nominal box of its node (rounding of cell_u and of the box corners)
+    uint32_t check;    // also count the non-finite coordinates of both clouds (first evaluation of a call)
+};
+
+// The nearest target point to q with d2 <= limit, as the key (d2 bits << 32) | (index in the target's input order), or ~0 when
+// there is none: the smallest key is the smallest d2 and, among equal ones, the smallest index.  Called by all 32 lanes with
+// the same q; the result is the same in every lane.  The search is dfs_knn's for one neighbour: depth-first through the table
+// pyramid, the four nearest open nodes per step (8 lanes per node), nodes of at most leaf_points points scanned.  It starts at
+// the <= 2x2x2 nodes of the lowest level that cover every cell within sqrt(limit) of q, and a node is dropped when its box is
+// farther than min(limit, best d2 so far).  So a query with no target point within the bound only visits the nodes that touch
+// its ball, never a scan of the cells around it.  Nodes at exactly the best d2 are kept: an equally near point with a smaller
+// index must still be seen.
+__device__ __forceinline__ uint64_t icp_nearest(const Point16 q, float limit, float slack, const Point16 *__restrict__ spts16, const uint64_t *__restrict__ sorted,
+                                                const GridParams &gp, const uint2 *__restrict__ table, uint32_t leaf_points, FarNode *stack) {
+    const unsigned lane = lane_id();
+    const uint64_t idxmask = (1ull << gp.idxbits) - 1ull;
+    uint64_t best = ~0ull; // this lane's best key
+    float tau = limit;     // pruning bound, the same in every lane
+    int sp = 0;
+    auto consider = [&](uint32_t c) { // position c of the cell-ordered target
+        const float d2 = dist2(q, spts16[c]);
+        if (d2 <= limit && __float_as_uint(d2) <= (uint32_t)(best >> 32)) best = min(best, ((uint64_t)__float_as_uint(d2) << 32) | (sorted[c] & idxmask));
+    };
+    auto refresh = [&] {
+        const uint32_t hi = __reduce_min_sync(FULL_MASK, (uint32_t)(best >> 32)); // non-negative floats order like their bits
+        if (hi != 0xffffffffu) tau = __uint_as_float(hi);
+    };
+    // Lanes that `want` their node (level cl, (chx, chy, chz)) push it when it holds points and its box is within tau; the
+    // pushed nodes are ranked by (distance, lane), the nearest on top.
+    auto push_nodes = [&](bool want, int cl, uint32_t chx, uint32_t chy, uint32_t chz) {
+        uint2 r = make_uint2(0u, 0u);
+        float mind2 = INFINITY;
+        bool admit = false;
+        if (want && chx < (uint32_t)level_dim(gp.gdim[0], cl) && chy < (uint32_t)level_dim(gp.gdim[1], cl) && chz < (uint32_t)level_dim(gp.gdim[2], cl)) {
+            r = table[table_index(gp, cl, chx, chy, chz)];
+            if (r.y > r.x) {
+                const float pitch = ldexpf(gp.h, cl);
+                const float lo[3] = {gp.gmin[0] + (float)chx * pitch, gp.gmin[1] + (float)chy * pitch, gp.gmin[2] + (float)chz * pitch};
+                const float qq[3] = {q.x, q.y, q.z};
+                mind2 = 0.f;
+#pragma unroll
+                for (int a = 0; a < 3; a++) {
+                    const float d = fmaxf(fmaxf(lo[a] - qq[a], qq[a] - (lo[a] + pitch)) - slack, 0.f);
+                    mind2 += d * d;
+                }
+                admit = !(mind2 * 0.9999f > tau);
+            }
+        }
+        const unsigned adm = __ballot_sync(FULL_MASK, admit);
+        if (adm == 0u) return;
+        const uint32_t mine = __float_as_uint(mind2);
+        int rank = 0;
+        for (unsigned m = adm; m; m &= m - 1u) {
+            const int src = __ffs(m) - 1;
+            const uint32_t other = __shfl_sync(FULL_MASK, mine, src);
+            rank += (other < mine || (other == mine && src < (int)lane)) ? 1 : 0;
+        }
+        const int nadm = __popc(adm);
+        if (admit) {
+            FarNode ch;
+            ch.pb = r.x; ch.pe = r.y; ch.xy = chx | (chy << 16); ch.zl = chz | ((uint32_t)cl << 16); ch.mind2 = mind2;
+            stack[sp + nadm - 1 - rank] = ch;
+        }
+        sp += nadm;
+    };
+
+    {
+        // the lowest level at which the cells within the bound span at most two nodes per axis (the root at the latest)
+        const float rcells = (sqrtf(limit) + slack) * gp.inv_h * 1.000001f + 0.02f;
+        const float u[3] = {cell_u(q.x, gp.gmin[0], gp.inv_h), cell_u(q.y, gp.gmin[1], gp.inv_h), cell_u(q.z, gp.gmin[2], gp.inv_h)};
+        uint32_t lo[3], hi[3];
+#pragma unroll
+        for (int a = 0; a < 3; a++) {
+            lo[a] = (uint32_t)min(max((int)floorf(u[a] - rcells), 0), gp.gdim[a] - 1);
+            hi[a] = (uint32_t)min(max((int)floorf(u[a] + rcells), 0), gp.gdim[a] - 1);
+        }
+        int level = 0;
+        while (level < gp.top_level && !((hi[0] >> level) - (lo[0] >> level) <= 1u && (hi[1] >> level) - (lo[1] >> level) <= 1u && (hi[2] >> level) - (lo[2] >> level) <= 1u)) level++;
+        push_nodes(lane < 8u, level, (lo[0] >> level) + ((lane >> 2) & 1u), (lo[1] >> level) + ((lane >> 1) & 1u), (lo[2] >> level) + (lane & 1u));
+        __syncwarp();
+    }
+    const int group = (int)(lane >> 3);
+    while (sp > 0) {
+        const int take = min(sp, 4);
+        const FarNode node = stack[sp - 1 - min(group, take - 1)]; // lane group g looks at the g-th nearest open node
+        const bool have = group < take && !(node.mind2 * 0.9999f > tau);
+        const int node_level = (int)(node.zl >> 16);
+        sp -= take;
+        __syncwarp();
+        if (__all_sync(FULL_MASK, !have || node.pe - node.pb <= 8u)) { // sparse neighbourhood: every node taken is scanned at once
+            const uint32_t c = node.pb + (lane & 7u);
+            if (have && c < node.pe) consider(c);
+            refresh();
+            continue;
+        }
+        const bool is_leaf = node_level == 0 || node.pe - node.pb <= leaf_points;
+        unsigned todo = __ballot_sync(FULL_MASK, have && is_leaf) & 0x01010101u; // the groups' first lanes vote
+        while (todo) {
+            const int src = __ffs(todo) - 1;
+            todo &= todo - 1u;
+            const uint32_t pb = __shfl_sync(FULL_MASK, node.pb, src), pe = __shfl_sync(FULL_MASK, node.pe, src);
+            if (__shfl_sync(FULL_MASK, node.mind2, src) * 0.9999f > tau) continue; // (the bound may have dropped since the vote)
+            for (uint32_t base = pb; base < pe; base += 32)
+                if (base + lane < pe) consider(base + lane);
+            refresh();
+        }
+        const bool expand = have && !is_leaf && !(node.mind2 * 0.9999f > tau);
+        push_nodes(expand, node_level - 1, 2u * (node.xy & 0xffffu) + ((lane >> 2) & 1u), 2u * (node.xy >> 16) + ((lane >> 1) & 1u), 2u * (node.zl & 0xffffu) + (lane & 1u));
+        __syncwarp();
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) best = min(best, (uint64_t)__shfl_xor_sync(FULL_MASK, (unsigned long long)best, o));
+    return best;
+}
+
+__device__ __forceinline__ bool finite_point(const Point16 &p) { return isfinite(p.x) && isfinite(p.y) && isfinite(p.z); }
+__device__ __forceinline__ double pick3(const double (&v)[3], unsigned i) { return i == 0 ? v[0] : (i == 1 ? v[1] : v[2]); }
+
+// One warp per source point (grid-stride): p' = T p with cwipc_cuda_transform's arithmetic, computed on the fly, and its
+// nearest target point within the bound.  Lane j of a warp adds up term j of the ICP_NSUMS sums over the warp's
+// correspondences, in the warp's (fixed) query order: count, sum d2, sum p' (3), sum q (3), sum p'_a q_b (9, row-major), all in
+// double relative to ip.origin; term 17 is the number of non-finite points of both clouds when ip.check is set.  The warp
+// stores its sums in partial[warp][ICP_NSUMS]; icp_reduce_kernel adds them up in warp order.
+__global__ void __launch_bounds__(ICP_THREADS) icp_match_kernel(const cwipc_point *__restrict__ src, uint32_t ns, const cwipc_point *__restrict__ tgt, uint32_t nt,
+                                                                const cwipc_point *__restrict__ spts, const uint64_t *__restrict__ sorted, const __grid_constant__ GridParams gp,
+                                                                const uint2 *__restrict__ table, uint32_t leaf_points, const __grid_constant__ IcpParams ip, double *__restrict__ partial) {
+    __shared__ __align__(16) FarNode s_stack[ICP_WARPS][KF_STACK];
+    const unsigned lane = lane_id(), warp = threadIdx.x >> 5;
+    const uint32_t gwarp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, warps_total = (gridDim.x * blockDim.x) >> 5;
+    const Point16 *spts16 = reinterpret_cast<const Point16 *>(spts);
+    double acc = 0.0;
+    for (uint32_t qi = gwarp; qi < ns; qi += warps_total) {
+        const Point16 p = ld_point(src, qi);
+        Point16 q;
+        q.x = affine_row(ip.m, p.x, p.y, p.z);
+        q.y = affine_row(ip.m + 4, p.x, p.y, p.z);
+        q.z = affine_row(ip.m + 8, p.x, p.y, p.z);
+        q.rgbt = 0u;
+        if (!finite_point(q)) continue; // (a non-finite input point, counted below; or a float overflow of the motion)
+        const uint64_t key = icp_nearest(q, ip.limit, ip.slack, spts16, sorted, gp, table, leaf_points, s_stack[warp]);
+        if (key == ~0ull) continue;
+        const Point16 t = ld_point(tgt, (uint32_t)key);
+        const double pr[3] = {(double)q.x - ip.origin[0], (double)q.y - ip.origin[1], (double)q.z - ip.origin[2]};
+        const double qr[3] = {(double)t.x - ip.origin[0], (double)t.y - ip.origin[1], (double)t.z - ip.origin[2]};
+        double term = 0.0;
+        if (lane == 0) term = 1.0;
+        else if (lane == 1) term = (double)__uint_as_float((uint32_t)(key >> 32));
+        else if (lane < 5) term = pick3(pr, lane - 2);
+        else if (lane < 8) term = pick3(qr, lane - 5);
+        else if (lane < 17) term = pick3(pr, (lane - 8) / 3) * pick3(qr, (lane - 8) % 3);
+        acc += term;
+    }
+    if (ip.check) {
+        uint32_t bad = 0;
+        for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < ns; i += gridDim.x * blockDim.x) bad += finite_point(ld_point_stream(src, i)) ? 0u : 1u;
+        for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < nt; i += gridDim.x * blockDim.x) bad += finite_point(ld_point_stream(tgt, i)) ? 0u : 1u;
+        bad = warp_sum(bad);
+        if (lane == 17) acc = (double)bad;
+    }
+    if (lane < ICP_NSUMS) partial[(size_t)gwarp * ICP_NSUMS + lane] = acc;
+}
+
+// Warp j adds up sum j of every warp's partial sums: lane l the warps l, l + 32, ... in order, then a fixed butterfly.  With
+// the per-warp order of icp_match_kernel this is a fixed order: the same bits on every run and with any number of callers.
+__global__ void __launch_bounds__(ICP_NSUMS * 32) icp_reduce_kernel(const double *__restrict__ partial, uint32_t nwarps, double *__restrict__ out) {
+    const unsigned lane = lane_id(), j = threadIdx.x >> 5;
+    double s = 0.0;
+    for (uint32_t w = lane; w < nwarps; w += 32) s += partial[(size_t)w * ICP_NSUMS + j];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(FULL_MASK, s, o);
+    if (lane == 0) out[j] = s;
+}
+
 } // namespace
 
 namespace {
@@ -1696,6 +1878,69 @@ size_t remove_outliers_per_tile(const cwipc_point *in, size_t n, cwipc_point *ou
             log(CWIPC_LOG_LEVEL_WARNING, "cwipc_remove_outliers", "fewer points than kNeighbors+1 (" + std::to_string(h[T + 1 + t]) + " <= " + std::to_string(k) + "): keeping all points");
     profile_add_bytes("compact_kernel", 16 * (size_t)h[T]);
     return h[T];
+}
+
+struct IcpMatcher::Impl {
+    KnnIndex ix;
+    const cwipc_point *target;
+    size_t nt;
+    double origin[3];
+    float slack;
+    int dev;
+    cudaStream_t s;
+    uint32_t max_warps;
+    Scratch partial; // [max_warps + 1][ICP_NSUMS]: the warps' sums, then the totals
+};
+
+IcpMatcher::IcpMatcher(const cwipc_point *target, size_t nt, float hint_spacing, const float *bounds, int dev, cudaStream_t s) : m(new Impl) {
+    m->target = target;
+    m->nt = nt;
+    m->dev = dev;
+    m->s = s;
+    float box[6];
+    if (bounds) {
+        memcpy(box, bounds, sizeof(box));
+    } else {
+        global_bbox(target, nt, box, box + 3, dev, s);
+        for (int a = 0; a < 6; a++)
+            if (!std::isfinite(box[a])) throw CudaError{cudaErrorInvalidValue, "the target contains non-finite coordinates"};
+    }
+    float maxabs = 0.f;
+    for (int a = 0; a < 3; a++) {
+        m->origin[a] = 0.5 * ((double)box[a] + (double)box[3 + a]);
+        maxabs = std::max(maxabs, std::max(std::fabs(box[a]), std::fabs(box[3 + a])));
+    }
+    build_index(m->ix, target, nt, 1, hint_spacing, box, dev, s);
+    // a node's box corners are rounded to float like the points themselves: allow a few units in the last place of the
+    // largest coordinate besides the 0.01 pitch of cell_u's rounding
+    m->slack = std::max(0.01f * m->ix.gp.h, 8.f * std::ldexp(maxabs, -23));
+    m->max_warps = (uint32_t)sm_count(dev) * ICP_BLOCKS_PER_SM * ICP_WARPS;
+    m->partial = Scratch(((size_t)m->max_warps + 1) * ICP_NSUMS * sizeof(double), s);
+}
+
+IcpMatcher::~IcpMatcher() = default;
+
+const double *IcpMatcher::origin() const { return m->origin; }
+
+void IcpMatcher::evaluate(const cwipc_point *source, size_t ns, const double motion[16], float limit, bool check_finite, double sums[ICP_NSUMS]) {
+    IcpParams ip;
+    memcpy(ip.m, motion, sizeof(ip.m));
+    memcpy(ip.origin, m->origin, sizeof(ip.origin));
+    ip.limit = limit;
+    ip.slack = m->slack;
+    ip.check = check_finite ? 1u : 0u;
+    const unsigned grid = (unsigned)std::max<size_t>(1, std::min(div_up(ns, (size_t)ICP_WARPS), (size_t)sm_count(m->dev) * ICP_BLOCKS_PER_SM));
+    const uint32_t nwarps = grid * ICP_WARPS;
+    double *partial = m->partial.as<double>(), *d_out = partial + (size_t)m->max_warps * ICP_NSUMS;
+    launch("icp_match_kernel", m->s, 16 * ns, [&] {
+        icp_match_kernel<<<grid, ICP_THREADS, 0, m->s>>>(source, (uint32_t)ns, m->target, (uint32_t)m->nt, m->ix.spts.as<cwipc_point>(), m->ix.sorted, m->ix.gp, m->ix.table.as<uint2>(),
+                                                        far_leaf_points(), ip, partial);
+    });
+    launch("icp_reduce_kernel", m->s, 8 * (size_t)nwarps * ICP_NSUMS, [&] { icp_reduce_kernel<<<1, ICP_NSUMS * 32, 0, m->s>>>(partial, nwarps, d_out); });
+    double *h = static_cast<double *>(thread_pinned(ICP_NSUMS * sizeof(double)));
+    CWCU_CHECK(cudaMemcpyAsync(h, d_out, ICP_NSUMS * sizeof(double), cudaMemcpyDeviceToHost, m->s));
+    stream_sync(m->s);
+    memcpy(sums, h, ICP_NSUMS * sizeof(double));
 }
 
 } // namespace cwcu

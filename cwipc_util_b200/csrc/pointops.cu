@@ -304,7 +304,7 @@ __global__ void __launch_bounds__(TR_THREADS) transform_kernel(const cwipc_point
                 float r[3];
 #pragma unroll
                 for (int a = 0; a < 3; a++)
-                    r[a] = __double2float_rn(__dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(m[4 * a], x), __dmul_rn(m[4 * a + 1], y)), __dmul_rn(m[4 * a + 2], z)), m[4 * a + 3]));
+                    r[a] = affine_row(m + 4 * a, x, y, z);
                 p[i].x = r[0];
                 p[i].y = r[1];
                 p[i].z = r[2];

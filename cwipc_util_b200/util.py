@@ -14,7 +14,7 @@ from __future__ import annotations
 import ctypes
 import os
 from collections.abc import Mapping
-from typing import Any, Iterable, List, Optional, Sequence, Union
+from typing import Any, Iterable, List, NamedTuple, Optional, Sequence, Union
 
 import numpy
 
@@ -27,6 +27,7 @@ __all__ = [
     "cwipc_from_points", "cwipc_from_numpy_array", "cwipc_from_numpy_matrix", "cwipc_from_packet", "cwipc_synthetic",
     "cwipc_downsample", "cwipc_remove_outliers", "cwipc_tilefilter", "cwipc_tilemap", "cwipc_colormap", "cwipc_crop",
     "cwipc_join", "cwipc_join_multi", "cwipc_tilefilter_masked", "cwipc_downsample_pertile", "cwipc_transform",
+    "cwipc_icp", "cwipc_icp_result",
     "cuda_device_count", "cuda_set_device", "cuda_synchronize", "cuda_kernel_launches",
 ]
 
@@ -37,6 +38,12 @@ CWIPC_LOG_LEVEL_NONE, CWIPC_LOG_LEVEL_ERROR, CWIPC_LOG_LEVEL_WARNING, CWIPC_LOG_
 
 class CwipcError(RuntimeError):
     pass
+
+
+class cwipc_cuda_icp_result(ctypes.Structure):
+    """struct cwipc_cuda_icp_result of include/cwipc_util_cuda.h."""
+    _fields_ = [("matrix", ctypes.c_double * 16), ("fitness", ctypes.c_double), ("inlier_rmse", ctypes.c_double),
+                ("iterations", ctypes.c_int32), ("correspondences", ctypes.c_int32)]
 
 
 class cwipc_point(ctypes.Structure):
@@ -146,6 +153,8 @@ def cwipc_util_dll_load(libname: Optional[str] = None) -> ctypes.CDLL:
         "cwipc_cuda_tilefilter_masked": ([cwipc_pointcloud_p, ctypes.c_int], cwipc_pointcloud_p),
         "cwipc_cuda_downsample_pertile": ([cwipc_pointcloud_p, ctypes.c_float], cwipc_pointcloud_p),
         "cwipc_cuda_transform": ([cwipc_pointcloud_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int], cwipc_pointcloud_p),
+        "cwipc_cuda_icp": ([cwipc_pointcloud_p, cwipc_pointcloud_p, ctypes.c_void_p, ctypes.c_double, ctypes.c_int, ctypes.c_double, ctypes.c_double,
+                            ctypes.POINTER(cwipc_cuda_icp_result)], ctypes.c_int),
         "cwipc_tilemap": ([cwipc_pointcloud_p, ctypes.c_char_p], cwipc_pointcloud_p),
         "cwipc_colormap": ([cwipc_pointcloud_p, ctypes.c_uint32, ctypes.c_uint32], cwipc_pointcloud_p),
         "cwipc_crop": ([cwipc_pointcloud_p, ctypes.POINTER(ctypes.c_float)], cwipc_pointcloud_p),
@@ -484,6 +493,35 @@ def cwipc_transform(pc: cwipc_pointcloud_wrapper, matrices: Any) -> cwipc_pointc
         raise ValueError("cwipc_transform: tile values are 0..255")
     t = numpy.array([int(v) for v in tiles], numpy.uint8)
     return cwipc_pointcloud_wrapper(cwipc_util_dll_load().cwipc_cuda_transform(pc.as_cwipc_p(), table.ctypes.data, t.ctypes.data, len(ms)))
+
+
+class cwipc_icp_result(NamedTuple):
+    """What cwipc_icp found: the final source -> target motion (init included) and the last evaluation of it."""
+    matrix: numpy.ndarray  # (4, 4) float64
+    fitness: float         # correspondences / source points
+    inlier_rmse: float     # sqrt(mean d^2) over the correspondences, 0 when there are none
+    iterations: int        # updates applied
+    correspondences: int
+
+
+def cwipc_icp(source: cwipc_pointcloud_wrapper, target: cwipc_pointcloud_wrapper, max_correspondence_distance: float, init: Any = None,
+              max_iterations: int = 30, relative_fitness: float = 1e-6, relative_rmse: float = 1e-6) -> cwipc_icp_result:
+    """Point-to-point ICP of `source` against `target` on the device (cwipc_cuda_icp in include/cwipc_util_cuda.h): the
+    loop of open3d's registration_icp(source, target, max_correspondence_distance, init,
+    TransformationEstimationPointToPoint(), ICPConvergenceCriteria(relative_fitness, relative_rmse, max_iterations)), with
+    the same defaults.  init: a (4, 4) array-like, None for the identity; another shape raises ValueError before the
+    library is called.  A failure of the library (an invalid argument, non-finite coordinates) raises CwipcError."""
+    m = None
+    if init is not None:
+        m = numpy.ascontiguousarray(init, dtype=numpy.float64)
+        if m.shape != (4, 4):
+            raise ValueError(f"cwipc_icp: init must have shape (4, 4), not {m.shape}")
+    res = cwipc_cuda_icp_result()
+    rv = cwipc_util_dll_load().cwipc_cuda_icp(source.as_cwipc_p(), target.as_cwipc_p(), None if m is None else m.ctypes.data, float(max_correspondence_distance),
+                                              int(max_iterations), float(relative_fitness), float(relative_rmse), ctypes.byref(res))
+    if rv != 0:
+        raise CwipcError("cwipc_cuda_icp failed (the ERROR log says why)")
+    return cwipc_icp_result(numpy.array(res.matrix, numpy.float64).reshape(4, 4), res.fitness, res.inlier_rmse, res.iterations, res.correspondences)
 
 
 def cwipc_tilemap(pc: cwipc_pointcloud_wrapper, mapping: Union[List[int], dict, bytes]) -> cwipc_pointcloud_wrapper:

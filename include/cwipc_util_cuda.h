@@ -338,6 +338,39 @@ _CWIPC_UTIL_EXPORT cwipc_pointcloud *cwipc_cuda_downsample_pertile(cwipc_pointcl
  *   The cellsize is the input's even when a matrix scales the cloud (set it with _set_cellsize where that matters).  No
  *   metadata is carried over.  The result carries no bounding box: the input's does not bound the moved points. */
 _CWIPC_UTIL_EXPORT cwipc_pointcloud *cwipc_cuda_transform(cwipc_pointcloud *pc, const double *matrices, const uint8_t *tiles, int n);
+/* Point-to-point ICP of `source` against `target`: the fine step of multi-camera registration, the loop of open3d's
+ * registration_icp with TransformationEstimationPointToPoint(with_scaling = false) and
+ * ICPConvergenceCriteria(relative_fitness, relative_rmse, max_iterations).  init: row-major 4x4 doubles, the starting
+ * source -> target motion T; NULL is the identity.
+ *   Evaluate T: every source point p becomes p' = T * (x, y, z, 1) with exactly cwipc_cuda_transform's arithmetic (double,
+ *   no fused multiply-add, rounded to float).  Its candidate q is the target point with the smallest float
+ *   d2 = ((dx*dx + dy*dy) + dz*dz), every operation rounded to float; of equal d2 the one with the smallest index in the
+ *   target's order.  (p', q) is a correspondence iff d2 <= (float)(max_correspondence_distance^2), the square taken in
+ *   double.  fitness = correspondences / source points; inlier_rmse = sqrt(sum (double)d2 / correspondences), 0 without any.
+ *   Update: with fewer than 3 correspondences the loop stops without one.  Otherwise the rigid motion dT (a proper rotation
+ *   and a translation, no scaling, solved in double) that minimises sum |R p' + t - q|^2 over the correspondences gives
+ *   T <- dT * T, and T is evaluated again.  The composed T is always applied to the ORIGINAL source points (open3d moves
+ *   its copy of the cloud by every dT in turn, so that its rounding accumulates; this call does not).
+ *   Stop when |fitness - previous fitness| < relative_fitness and |rmse - previous rmse| < relative_rmse (absolute
+ *   differences, as in open3d), or after max_iterations updates.  max_iterations = 0 only evaluates init.
+ *   Result: 0, with *result filled from the last evaluation: matrix = the final T (init included), iterations = updates
+ *   applied.  An empty source or target: 0 correspondences, fitness 0, rmse 0, matrix = init, 0 iterations.  source and
+ *   target may be the same cloud.  Both must live on the same device; x-slab (partitioned) clouds are not supported.
+ *   Errors: max_correspondence_distance not finite or not > 0, max_iterations < 0, a negative or non-finite criterion, an
+ *   init with a non-finite entry or a last row other than exactly (0, 0, 0, 1), result == NULL, clouds on two devices, or
+ *   non-finite coordinates in either cloud give -1 and one ERROR log naming cwipc_cuda_icp; the inputs stay usable.
+ *   NULL source or target: -1, silently, before any argument check.
+ *   Cost: one search index over the target per call, then per iteration one search kernel, one reduction kernel and one
+ *   read-back of 18 numbers.  Results are bit-identical from run to run and under concurrent callers. */
+struct cwipc_cuda_icp_result {
+    double matrix[16];       /* row-major 4x4: the final source -> target motion (init included) */
+    double fitness;          /* correspondences / source points of the last evaluation */
+    double inlier_rmse;      /* sqrt(sum d^2 / correspondences) of the last evaluation, 0 when there are none */
+    int32_t iterations;      /* updates applied */
+    int32_t correspondences;
+};
+_CWIPC_UTIL_EXPORT int cwipc_cuda_icp(cwipc_pointcloud *source, cwipc_pointcloud *target, const double init[16], double max_correspondence_distance, int max_iterations,
+                                      double relative_fitness, double relative_rmse, struct cwipc_cuda_icp_result *result);
 /* Per-point mean k-neighbour distance of cwipc_remove_outliers' first pass, copied to host
  * (dist[count]); returns count or -1.  Diagnostic hook used by the parity tests. */
 _CWIPC_UTIL_EXPORT int cwipc_cuda_knn_mean_distances(cwipc_pointcloud *pc, int kNeighbors, float *dist, size_t ndist);

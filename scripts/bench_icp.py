@@ -1,0 +1,124 @@
+#!/usr/bin/env python
+"""cwipc_cuda_icp against the numpy/cKDTree ICP loop of tests/icp_reference.py, on the registration step it serves: each
+camera of the 4-camera synthetic cloud (synthetic.camera_cloud) registered against the other three.
+
+Every camera is first moved by a known seeded pose (2-4 degrees about its centre, 2-4 cm) with cwipc_transform, then
+cwipc_icp(source = that camera, target = cwipc_tilefilter_masked(pc, ~tile & 0xff), 0.05, max_iterations=30) runs with
+open3d's default criteria.  Two sizes: the raw 1 M-point frame, and the frame after cwipc_downsample_pertile(0.005).
+
+Columns: `call_ms` is a host clock around the call, which ends with its own read-back (a device synchronise);
+`index_ms` is the device time of the kernels that build the target's search index (bounding box, keys, radix sort,
+layout), and `per_iter_ms` the device time of one evaluation (icp_match_kernel + icp_reduce_kernel), both from the
+library's launch profile (CUDA events) in a separate call; `ref_s` the reference loop's wall time in the same process.
+The recovered matrices must agree: rotation within 1e-6 and the motion of the camera's centre within 1e-5 m.  The
+card's name and power limit are read, never set.
+
+    python scripts/bench_icp.py [--reps 5]
+"""
+import argparse
+import ctypes
+import json
+import os
+import subprocess
+import sys
+import time
+
+import numpy as np
+from scipy.spatial.transform import Rotation
+
+REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, REPO)
+sys.path.insert(0, os.path.join(REPO, "tests"))
+sys.dont_write_bytecode = True
+
+INDEX_KERNELS = ("bbox_octree_kernel", "knn_keygen_kernel", "radix_cluster_kernel", "radix_fused_kernel", "radix_hist_kernel", "radix_onesweep_kernel",
+                 "radix_scan_kernel", "knn_layout_kernel")
+EVAL_KERNELS = ("icp_match_kernel", "icp_reduce_kernel")
+
+
+def card():
+    try:
+        out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", "0"], capture_output=True, text=True, timeout=30).stdout
+        name, power = [f.strip() for f in out.strip().split(",")[:2]]
+        return {"name": name, "power_limit": power}
+    except Exception as e:  # pragma: no cover
+        return {"name": None, "power_limit": None, "error": repr(e)}
+
+
+def pose(seed, centre):
+    rng = np.random.default_rng(seed)
+    axis = rng.normal(size=3)
+    R = Rotation.from_rotvec(np.radians(rng.uniform(2, 4)) * axis / np.linalg.norm(axis)).as_matrix()
+    t = rng.normal(size=3)
+    T = np.eye(4)
+    T[:3, :3] = R
+    T[:3, 3] = centre - R @ centre + rng.uniform(0.02, 0.04) * t / np.linalg.norm(t)
+    return T
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--reps", type=int, default=5)
+    args = ap.parse_args()
+    import cwipc_util_b200 as cw
+    from cwipc_util_b200 import synthetic
+    import icp_reference as ref
+    lib = cw.util.cwipc_util_dll_load()
+    if cw.cuda_device_count() <= 0:
+        raise SystemExit("bench_icp.py: no CUDA device")
+
+    def profiled(fn):
+        lib.cwipc_cuda_profile_reset()
+        lib.cwipc_cuda_profile_enable(1)
+        out = fn()
+        cw.cuda_synchronize()
+        lib.cwipc_cuda_profile_enable(0)
+        need = lib.cwipc_cuda_profile_report(None, 0)
+        buf = ctypes.create_string_buffer(need)
+        lib.cwipc_cuda_profile_report(buf, need)
+        return out, json.loads(buf.value.decode())
+
+    res = {"card": card(), "reps": args.reps, "rows": []}
+    print(json.dumps(res["card"]), file=sys.stderr)
+    raw = cw.cwipc_from_numpy_array(synthetic.camera_cloud(1000000, seed=1), 1)
+    for size, pc in (("raw 1 M", raw), ("downsample_pertile(0.005)", cw.cwipc_downsample_pertile(raw, 0.005))):
+        for tile in (1, 2, 4, 8):
+            cam = cw.cwipc_tilefilter(pc, tile)
+            centre = ref.xyz32(cam.get_numpy_array()).astype(np.float64).mean(0)
+            P = pose(100 + tile, centre)
+            src = cw.cwipc_transform(cam, P)
+            tgt = cw.cwipc_tilefilter_masked(pc, ~tile & 0xff)
+            call = lambda: cw.cwipc_icp(src, tgt, 0.05, max_iterations=30)
+            call()  # warm-up
+            walls = []
+            for _ in range(args.reps):
+                cw.cuda_synchronize()
+                t0 = time.perf_counter()
+                r = call()
+                walls.append((time.perf_counter() - t0) * 1e3)
+            r, prof = profiled(call)
+            index_ms = sum(prof[k]["total_ms"] for k in INDEX_KERNELS if k in prof)
+            evals = prof["icp_match_kernel"]["launches"]
+            per_iter = sum(prof[k]["total_ms"] for k in EVAL_KERNELS) / evals
+            S, T = ref.xyz32(src.get_numpy_array()), ref.xyz32(tgt.get_numpy_array())
+            t0 = time.perf_counter()
+            want = ref.icp(S, T, 0.05, max_iterations=30)
+            ref_s = time.perf_counter() - t0
+            d = r.matrix - want.matrix
+            agree = bool(np.abs(d[:3, :3]).max() < 1e-6 and np.abs(d[:3, :3] @ centre + d[:3, 3]).max() < 1e-5)
+            E = r.matrix @ P   # what is left of the known displacement
+            row = {"size": size, "camera": tile, "source_points": cam.count(), "target_points": tgt.count(), "iterations": r.iterations,
+                   "fitness": round(r.fitness, 6), "inlier_rmse": r.inlier_rmse, "call_ms": round(float(np.median(walls)), 3),
+                   "call_range_ms": [round(min(walls), 3), round(max(walls), 3)], "index_ms": round(index_ms, 3), "per_iter_ms": round(per_iter, 3),
+                   "evaluations": evals, "ref_s": round(ref_s, 2), "ref_iterations": want.iterations, "matrices_agree": agree,
+                   "residual_deg": float(np.degrees(np.arccos(np.clip((np.trace(E[:3, :3]) - 1) / 2, -1, 1)))),
+                   "residual_centre_m": float(np.linalg.norm(E[:3, :3] @ centre + E[:3, 3] - centre))}
+            res["rows"].append(row)
+            print(json.dumps(row), file=sys.stderr)
+    print(json.dumps(res))
+    if not all(r["matrices_agree"] for r in res["rows"]):
+        raise SystemExit("bench_icp.py: the library's and the reference's matrices differ")
+
+
+if __name__ == "__main__":
+    main()
