@@ -63,8 +63,7 @@ struct OctreeBox {
     // fused pass only: leaf index of the final octree = leaf index relative to the first point's box + shift
     int shift[3];
     int fallback; // 1: the relative keys cannot be trusted (rounding at a leaf face): redo with the two-pass path
-    unsigned long long tail_ns; // diagnostics: time the last block spent on the replay and the checks
-    double m0[3];               // min corner of the first point's box: what the relative leaf indices count from
+    double m0[3]; // min corner of the first point's box: what the relative leaf indices count from
 };
 
 // ---- per-chunk bounding boxes --------------------------------------------------------------------------
@@ -576,10 +575,6 @@ struct StreamArgs {
     uint32_t *super_bbox;         // in the zeroed workspace, behind the table
     double res;
     OctreeBox *box_out;
-    KeyTables *tables_out;        // the block-built tables, for the host-side diagnostics (may be null)
-    // $CWIPC_CUDA_DEBUG_STREAM: globaltimer stamps (ns) -- [0] first block start (min), [1] tables built (max), [2] last warp out of
-    // its tile loop (max), [3] last warp drained (max), [4] last block done, [5] sum and [6] count of the warps' tile-loop times
-    unsigned long long *dbg;
 };
 
 __device__ __forceinline__ void cp_async16(void *smem_dst, const void *gsrc, uint32_t src_bytes) {
@@ -875,8 +870,8 @@ __device__ __forceinline__ void lookup_leaf(const KeyTables *tab, float cx, floa
     *out = ls;
 }
 
-// WIDE: slot layout (VoxelSlot); DBG: per-phase time accounting of the tile loop (diagnostics build of the fused pass only)
-template <int MODE, bool WIDE, bool DBG = false>
+// WIDE: slot layout (VoxelSlot)
+template <int MODE, bool WIDE>
 __global__ void __launch_bounds__(VS_THREADS, 2) voxel_stream_kernel(const __grid_constant__ StreamArgs a, const __grid_constant__ KeyTables g_tab) {
     extern __shared__ __align__(128) unsigned char vs_smem_raw[];
     WarpStage *stages = reinterpret_cast<WarpStage *>(vs_smem_raw);
@@ -886,12 +881,6 @@ __global__ void __launch_bounds__(VS_THREADS, 2) voxel_stream_kernel(const __gri
     const unsigned lane = lane_id(), warp = threadIdx.x >> 5;
     const unsigned lt = lanemask_lt(), le = lt | (1u << lane);
     WarpStage &ws = stages[warp];
-    auto now_ns = [] {
-        unsigned long long t;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-        return t;
-    };
-    if (a.dbg && threadIdx.x == 0) atomicMin(a.dbg + 0, now_ns());
 
     if (MODE == VS_TABLES) {
         const uint32_t *src = reinterpret_cast<const uint32_t *>(&g_tab); // kernel parameter (constant bank) -> shared
@@ -912,20 +901,7 @@ __global__ void __launch_bounds__(VS_THREADS, 2) voxel_stream_kernel(const __gri
         build_relative_tables(tab, s_m0, a.res, a.kp.inv_cs, &a.header->pad[5]);
     }
     __syncthreads();
-    if (MODE == VS_FUSED && blockIdx.x == 0 && a.tables_out != nullptr) {
-        const uint32_t *src = reinterpret_cast<const uint32_t *>(&tab);
-        uint32_t *dst = reinterpret_cast<uint32_t *>(a.tables_out);
-        for (uint32_t i = threadIdx.x; i < sizeof(KeyTables) / 4; i += VS_THREADS) dst[i] = src[i];
-    }
 
-    __shared__ unsigned long long s_loop0[VS_WARPS]; // (diagnostics) kept out of the registers across the tile loop
-    __shared__ unsigned long long s_acc[DBG ? VS_WARPS : 1][8]; // DBG: ns per warp in [0] load wait [1] chunk box [2] run loop (with drains) [3] drains [4] join
-    if (DBG && lane == 0)
-        for (int i = 0; i < 8; i++) s_acc[warp][i] = 0;
-    if (a.dbg && lane == 0) {
-        s_loop0[warp] = now_ns();
-        if (warp == 0) atomicMax(a.dbg + 1, s_loop0[0]);
-    }
     const float inv = a.kp.inv;
     const uint32_t gw = blockIdx.x * VS_WARPS + warp, nw = gridDim.x * VS_WARPS;
     const Point16 *gpts = reinterpret_cast<const Point16 *>(a.pts);
@@ -941,10 +917,7 @@ __global__ void __launch_bounds__(VS_THREADS, 2) voxel_stream_kernel(const __gri
         dctx.header = a.header;
         dctx.slot_mask = a.slot_mask;
         dctx.claim_limit = a.claim_limit;
-        unsigned long long t0 = 0;
-        if (DBG) t0 = now_ns();
         seen_claims = drain_queue<WIDE>(qaddr, count, dctx, lane, seen_claims);
-        if (DBG && lane == 0) s_acc[warp][3] += now_ns() - t0;
     };
 
     // lane `lane` copies points c*32 + lane (c = 0..7) of a tile: 512 contiguous bytes per instruction.  Point i of the tile
@@ -968,18 +941,8 @@ __global__ void __launch_bounds__(VS_THREADS, 2) voxel_stream_kernel(const __gri
     for (; tile < a.ntiles; tile += nw, st ^= 1) {
         if (tile + nw < a.ntiles) issue(tile + nw, st ^ 1);
         cp_async_commit();
-        unsigned long long t_ph = 0;
-        if (DBG) t_ph = now_ns();
         cp_async_wait<1>();
         __syncwarp();
-        auto phase = [&](int i) { // DBG: time since the previous phase boundary goes to s_acc[warp][i]
-            if (DBG) {
-                const unsigned long long t = now_ns();
-                if (lane == 0) s_acc[warp][i] += t - t_ph;
-                t_ph = t;
-            }
-        };
-        phase(0);
 
         const uint32_t base = tile * VS_TILE;
         const uint32_t cnt = min((uint32_t)VS_TILE, a.n - base);
@@ -1032,7 +995,6 @@ __global__ void __launch_bounds__(VS_THREADS, 2) voxel_stream_kernel(const __gri
             }
         }
 
-        phase(1);
 #pragma unroll 2
         for (int j = 0; j < VS_L; j++) {
             if (qn > (uint32_t)(VS_QCAP - 32)) {
@@ -1105,7 +1067,6 @@ __global__ void __launch_bounds__(VS_THREADS, 2) voxel_stream_kernel(const __gri
             }
         }
 
-        phase(2);
         // ---- join the lanes' partial runs: a run that crosses lane boundaries is summed by a segmented scan ----
         const bool has_t = have;
         const bool single = has_t && nclosed == 0;          // the whole segment is one run
@@ -1143,19 +1104,9 @@ __global__ void __launch_bounds__(VS_THREADS, 2) voxel_stream_kernel(const __gri
         }
         qn += __popc(mh);
         __syncwarp();
-        phase(4);
     }
     cp_async_wait<0>();
-    if (DBG && a.dbg && lane == 0)
-        for (int i = 0; i < 5; i++) atomicAdd(a.dbg + 8 + i, s_acc[warp][i]);
-    if (a.dbg && lane == 0) {
-        const unsigned long long t = now_ns();
-        atomicMax(a.dbg + 2, t);
-        atomicAdd(a.dbg + 5, t - s_loop0[warp]);
-        atomicAdd(a.dbg + 6, 1ull);
-    }
     if (qn > 0) drain(qn);
-    if (a.dbg && lane == 0) atomicMax(a.dbg + 3, now_ns());
     if (bad) atomicOr(&a.header->error, 1u);
     if (amb) atomicOr(&a.header->pad[5], VS_FLAG_AMBIGUOUS);
 
@@ -1171,8 +1122,6 @@ __global__ void __launch_bounds__(VS_THREADS, 2) voxel_stream_kernel(const __gri
     __syncthreads();
     if (!s_last) return;
     __threadfence();
-    unsigned long long t_tail0;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_tail0));
     OctreeSeed none;
     none.valid = 0;
     none.depth = 0;
@@ -1221,10 +1170,6 @@ __global__ void __launch_bounds__(VS_THREADS, 2) voxel_stream_kernel(const __gri
         a.box_out->m0[0] = s_m0[0];
         a.box_out->m0[1] = s_m0[1];
         a.box_out->m0[2] = s_m0[2];
-        unsigned long long t_tail1;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_tail1));
-        a.box_out->tail_ns = t_tail1 - t_tail0;
-        if (a.dbg) a.dbg[4] = t_tail1;
     }
 }
 
@@ -1499,22 +1444,11 @@ void launch_stream(const StreamArgs &args, const KeyTables &tab, int dev, cudaSt
     static std::once_flag once[64];
     std::call_once(once[dev & 63], [&] {
         CWCU_CHECK(cudaFuncSetAttribute(voxel_stream_kernel<MODE, WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)VS_SMEM_BYTES));
+        // two blocks of 106 KB per SM need the largest carve-out
+        CWCU_CHECK(cudaFuncSetAttribute(voxel_stream_kernel<MODE, WIDE>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
     });
-    // two blocks of 106 KB per SM need the largest carve-out ($CWIPC_CUDA_DS_CARVEOUT, $CWIPC_CUDA_DS_BLOCKS_PER_SM: tuning only)
-    static const int carveout = [] { const char *e = getenv("CWIPC_CUDA_DS_CARVEOUT"); return e && *e ? atoi(e) : (int)cudaSharedmemCarveoutMaxShared; }();
-    static const size_t blocks_per_sm = [] { const char *e = getenv("CWIPC_CUDA_DS_BLOCKS_PER_SM"); return (size_t)std::max(1, std::min(2, e && *e ? atoi(e) : 2)); }();
-    tune_kernel(voxel_stream_kernel<MODE, WIDE>, carveout, true);
     // persistent warps: two blocks of eight warps per SM, every warp takes tiles gw, gw + nw, ...
-    static const size_t tiles_per_warp = [] { const char *e = getenv("CWIPC_CUDA_DS_TILES_PER_WARP"); return (size_t)std::max(1, e && *e ? atoi(e) : 1); }(); // tuning only
-    const unsigned grid = (unsigned)std::max<size_t>(1, std::min(div_up((size_t)args.ntiles, (size_t)VS_WARPS * tiles_per_warp), (size_t)sm_count(dev) * blocks_per_sm));
-    if constexpr (MODE == VS_FUSED) {
-        if (args.dbg) { // $CWIPC_CUDA_DEBUG_STREAM: the build with per-phase time accounting
-            CWCU_CHECK(cudaFuncSetAttribute(voxel_stream_kernel<MODE, WIDE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)VS_SMEM_BYTES));
-            tune_kernel(voxel_stream_kernel<MODE, WIDE, true>, carveout, true);
-            launch("voxel_stream_kernel", s, 16 * (size_t)args.n, [&] { voxel_stream_kernel<MODE, WIDE, true><<<grid, VS_THREADS, VS_SMEM_BYTES, s>>>(args, tab); });
-            return;
-        }
-    }
+    const unsigned grid = (unsigned)std::max<size_t>(1, std::min(div_up((size_t)args.ntiles, (size_t)VS_WARPS), (size_t)sm_count(dev) * 2));
     launch("voxel_stream_kernel", s, 16 * (size_t)args.n, [&] { voxel_stream_kernel<MODE, WIDE><<<grid, VS_THREADS, VS_SMEM_BYTES, s>>>(args, tab); });
 }
 
@@ -1625,24 +1559,7 @@ DownsampleRange downsample_impl(const cwipc_point *pts, size_t n, float cellsize
                 args.chunk_bbox = chunk_bbox.as<float>();
                 args.super_bbox = reinterpret_cast<uint32_t *>(wsp + ZW_HEADER_BYTES + capacity * sizeof(VoxelSlot));
                 args.box_out = box.as<OctreeBox>();
-                static const bool debug_stream = getenv("CWIPC_CUDA_DEBUG_STREAM") != nullptr;
-                Scratch dbg(debug_stream ? 16 * sizeof(unsigned long long) : 0, s);
-                if (debug_stream) {
-                    CWCU_CHECK(cudaMemsetAsync(dbg.p, 0, 16 * sizeof(unsigned long long), s));
-                    CWCU_CHECK(cudaMemsetAsync(dbg.p, 0xff, sizeof(unsigned long long), s));
-                    args.dbg = dbg.as<unsigned long long>();
-                }
                 wide ? launch_stream<VS_FUSED, true>(args, plan.tables, dev, s) : launch_stream<VS_FUSED, false>(args, plan.tables, dev, s);
-                if (debug_stream) {
-                    unsigned long long h[16];
-                    CWCU_CHECK(cudaMemcpyAsync(h, dbg.p, sizeof(h), cudaMemcpyDeviceToHost, s));
-                    stream_sync(s);
-                    if (h[6])
-                        fprintf(stderr, "  per warp (mean us): load wait %.1f, chunk box %.1f, run loop %.1f of which drains %.1f, join %.1f (join's own drains are in both)\n", (double)h[8] / h[6] / 1e3,
-                                (double)h[9] / h[6] / 1e3, (double)h[10] / h[6] / 1e3, (double)h[11] / h[6] / 1e3, (double)h[12] / h[6] / 1e3);
-                    fprintf(stderr, "voxel_stream_kernel n=%zu: tables %.1f us, tile loops end %.1f (mean per warp %.1f), drained %.1f, last block done %.1f us after the first block started\n", n,
-                            (double)(h[1] - h[0]) / 1e3, (double)(h[2] - h[0]) / 1e3, h[6] ? (double)h[5] / (double)h[6] / 1e3 : 0.0, (double)(h[3] - h[0]) / 1e3, (double)(h[4] - h[0]) / 1e3);
-                }
             } else {
                 args.kp = plan.kp;
                 if (!octree_split) wide ? launch_stream<VS_LINEAR, true>(args, plan.tables, dev, s) : launch_stream<VS_LINEAR, false>(args, plan.tables, dev, s);
@@ -1679,7 +1596,6 @@ DownsampleRange downsample_impl(const cwipc_point *pts, size_t n, float cellsize
             };
             if (fused) {
                 ob = h->box;
-                if (getenv("CWIPC_CUDA_DEBUG_TAIL")) fprintf(stderr, "voxel_stream_kernel: last block spent %.1f us on the octree replay (depth %d, shift %d %d %d, flags %u, fallback %d, error %d)\n", (double)ob.tail_ns / 1e3, ob.depth, ob.shift[0], ob.shift[1], ob.shift[2], flags, ob.fallback, ob.error);
                 const bool redo = (flags & VS_FLAG_AMBIGUOUS) != 0 || ob.fallback != 0 || ob.error != 0 || ob.depth > MAX_OCTREE_DEPTH;
                 if (redo) { // a point on a leaf face, or an extent the relative keys do not cover: the two-pass path decides
                     clear_table();
@@ -1719,8 +1635,6 @@ DownsampleRange downsample_impl(const cwipc_point *pts, size_t n, float cellsize
                 return result;
             }
             Scratch words(v * sizeof(uint64_t), s), other(v * sizeof(uint64_t), s);
-            tune_kernel(voxel_words_kernel, CHAIN_CARVEOUT);
-            tune_kernel(wide ? voxel_emit_kernel<true> : voxel_emit_kernel<false>, CHAIN_CARVEOUT);
             launch("voxel_words_kernel", s, 16 * v, [&] {
                 voxel_words_kernel<<<(unsigned)std::max<size_t>(1, div_up(v, 256)), 256, 0, s>>>(list_keys.as<uint64_t>(), (uint32_t)v, cbits, fused ? 1 : 0, ob.shift[0], ob.shift[1], ob.shift[2],
                                                                                                  depth, words.as<uint64_t>(), header);

@@ -1274,8 +1274,8 @@ unsigned stream_grid(size_t n, int dev) {
     return (unsigned)std::max<size_t>(1, std::min(div_up(n, 256), (size_t)sm_count(dev) * 8));
 }
 
-// Tunables of the pitch heuristic (results never depend on them).  CWIPC_CUDA_KNN_PITCH scales the
-// pitch relative to the expected k-neighbour radius; CWIPC_CUDA_KNN_RC is the cover radius in pitches.
+// Test hooks of the kNN index (results never depend on them): CWIPC_CUDA_KNN_PITCH scales the pitch relative to the
+// expected k-neighbour radius, the others move work between the main pass, the second scan and the tree search.
 float env_float(const char *name, float dflt, float lo, float hi) {
     const char *e = getenv(name);
     if (!e || !*e) return dflt;
@@ -1289,10 +1289,10 @@ struct GridPlan {
 };
 
 // Pitch ~ a fraction of the expected k-neighbour radius of a surface sampled at `spacing`; the main
-// pass covers rc pitches around each query group.  The dense tables bound the number of cells.
+// pass covers rc = 1 pitch around each query group.  The dense tables bound the number of cells.
 GridPlan choose_grid(const float gmin[3], const float gmax[3], size_t n, int k, float hint_spacing, int bands = 1) {
     static const float pitch_factor = env_float("CWIPC_CUDA_KNN_PITCH", 1.0f, 0.05f, 20.f);
-    static const float rc = env_float("CWIPC_CUDA_KNN_RC", 1.0f, 0.25f, 1.0f);
+    constexpr float rc = 1.0f;
     static const float rc_far = env_float("CWIPC_CUDA_KNN_RC_FAR", 2.0f, 0.f, 8.f); // 0: no second scan
     GridPlan plan;
     GridParams &gp = plan.gp;
@@ -1318,9 +1318,7 @@ GridPlan choose_grid(const float gmin[3], const float gmax[3], size_t n, int k, 
     // dense tables: 9.1 bytes per cell over all levels.  16 cells per point (146 MB at 1 M points), at most 2^27 cells
     // (1.2 GB, reached from 8 M points on).  Round 1 allowed 4 per point / 2^25: an 8 M-point cloud and the per-tile bands of a
     // 1 M-point cloud then got a pitch 1.6-2x the wanted one, i.e. 2.5-4x the candidates per query (8 M raw: 9.3 -> 6.5 ms).
-    static const float cells_per_point = env_float("CWIPC_CUDA_KNN_CELLS_PER_POINT", 16.f, 0.25f, 1024.f);
-    static const float max_cells_log2 = env_float("CWIPC_CUDA_KNN_MAX_CELLS_LOG2", 27.f, 16.f, 30.f);
-    const double cell_cap = std::min(std::max((double)cells_per_point * (double)n, 65536.0), std::ldexp(1.0, (int)max_cells_log2)) / (bands > 1 ? 2.0 * (double)bands : 1.0);
+    const double cell_cap = std::min(std::max(16.0 * (double)n, 65536.0), std::ldexp(1.0, 27)) / (bands > 1 ? 2.0 * (double)bands : 1.0);
     while (true) {
         const double cells = (std::floor(ext[0] / h) + 2) * (std::floor(ext[1] / h) + 2) * (std::floor(ext[2] / h) + 2);
         if (longest / h < (double)((1 << max_axis_bits) - 1) && cells <= cell_cap) break;
@@ -1356,11 +1354,8 @@ GridPlan choose_grid(const float gmin[3], const float gmax[3], size_t n, int k, 
     return plan;
 }
 
-uint32_t far_leaf_points() {
-    // nodes with at most this many points are scanned directly instead of being expanded
-    static const uint32_t v = (uint32_t)env_float("CWIPC_CUDA_KNN_LEAF", 128.f, 1.f, 65536.f);
-    return v;
-}
+// tree search: nodes with at most this many points are scanned directly instead of being expanded
+constexpr uint32_t FAR_LEAF_POINTS = 128;
 
 template <int KCAP>
 void run_knn(const cwipc_point *spts, const uint64_t *sorted, size_t n, const GridParams &gp, int k, const uint2 *table, float *d_dist, float *d_kth, size_t nquery,
@@ -1374,7 +1369,6 @@ void run_knn(const cwipc_point *spts, const uint64_t *sorted, size_t n, const Gr
     });
     const size_t nitems = div_up(n, (size_t)32);
     const unsigned grid = (unsigned)std::max<size_t>(1, std::min(div_up(nitems, (size_t)KT_WARPS), (size_t)sm_count(dev) * KT_BLOCKS_PER_SM));
-    tune_kernel(knn_tile_kernel<KCAP>, CHAIN_CARVEOUT);
     launch("knn_tile_kernel", s, 28 * (size_t)n, [&] {
         knn_tile_kernel<KCAP><<<grid, KT_THREADS, smem, s>>>(spts, sorted, (uint32_t)n, gp, kk, k, table, d_dist, d_kth, (uint32_t)nquery, far_list, far_count);
     });
@@ -1385,21 +1379,18 @@ void run_knn(const cwipc_point *spts, const uint64_t *sorted, size_t n, const Gr
     // queue) its per-group latency is not bought back.  Measured: 47 K-point frames -2..-5 % throughput, 1 M raw points -23 % time.
     static const float second_from_n = env_float("CWIPC_CUDA_KNN_SECOND_FROM_N", 262144.f, 0.f, 4.0e9f);
     if (gp.rc_far > gp.rc && (double)std::min(nquery, n) >= (double)second_from_n) {
-        static const float share = env_float("CWIPC_CUDA_KNN_SECOND_SHARE", 0.f, 0.f, 1.f);
-        second_from = (uint32_t)std::max(1.0, std::ceil((double)share * (double)std::min(nquery, n)));
+        second_from = 1;
         // open queries with a bound within rc_far pitches: scanned once more, group by group; the rest goes to the second list
-        tune_kernel(knn_second_kernel<KCAP>, CHAIN_CARVEOUT);
         launch("knn_second_kernel", s, (size_t)0, [&] {
             knn_second_kernel<KCAP><<<(unsigned)sm_count(dev) * KT_BLOCKS_PER_SM, KT_THREADS, smem, s>>>(spts, sorted, gp, kk, k, table, d_dist, d_kth, far_list, far_count, second_from,
                                                                                                          far_list + (n + 64), far_count + 1);
         });
     }
     constexpr int KPL = KCAP > 32 ? 2 : 1;
-    tune_kernel(knn_far_kernel<KPL>, CHAIN_CARVEOUT);
     launch("knn_far_kernel", s, (size_t)0, [&] {
         // CWIPC_CUDA_KNN_FAR_START=0 (tests / A-B only): every search starts at the root with no bound, as in round 1
         static const bool far_start_on = env_float("CWIPC_CUDA_KNN_FAR_START", 1.f, 0.f, 1.f) != 0.f;
-        knn_far_kernel<KPL><<<(unsigned)sm_count(dev) * 8, KF_THREADS, 0, s>>>(spts, sorted, (uint32_t)n, gp, kk, k, table, d_dist, d_kth, far_list, far_count, second_from, far_leaf_points(),
+        knn_far_kernel<KPL><<<(unsigned)sm_count(dev) * 8, KF_THREADS, 0, s>>>(spts, sorted, (uint32_t)n, gp, kk, k, table, d_dist, d_kth, far_list, far_count, second_from, FAR_LEAF_POINTS,
                                                                                far_start_on);
     });
 }
@@ -1414,7 +1405,7 @@ void run_knn_wide(const cwipc_point *spts, const uint64_t *sorted, size_t n, con
     });
     launch("knn_far_kernel", s, (size_t)0, [&] {
         static const bool far_start_on = env_float("CWIPC_CUDA_KNN_FAR_START", 1.f, 0.f, 1.f) != 0.f;
-        knn_far_kernel<KPL><<<(unsigned)sm_count(dev) * 8, KF_THREADS, 0, s>>>(spts, sorted, (uint32_t)n, gp, k + 1, k, table, d_dist, d_kth, far_list, far_count, 0xffffffffu, far_leaf_points(),
+        knn_far_kernel<KPL><<<(unsigned)sm_count(dev) * 8, KF_THREADS, 0, s>>>(spts, sorted, (uint32_t)n, gp, k + 1, k, table, d_dist, d_kth, far_list, far_count, 0xffffffffu, FAR_LEAF_POINTS,
                                                                                far_start_on);
     });
 }
@@ -1455,8 +1446,6 @@ void build_index(KnnIndex &ix, const cwipc_point *in, size_t n, int k, float hin
     ix.spts = Scratch(n * sizeof(cwipc_point), s);
     ix.table = Scratch((plan.table_entries + 2) * sizeof(uint2), s);
     ix.far_count = reinterpret_cast<uint32_t *>(ix.table.as<uint2>() + plan.table_entries);
-    tune_kernel(knn_keygen_kernel, CHAIN_CARVEOUT);
-    tune_kernel(knn_layout_kernel, CHAIN_CARVEOUT);
     launch("knn_keygen_kernel", s, 24 * (size_t)n, [&] {
         knn_keygen_kernel<<<stream_grid(std::max(n, plan.table_entries / 4), dev), 256, 0, s>>>(in, (uint32_t)n, gp, band_lut, ix.keys_a.as<uint64_t>(), ix.table.as<uint2>(),
                                                                                                  (uint32_t)(plan.table_entries + 2));
@@ -1708,7 +1697,7 @@ void knn_lists(const cwipc_point *in, size_t n, const cwipc_point *d_queries, co
     launch("knn_list_kernel", s, (size_t)0, [&] {
         auto go = [&](auto kpl) {
             knn_list_kernel<decltype(kpl)::value><<<grid, KF_THREADS, 0, s>>>(ix.spts.as<cwipc_point>(), (uint32_t)n, ix.gp, kk, ix.table.as<uint2>(), d_queries, d_limits, (uint32_t)nq, d_lists,
-                                                                              far_leaf_points());
+                                                                              FAR_LEAF_POINTS);
         };
         if (kk <= 32) go(std::integral_constant<int, 1>{});
         else if (kk <= 64) go(std::integral_constant<int, 2>{});
@@ -1833,7 +1822,6 @@ size_t remove_outliers_points(const cwipc_point *in, size_t n, cwipc_point *out,
     Scratch partial((2 * ST_BLOCKS + 1) * sizeof(double), s);
     uint32_t *counter = static_cast<uint32_t *>(thread_zeroed(dev, ZW_HEADER_BYTES, s)) + 6; // word 6 of the zeroed workspace header
     double *d_thr = partial.as<double>() + 2 * ST_BLOCKS;
-    tune_kernel(stats_threshold_kernel, CHAIN_CARVEOUT);
     launch("stats_kernel", s, 4 * (size_t)n, [&] {
         stats_threshold_kernel<<<ST_BLOCKS, ST_THREADS, 0, s>>>(dist.as<float>(), (uint32_t)n, partial.as<double>(), counter, (double)stddev_mul, d_thr);
     });
@@ -1934,7 +1922,7 @@ void IcpMatcher::evaluate(const cwipc_point *source, size_t ns, const double mot
     double *partial = m->partial.as<double>(), *d_out = partial + (size_t)m->max_warps * ICP_NSUMS;
     launch("icp_match_kernel", m->s, 16 * ns, [&] {
         icp_match_kernel<<<grid, ICP_THREADS, 0, m->s>>>(source, (uint32_t)ns, m->target, (uint32_t)m->nt, m->ix.spts.as<cwipc_point>(), m->ix.sorted, m->ix.gp, m->ix.table.as<uint2>(),
-                                                        far_leaf_points(), ip, partial);
+                                                        FAR_LEAF_POINTS, ip, partial);
     });
     launch("icp_reduce_kernel", m->s, 8 * (size_t)nwarps * ICP_NSUMS, [&] { icp_reduce_kernel<<<1, ICP_NSUMS * 32, 0, m->s>>>(partial, nwarps, d_out); });
     double *h = static_cast<double *>(thread_pinned(ICP_NSUMS * sizeof(double)));

@@ -161,7 +161,6 @@ size_t run_compact(const cwipc_point *in, size_t n, cwipc_point *out, Pred pred,
     uint32_t *ticket = words;
     uint32_t *d_total = chain_total ? chain_total : words + 1;
     uint64_t *status = reinterpret_cast<uint64_t *>(words + 4);
-    tune_kernel(compact_kernel<Pred>, CHAIN_CARVEOUT);
     launch("compact_kernel", s, pred_bytes * (size_t)n, [&] {
         compact_kernel<Pred><<<(unsigned)ntiles, CP_THREADS, 0, s>>>(in, (uint32_t)n, out, pred, ticket, status, d_total, done, chain_base);
     });

@@ -497,7 +497,6 @@ bool launch_cluster_sort(const uint64_t *in, uint64_t *out, size_t n, int begin_
         if (e != cudaSuccess) (void)cudaGetLastError();
     });
     if (ok[dev & 63] != 1) return false;
-    tune_kernel(radix_cluster_kernel<IPT>, CHAIN_CARVEOUT);
     const size_t cap = (size_t)RC_THREADS * IPT;
     const unsigned nctas = (unsigned)div_up(n, cap);
     cudaLaunchConfig_t cfg = {};

@@ -531,31 +531,6 @@ void copy_to_host(void *dst, const void *src, size_t bytes, cudaStream_t s) {
     ring.st.next = (unsigned)((base + nchunks) % SLOTS);
 }
 
-void tune_kernel(const void *func, int dflt, bool fixed) {
-    static const int forced = [] {
-        const char *e = getenv("CWIPC_CUDA_CARVEOUT");
-        return (e && *e) ? atoi(e) : -2;
-    }();
-    const int want = (!fixed && forced >= -1) ? forced : dflt;
-    if (want < -1) return;
-    int dev = 0;
-    CWCU_CHECK(cudaGetDevice(&dev));
-    // applied once per (kernel, device); the per-thread list keeps the steady-state launch path free of locks
-    thread_local std::vector<std::pair<const void *, int>> seen;
-    for (const auto &e : seen)
-        if (e.first == func && e.second == dev) return;
-    seen.emplace_back(func, dev);
-    static std::mutex mu;
-    static std::map<std::pair<const void *, int>, int> done;
-    {
-        std::lock_guard<std::mutex> lk(mu);
-        auto it = done.find({func, dev});
-        if (it != done.end() && it->second == want) return;
-        done[{func, dev}] = want;
-    }
-    CWCU_CHECK(cudaFuncSetAttribute(func, cudaFuncAttributePreferredSharedMemoryCarveout, want));
-}
-
 bool is_pinned_host(const void *p) {
     if (!p) return false;
     cudaPointerAttributes attr;

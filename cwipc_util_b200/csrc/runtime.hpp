@@ -195,15 +195,6 @@ inline void launch(const char *name, cudaStream_t s, size_t algorithmic_bytes, F
     f();
     check_launch(name);
 }
-// Shared-memory carve-out preference of a kernel (a percentage of the SM's shared memory, cudaSharedmemCarveoutMaxShared
-// = 100, or -1 = the driver's choice), applied once per kernel and device.  Kernels of several streams can only share an
-// SM when its L1 / shared-memory split suits them all, so the kernels of the frame chain state a common preference;
-// `dflt` < -1 leaves the kernel alone.  $CWIPC_CUDA_CARVEOUT overrides `dflt` for every kernel (tuning only).
-constexpr int CHAIN_CARVEOUT = -2; // default preference of the frame chain's kernels (-2: none stated)
-void tune_kernel(const void *func, int dflt, bool fixed = false); // fixed: $CWIPC_CUDA_CARVEOUT does not apply
-template <class K>
-inline void tune_kernel(K *kernel, int dflt, bool fixed = false) { tune_kernel(reinterpret_cast<const void *>(kernel), dflt, fixed); }
-
 // bytes that are only known after a readback (e.g. survivors written by a compaction)
 void profile_add_bytes(const char *name, size_t bytes);
 

@@ -1,8 +1,8 @@
 #!/usr/bin/env python
-"""Quick A/B of the bench's `value` (device-resident frame chain, 15 host threads on one GPU) for library tuning knobs
-that are read from the environment at load time: one process per variant, a fraction of bench.py's run time.
+"""Quick A/B of the bench's `value` (device-resident frame chain, 15 host threads on one GPU) for another build of the
+library or a setting read from the environment at load time: one process per variant, a fraction of bench.py's run time.
 
-    CWIPC_CUDA_CARVEOUT=100 python scripts/ab_value.py [--frames 60] [--steps 6] [--pageable] [--profile]
+    CWIPC_CUDA_LIBRARY=/path/to/libcwipc_util_cuda.so python scripts/ab_value.py [--frames 60] [--steps 6] [--pageable] [--profile]
 
 Prints one JSON line: value (Mpoints/s), optionally the pageable end-to-end figure and the per-kernel times of a
 single-stream replay.  Diagnostics only; the numbers of record come from bench.py.

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """cwipc_remove_outliers timing on the bench's own frames (1M points -> downsample 0.01 -> ~47K voxels) and on raw clouds,
-CUDA-event timed, per-kernel profile.  Tunables come from the environment (CWIPC_CUDA_KNN_PITCH / _RC / _LEAF).
+CUDA-event timed, per-kernel profile.  The kNN index settings come from the environment (CWIPC_CUDA_KNN_PITCH / _RC_FAR).
 
     python scripts/bench_sor.py [--reps 20]
 """

@@ -17,7 +17,6 @@ def run(path):
     else: os.environ.pop("CWIPC_CUDA_DS_PATH", None)
     pc = cw.cwipc_from_numpy_array(whole, 7); pc._set_cellsize(cs0)
     return cw.cwipc_downsample(pc, 0.005).get_numpy_array().copy()
-os.environ["CWIPC_CUDA_DEBUG_TAIL"] = "1"
 res = {p or "fused": run(p) for p in (None, "twopass", "generic")}
 for name, got in res.items():
     same_len = len(got) == len(want)
