@@ -46,13 +46,6 @@ constexpr int WL_BITS = 19;      // 72^3 = 373248 < 2^19
 constexpr int MAX_OCTREE_DEPTH = 14;
 constexpr int REL_BIAS = 16384;  // leaf index relative to the first point's box, biased into 15 bits
 
-struct OctreeSeed { // box state to continue from (a cloud partitioned over several GPUs is replayed part by part)
-    double min[3];
-    double max[3];
-    int depth;
-    int valid; // 0: start from this cloud's first point
-};
-
 struct OctreeBox {
     double min[3];
     double max[3];
@@ -145,9 +138,11 @@ __device__ __forceinline__ float dec_float(uint32_t e) { return __uint_as_float(
 
 // Called by a whole block of THREADS threads.  chunk_bbox holds one box per CHUNK consecutive points; super_bbox (or
 // nullptr) one encoded box per SUPER chunks, searched first (with 256-point chunks an 8 M-point cloud has 31 K of them).
+// The replay continues from `seed` (a cloud partitioned over several GPUs is replayed part by part); seed.valid == 0: it
+// starts from this cloud's first point.
 template <int THREADS, int CHUNK, int SUPER>
 __device__ __forceinline__ void octree_box_block(const cwipc_point *__restrict__ pts, uint32_t n, const float *chunk_bbox, uint32_t nchunks, uint32_t *super_bbox, double res,
-                                                  int do_octree, const OctreeSeed &seed, OctreeBox *__restrict__ out) {
+                                                  int do_octree, const cwipc_cuda_octree_state &seed, OctreeBox *__restrict__ out) {
     __shared__ float s_red[6][32];
     __shared__ double s_min[3], s_max[3];
     __shared__ int s_depth, s_error;
@@ -321,7 +316,7 @@ __device__ __forceinline__ void octree_box_block(const cwipc_point *__restrict__
 // One launch: every block boxes its 4096-point chunk; the block that finishes last reduces the chunk boxes
 // and replays the octree growth (the classic "last block" pattern: fence, ticket, fence).
 __global__ void __launch_bounds__(BB_THREADS) bbox_octree_kernel(const cwipc_point *__restrict__ pts, uint32_t n, float *chunk_bbox, uint32_t nchunks, double res, int do_octree,
-                                                                OctreeSeed seed, uint32_t *__restrict__ done_counter, OctreeBox *__restrict__ out) {
+                                                                cwipc_cuda_octree_state seed, uint32_t *__restrict__ done_counter, OctreeBox *__restrict__ out) {
     __shared__ bool s_last;
     chunk_bbox_block(pts, n, chunk_bbox);
     __threadfence();
@@ -1122,11 +1117,7 @@ __global__ void __launch_bounds__(VS_THREADS, 2) voxel_stream_kernel(const __gri
     __syncthreads();
     if (!s_last) return;
     __threadfence();
-    OctreeSeed none;
-    none.valid = 0;
-    none.depth = 0;
-    for (int ax = 0; ax < 3; ax++) none.min[ax] = none.max[ax] = 0.0;
-    octree_box_block<VS_THREADS, VS_TILE, VS_SUPER>(a.pts, a.n, a.chunk_bbox, a.ntiles, a.super_bbox, a.res, 1, none, a.box_out);
+    octree_box_block<VS_THREADS, VS_TILE, VS_SUPER>(a.pts, a.n, a.chunk_bbox, a.ntiles, a.super_bbox, a.res, 1, cwipc_cuda_octree_state{}, a.box_out);
     __syncthreads();
     // shift of the leaf indices: (m0 - final min) / res must be a whole number (the box only ever moves by multiples of res),
     // and every table threshold inside the cloud's extent must be a threshold of the FINAL box too
@@ -1289,15 +1280,6 @@ __global__ void __launch_bounds__(256) voxel_clear_kernel(uint32_t v, const uint
     raw[3] = zero;
 }
 
-int bit_length(uint64_t v) {
-    int b = 0;
-    while (v) {
-        b++;
-        v >>= 1;
-    }
-    return b;
-}
-
 // the "last block" ticket of bbox_octree_kernel / voxel_stream_kernel: a word of the thread's zeroed workspace header (pad[0])
 uint32_t *bbox_counter(int dev, cudaStream_t s) {
     TableHeader *h = static_cast<TableHeader *>(thread_zeroed(dev, ZW_HEADER_BYTES, s));
@@ -1311,8 +1293,6 @@ struct Plan {
     }
     KeyParams kp;
     int keybits = 0;
-    bool failed = false;
-    std::string error;
     float gmin[3] = {0, 0, 0}, gmax[3] = {0, 0, 0};
     bool use_tables = false;
     KeyTables tables;
@@ -1320,7 +1300,7 @@ struct Plan {
 
 // One launch + one readback: bounding box of the points and the octree box after inserting them in order
 // (continuing from `seed` when it is valid).
-OctreeBox measure_box(const cwipc_point *pts, size_t n, float cellsize, bool octree_split, const OctreeSeed &seed, int dev, cudaStream_t s) {
+OctreeBox measure_box(const cwipc_point *pts, size_t n, float cellsize, bool octree_split, int dev, cudaStream_t s, const cwipc_cuda_octree_state &seed = {}) {
     const uint32_t nchunks = (uint32_t)div_up(n, BB_CHUNK);
     Scratch chunk_bbox((size_t)nchunks * 6 * sizeof(float), s);
     Scratch box(sizeof(OctreeBox), s);
@@ -1376,35 +1356,33 @@ bool build_key_tables(const KeyParams &kp, const OctreeBox &ob, KeyTables &tab) 
     return true;
 }
 
-// Key layout and limits from the measured (or supplied) boxes.
-Plan derive_plan(const OctreeBox &ob, size_t n, float cellsize, bool octree_split) {
-    Plan plan;
-    const double res = (double)(64 * cellsize);
-    KeyParams &kp = plan.kp;
+// The key parameters that depend on the voxel size alone: all the fused pass needs (its idxbits stays 0).
+void fill_key_params(KeyParams &kp, float cellsize, bool octree_split) {
     memset(&kp, 0, sizeof(kp));
     kp.octree = octree_split ? 1 : 0;
     kp.inv = 1.0f / cellsize;
-    kp.idxbits = std::max(1, bit_length((uint64_t)n - 1));
-    kp.res = res;
-    kp.inv_res = 1.0 / res;
+    kp.res = (double)(64 * cellsize);
+    kp.inv_res = 1.0 / kp.res;
     kp.inv_cs = 1.0 / (double)cellsize;
+}
+
+// Key layout and limits from the measured (or supplied) boxes.  An input that cannot be downsampled throws.
+Plan derive_plan(const OctreeBox &ob, size_t n, float cellsize, bool octree_split) {
+    Plan plan;
+    KeyParams &kp = plan.kp;
+    fill_key_params(kp, cellsize, octree_split);
+    kp.idxbits = std::max(1, bit_length((uint64_t)n - 1));
     float maxabs = 0.f;
     for (int a = 0; a < 3; a++) {
         maxabs = std::max(maxabs, std::max(std::fabs(ob.gmin[a]), std::fabs(ob.gmax[a])));
         plan.gmin[a] = ob.gmin[a];
         plan.gmax[a] = ob.gmax[a];
     }
-    if (!std::isfinite(maxabs)) {
-        plan.failed = true;
-        plan.error = "pointcloud contains non-finite coordinates";
-        return plan;
-    }
+    if (!std::isfinite(maxabs)) throw CudaError{cudaErrorInvalidValue, "pointcloud contains non-finite coordinates"};
     if (octree_split) {
-        if (ob.error || ob.depth > MAX_OCTREE_DEPTH) {
-            plan.failed = true;
-            plan.error = "pointcloud extent too large for voxel size (octree depth " + std::to_string(ob.depth) + " > " + std::to_string(MAX_OCTREE_DEPTH) + ")";
-            return plan;
-        }
+        if (ob.error || ob.depth > MAX_OCTREE_DEPTH)
+            throw CudaError{cudaErrorInvalidValue,
+                            "pointcloud extent too large for voxel size (octree depth " + std::to_string(ob.depth) + " > " + std::to_string(MAX_OCTREE_DEPTH) + ")"};
         for (int a = 0; a < 3; a++) kp.omin[a] = ob.min[a];
         kp.depth = ob.depth;
         plan.keybits = WL_BITS + 3 * ob.depth;
@@ -1415,12 +1393,8 @@ Plan derive_plan(const OctreeBox &ob, size_t n, float cellsize, bool octree_spli
         const int64_t dx = (int64_t)((ob.gmax[0] - ob.gmin[0]) * inv) + 1;
         const int64_t dy = (int64_t)((ob.gmax[1] - ob.gmin[1]) * inv) + 1;
         const int64_t dz = (int64_t)((ob.gmax[2] - ob.gmin[2]) * inv) + 1;
-        if (dx * dy * dz > (int64_t)INT32_MAX) {
-            // PCL copies the input and leaves its leaf layout empty; cwipc's tile pass then throws out_of_range
-            plan.failed = true;
-            plan.error = "VoxelGrid std exception: leaf size is too small for the input dataset (integer indices would overflow)";
-            return plan;
-        }
+        if (dx * dy * dz > (int64_t)INT32_MAX) // PCL copies the input and leaves its leaf layout empty; cwipc's tile pass then throws out_of_range
+            throw CudaError{cudaErrorInvalidValue, "VoxelGrid std exception: leaf size is too small for the input dataset (integer indices would overflow)"};
         uint64_t cells = 1;
         for (int a = 0; a < 3; a++) {
             kp.minb[a] = (int)std::floor(ob.gmin[a] * inv);
@@ -1431,10 +1405,6 @@ Plan derive_plan(const OctreeBox &ob, size_t n, float cellsize, bool octree_spli
         plan.keybits = std::max(1, bit_length(cells - 1));
     }
     return plan;
-}
-
-unsigned stream_grid(size_t n, int dev) {
-    return (unsigned)std::max<size_t>(1, std::min(div_up(n, 256), (size_t)sm_count(dev) * 8));
 }
 
 constexpr size_t VS_SMEM_BYTES = sizeof(WarpStage) * VS_WARPS + sizeof(KeyTables);
@@ -1463,28 +1433,22 @@ void table_size(size_t n, bool full, size_t &claim_limit, size_t &capacity) {
 } // namespace
 
 namespace {
-// pts[0..n) -> voxels.  `dest(v)` is called once, when the voxel count v is known, and returns room for them.
-DownsampleRange downsample_impl(const cwipc_point *pts, size_t n, float cellsize, bool octree_split, const OctreeBox *external, uint64_t total_points,
+// pts[0..n) -> voxels.  `dest(v)` is called once, when the voxel count v is known, and returns room for them.  `planned`
+// and `bounds` (both or neither): the octree box and the bounding box of the whole cloud pts belongs to.  An input that
+// cannot be downsampled throws.
+DownsampleRange downsample_impl(const cwipc_point *pts, size_t n, float cellsize, bool octree_split, const cwipc_cuda_octree_state *planned, const float *bounds,
                                 const std::function<cwipc_point *(size_t)> &dest, int dev, cudaStream_t s) {
     DownsampleRange result;
     if (n == 0) {
-        if (octree_split) {
-            // no octree leaves: an empty, non-NULL cloud (python/test_cwipc_util.py:589-594)
-            (void)dest(0);
-        } else {
-            result.failed = true; // ref: src/cwipc_filters.cpp:58-62
-            result.error = "VoxelGrid filter produced empty pointcloud";
-        }
+        if (!octree_split) throw CudaError{cudaErrorInvalidValue, "VoxelGrid filter produced empty pointcloud"}; // ref: src/cwipc_filters.cpp:58-62
+        // no octree leaves: an empty, non-NULL cloud (python/test_cwipc_util.py:589-594)
+        (void)dest(0);
         return result;
     }
-    if (!(cellsize > 0.f) || !std::isfinite(cellsize)) {
-        result.failed = true;
-        result.error = "invalid voxel size " + std::to_string(cellsize);
-        return result;
-    }
+    if (!(cellsize > 0.f) || !std::isfinite(cellsize)) throw CudaError{cudaErrorInvalidValue, "invalid voxel size " + std::to_string(cellsize)};
     // fixed-point scale of the voxel-relative offsets: |offset| <= cellsize (1 + eps), n of them must fit 2^62 (a part of a
     // partitioned cloud uses the count of the whole cloud: same scale, same rounding as the one-GPU call)
-    int shift = 61 - bit_length(std::max((uint64_t)n, total_points));
+    int shift = 61 - bit_length(std::max((uint64_t)n, planned ? planned->points : 0));
     {
         int e;
         (void)std::frexp(cellsize, &e); // cellsize < 2^e
@@ -1501,29 +1465,30 @@ DownsampleRange downsample_impl(const cwipc_point *pts, size_t n, float cellsize
     const bool force_twopass = force && (!strcmp(force, "twopass") || !strcmp(force, "generic"));
     const bool force_generic = force && !strcmp(force, "generic");
     const bool force_small = force && !strcmp(force, "smalltable");
-    bool fused = octree_split && external == nullptr && !force_twopass;
+    bool fused = octree_split && !planned && !force_twopass;
     bool full_table = false;
     const bool wide = n > VS_NARROW_MAX_POINTS; // slot layout (VoxelSlot)
     OctreeBox ob;
     memset(&ob, 0, sizeof(ob));
+    if (planned) {
+        for (int a = 0; a < 3; a++) {
+            ob.min[a] = planned->min[a];
+            ob.max[a] = planned->max[a];
+            ob.gmin[a] = bounds[a];
+            ob.gmax[a] = bounds[3 + a];
+        }
+        ob.depth = planned->depth;
+    }
     Plan plan;
     bool have_plan = false;
-    if (external) ob = *external;
+    // an input error the stream pass finds; the table is cleared before it is thrown, so the workspace stays valid
+    std::string input_error;
 
     for (int attempt = 0; attempt < 4; attempt++) {
         if (!fused && !have_plan) {
-            if (!external) {
-                OctreeSeed none;
-                memset(&none, 0, sizeof(none));
-                ob = measure_box(pts, n, cellsize, octree_split, none, dev, s);
-            }
+            if (!planned) ob = measure_box(pts, n, cellsize, octree_split, dev, s);
             plan = derive_plan(ob, n, cellsize, octree_split);
             have_plan = true;
-            if (plan.failed) {
-                result.failed = true;
-                result.error = plan.error;
-                return result;
-            }
         }
         size_t claim_limit, capacity;
         table_size(n, full_table, claim_limit, capacity);
@@ -1550,12 +1515,7 @@ DownsampleRange downsample_impl(const cwipc_point *pts, size_t n, float cellsize
             args.header = header;
             args.res = (double)(64 * cellsize);
             if (fused) {
-                memset(&args.kp, 0, sizeof(args.kp));
-                args.kp.octree = 1;
-                args.kp.inv = 1.0f / cellsize;
-                args.kp.res = args.res;
-                args.kp.inv_res = 1.0 / args.res;
-                args.kp.inv_cs = 1.0 / (double)cellsize;
+                fill_key_params(args.kp, cellsize, true);
                 args.chunk_bbox = chunk_bbox.as<float>();
                 args.super_bbox = reinterpret_cast<uint32_t *>(wsp + ZW_HEADER_BYTES + capacity * sizeof(VoxelSlot));
                 args.box_out = box.as<OctreeBox>();
@@ -1605,9 +1565,8 @@ DownsampleRange downsample_impl(const cwipc_point *pts, size_t n, float cellsize
             }
             if (err != 0) {
                 clear_table();
-                result.failed = true;
-                result.error = "point coordinates out of range for voxel size " + std::to_string(cellsize) + " (|x/voxelsize| must stay below 2^22)";
-                return result;
+                input_error = "point coordinates out of range for voxel size " + std::to_string(cellsize) + " (|x/voxelsize| must stay below 2^22)";
+                break;
             }
             if (flags & VS_FLAG_OVERFLOW) {
                 clear_table();
@@ -1630,9 +1589,8 @@ DownsampleRange downsample_impl(const cwipc_point *pts, size_t n, float cellsize
             const int cbits = std::max(1, bit_length((uint64_t)v - 1));
             if (keybits + cbits > 64) {
                 clear_table();
-                result.failed = true;
-                result.error = "pointcloud too large for 64-bit voxel sort words (" + std::to_string(keybits) + " key bits + " + std::to_string(cbits) + " index bits)";
-                return result;
+                input_error = "pointcloud too large for 64-bit voxel sort words (" + std::to_string(keybits) + " key bits + " + std::to_string(cbits) + " index bits)";
+                break;
             }
             Scratch words(v * sizeof(uint64_t), s), other(v * sizeof(uint64_t), s);
             launch("voxel_words_kernel", s, 16 * v, [&] {
@@ -1668,65 +1626,45 @@ DownsampleRange downsample_impl(const cwipc_point *pts, size_t n, float cellsize
             throw;
         }
     }
+    if (!input_error.empty()) throw CudaError{cudaErrorInvalidValue, input_error};
     throw CudaError{cudaErrorUnknown, "downsample: no attempt succeeded"};
 }
 
-OctreeSeed no_seed() {
-    OctreeSeed none;
-    memset(&none, 0, sizeof(none));
-    return none;
-}
-
 // a new cloud of exactly the voxels
-DownsampleResult downsample_to_cloud(const StoragePtr &in, float cellsize, bool octree_split, const OctreeBox *external, uint64_t total_points, int dev, cudaStream_t s) {
+StoragePtr downsample_to_cloud(const StoragePtr &in, float cellsize, bool octree_split, const cwipc_cuda_octree_state *planned, const float *bounds, int dev, cudaStream_t s) {
     StoragePtr out;
-    const DownsampleRange r = downsample_impl(in->d_pts, in->count, cellsize, octree_split, external, total_points, [&](size_t v) {
+    const DownsampleRange r = downsample_impl(in->d_pts, in->count, cellsize, octree_split, planned, bounds, [&](size_t v) {
         out = std::make_shared<Storage>(dev, v, s);
         return out->d_pts;
     }, dev, s);
-    DownsampleResult result;
-    if (r.failed) {
-        result.failed = true;
-        result.error = r.error;
-        return result;
-    }
     out->count = r.count;
     out->has_bounds = r.has_bounds;
     memcpy(out->bounds_min, r.bounds_min, sizeof(out->bounds_min));
     memcpy(out->bounds_max, r.bounds_max, sizeof(out->bounds_max));
     out->mark_ready();
-    result.out = out;
-    return result;
+    return out;
 }
 } // namespace
 
-DownsampleResult downsample_points(const StoragePtr &in, float cellsize, bool octree_split, int dev, cudaStream_t s) {
-    return downsample_to_cloud(in, cellsize, octree_split, nullptr, 0, dev, s);
+StoragePtr downsample_points(const StoragePtr &in, float cellsize, bool octree_split, int dev, cudaStream_t s) {
+    return downsample_to_cloud(in, cellsize, octree_split, nullptr, nullptr, dev, s);
 }
 
 // the scale of the centroid sums comes from n, as for a cloud of these n points
 DownsampleRange downsample_range(const cwipc_point *pts, size_t n, float cellsize, bool octree_split, cwipc_point *dst, int dev, cudaStream_t s) {
-    return downsample_impl(pts, n, cellsize, octree_split, nullptr, 0, [dst](size_t) { return dst; }, dev, s);
+    return downsample_impl(pts, n, cellsize, octree_split, nullptr, nullptr, [dst](size_t) { return dst; }, dev, s);
 }
 
-// Partitioned clouds: the octree box and the bounding box of the WHOLE cloud are supplied by the caller.
-DownsampleResult downsample_points_planned(const StoragePtr &in, float cellsize, bool octree_split, const cwipc_cuda_octree_state &state, const float bounds[6], int dev, cudaStream_t s) {
-    OctreeBox ob;
-    memset(&ob, 0, sizeof(ob));
-    for (int a = 0; a < 3; a++) {
-        ob.min[a] = state.min[a];
-        ob.max[a] = state.max[a];
-        ob.gmin[a] = bounds[a];
-        ob.gmax[a] = bounds[3 + a];
+// Partitioned clouds: the octree box and the bounding box of the WHOLE cloud are supplied by the caller.  An empty part
+// contributes nothing, in either mode.
+StoragePtr downsample_points_planned(const StoragePtr &in, float cellsize, bool octree_split, const cwipc_cuda_octree_state &state, const float bounds[6], int dev, cudaStream_t s) {
+    if (in->count == 0) {
+        auto out = std::make_shared<Storage>(dev, 0, s);
+        out->mark_ready();
+        return out;
     }
-    ob.depth = state.depth;
-    if (octree_split && !state.valid && in->count > 0) {
-        DownsampleResult r;
-        r.failed = true;
-        r.error = "planned downsample needs the octree state of the whole cloud";
-        return r;
-    }
-    return downsample_to_cloud(in, cellsize, octree_split, &ob, state.points, dev, s);
+    if (octree_split && !state.valid) throw CudaError{cudaErrorInvalidValue, "planned downsample needs the octree state of the whole cloud"};
+    return downsample_to_cloud(in, cellsize, octree_split, &state, bounds, dev, s);
 }
 
 // Continue the octree bounding-box replay over this cloud's points; also returns its bounding box.
@@ -1736,17 +1674,7 @@ void octree_replay(const cwipc_point *in, size_t n, float cellsize, cwipc_cuda_o
         bounds[3 + a] = -INFINITY;
     }
     if (n == 0) return;
-    OctreeSeed seed;
-    memset(&seed, 0, sizeof(seed));
-    if (state.valid) {
-        for (int a = 0; a < 3; a++) {
-            seed.min[a] = state.min[a];
-            seed.max[a] = state.max[a];
-        }
-        seed.depth = state.depth;
-        seed.valid = 1;
-    }
-    const OctreeBox ob = measure_box(in, n, cellsize, true, seed, dev, s);
+    const OctreeBox ob = measure_box(in, n, cellsize, true, dev, s, state);
     if (ob.error) throw CudaError{cudaErrorInvalidValue, "octree replay: runaway growth (non-finite coordinates?)"};
     for (int a = 0; a < 3; a++) {
         state.min[a] = ob.min[a];
@@ -1760,26 +1688,15 @@ void octree_replay(const cwipc_point *in, size_t n, float cellsize, cwipc_cuda_o
 }
 
 void global_bbox(const cwipc_point *in, size_t n, float gmin[3], float gmax[3], int dev, cudaStream_t s) {
-    const uint32_t nchunks = (uint32_t)div_up(n, BB_CHUNK);
-    Scratch chunk_bbox((size_t)nchunks * 6 * sizeof(float), s);
-    Scratch box(sizeof(OctreeBox), s);
-    launch("bbox_octree_kernel", s, 16 * (size_t)n, [&] {
-        bbox_octree_kernel<<<nchunks, BB_THREADS, 0, s>>>(in, (uint32_t)n, chunk_bbox.as<float>(), nchunks, 1.0, 0, no_seed(), bbox_counter(dev, s), box.as<OctreeBox>());
-    });
-    OctreeBox *h = static_cast<OctreeBox *>(thread_pinned(sizeof(OctreeBox)));
-    CWCU_CHECK(cudaMemcpyAsync(h, box.p, sizeof(OctreeBox), cudaMemcpyDeviceToHost, s));
-    stream_sync(s);
-    for (int a = 0; a < 3; a++) {
-        gmin[a] = h->gmin[a];
-        gmax[a] = h->gmax[a];
-    }
+    const OctreeBox ob = measure_box(in, n, 0.f, false, dev, s); // no octree: the cell size is not used
+    memcpy(gmin, ob.gmin, sizeof(ob.gmin));
+    memcpy(gmax, ob.gmax, sizeof(ob.gmax));
 }
 
 void downsample_keys_to_host(const StoragePtr &in, float cellsize, bool octree_split, uint64_t *host_keys, int dev, cudaStream_t s) {
     const size_t n = in->count;
     if (n == 0) return;
-    Plan plan = derive_plan(measure_box(in->d_pts, n, cellsize, octree_split, no_seed(), dev, s), n, cellsize, octree_split);
-    if (plan.failed) throw CudaError{cudaErrorInvalidValue, plan.error};
+    const Plan plan = derive_plan(measure_box(in->d_pts, n, cellsize, octree_split, dev, s), n, cellsize, octree_split);
     Scratch keys(n * sizeof(uint64_t), s);
     Scratch flag(sizeof(uint32_t), s);
     CWCU_CHECK(cudaMemsetAsync(flag.p, 0, sizeof(uint32_t), s));

@@ -184,12 +184,7 @@ cwipc_pointcloud *cwipc_join(cwipc_pointcloud *pc1, cwipc_pointcloud *pc2) {
 cwipc_pointcloud *cwipc_downsample(cwipc_pointcloud *pc, float voxelsize) {
     return read_entry<cwipc_pointcloud *>("cwipc_downsample", pc, nullptr, [&](const StoragePtr &in, int dev, cudaStream_t s) -> cwipc_pointcloud * {
         const auto [octree_split, cellsize] = voxel_size(pc, voxelsize);
-        const DownsampleResult r = downsample_points(in, cellsize, octree_split, dev, s);
-        if (r.failed || !r.out) {
-            log(CWIPC_LOG_LEVEL_ERROR, "cwipc_downsample", r.error.empty() ? std::string("downsample failed") : r.error);
-            return nullptr;
-        }
-        return new_result(r.out, pc->timestamp(), cellsize);
+        return new_result(downsample_points(in, cellsize, octree_split, dev, s), pc->timestamp(), cellsize);
     });
 }
 
@@ -200,16 +195,22 @@ cwipc_pointcloud *cwipc_downsample(cwipc_pointcloud *pc, float voxelsize) {
 // ref: python/cwipc/registration/util.py:170-182, src/cwipc_filters.cpp:239-256
 cwipc_pointcloud *cwipc_cuda_downsample_pertile(cwipc_pointcloud *pc, float voxelsize) {
     return read_entry<cwipc_pointcloud *>("cwipc_cuda_downsample_pertile", pc, nullptr, [&](const StoragePtr &in, int dev, cudaStream_t s) -> cwipc_pointcloud * {
-        const auto [octree_split, cellsize] = voxel_size(pc, voxelsize);
+        const VoxelSize vs = voxel_size(pc, voxelsize);
         const size_t n = in->count;
         StoragePtr out;
-        std::string error;
         std::vector<size_t> counts;
         const std::vector<int> tiles = tiles_in_first_appearance_order(in->d_pts, n, s, &counts);
-        if (tiles.size() <= 1) { // the whole cloud is the only group (or there is none)
-            DownsampleResult r = downsample_points(in, cellsize, octree_split, dev, s);
-            out = r.out;
-            if (r.failed || !out) error = (tiles.empty() ? std::string() : "tile " + std::to_string(tiles[0]) + ": ") + (r.error.empty() ? std::string("downsample failed") : r.error);
+        // a group's failure names its tile
+        auto in_group = [](int tile, auto &&body) {
+            try {
+                return body();
+            } catch (const CudaError &e) {
+                throw CudaError{e.code, "tile " + std::to_string(tile) + ": " + e.what};
+            }
+        };
+        if (tiles.size() <= 1) { // the whole cloud is the only group (or there is none: an empty cloud, no tile to name)
+            auto whole = [&] { return downsample_points(in, vs.cellsize, vs.octree_split, dev, s); };
+            out = tiles.empty() ? whole() : in_group(tiles[0], whole);
         } else {
             // the non-zero groups side by side in one buffer; the tile-0 group is the input itself
             std::vector<int> split;
@@ -234,12 +235,7 @@ cwipc_pointcloud *cwipc_cuda_downsample_pertile(cwipc_pointcloud *pc, float voxe
                     cnt = counts[i];
                     offset += cnt;
                 }
-                const DownsampleRange r = downsample_range(src, cnt, cellsize, octree_split, out->d_pts + total, dev, s);
-                if (r.failed) {
-                    error = "tile " + std::to_string(tiles[i]) + ": " + r.error;
-                    out.reset();
-                    break;
-                }
+                const DownsampleRange r = in_group(tiles[i], [&] { return downsample_range(src, cnt, vs.cellsize, vs.octree_split, out->d_pts + total, dev, s); });
                 total += r.count;
                 // a box that holds every group's centroids
                 for (int a = 0; a < 3; a++) {
@@ -248,17 +244,11 @@ cwipc_pointcloud *cwipc_cuda_downsample_pertile(cwipc_pointcloud *pc, float voxe
                 }
                 first = false;
             }
-            if (out) {
-                out->count = total;
-                out->has_bounds = true;
-                out->mark_ready();
-            }
+            out->count = total;
+            out->has_bounds = true;
+            out->mark_ready();
         }
-        if (!out) {
-            log(CWIPC_LOG_LEVEL_ERROR, "cwipc_cuda_downsample_pertile", error);
-            return nullptr;
-        }
-        return new_result(out, pc->timestamp(), cellsize);
+        return new_result(out, pc->timestamp(), vs.cellsize);
     });
 }
 
@@ -342,18 +332,7 @@ cwipc_pointcloud *cwipc_cuda_downsample_planned(cwipc_pointcloud *pc, float voxe
     if (state == nullptr || bounds == nullptr) return nullptr;
     return read_entry<cwipc_pointcloud *>("cwipc_cuda_downsample_planned", pc, nullptr, [&](const StoragePtr &in, int dev, cudaStream_t s) -> cwipc_pointcloud * {
         const auto [octree_split, cellsize] = voxel_size(pc, voxelsize);
-        DownsampleResult r;
-        if (in->count == 0) {
-            r.out = std::make_shared<Storage>(dev, 0, s); // an empty part contributes nothing
-            r.out->mark_ready();
-        } else {
-            r = downsample_points_planned(in, cellsize, octree_split, *state, bounds, dev, s);
-        }
-        if (r.failed || !r.out) {
-            log(CWIPC_LOG_LEVEL_ERROR, "cwipc_cuda_downsample_planned", r.error.empty() ? std::string("downsample failed") : r.error);
-            return nullptr;
-        }
-        return new_result(r.out, pc->timestamp(), cellsize);
+        return new_result(downsample_points_planned(in, cellsize, octree_split, *state, bounds, dev, s), pc->timestamp(), cellsize);
     });
 }
 

@@ -47,19 +47,14 @@ void split_by_tile(const cwipc_point *in, size_t n, const std::vector<int> &tile
 void synthetic_points(cwipc_point *out, int side, float dh, float da, const float *d_radius, const double *d_sin, const double *d_cos, float angle, bool eyes_lit, cudaStream_t s);
 
 // ---- downsample.cu -------------------------------------------------------------------------
-struct DownsampleResult {
-    StoragePtr out;    // nullptr on failure
-    bool failed = false;
-    std::string error; // reference-compatible error text when failed
-};
+// An input that cannot be downsampled (empty in single-grid mode, invalid voxel size, non-finite coordinates, too large an
+// extent for the voxel size, ...) throws CudaError{cudaErrorInvalidValue} with the reference-compatible error text.
 // cellsize > 0 already resolved against the cloud's own cellsize.  octree_split selects the
 // reference's positive-size path (per-octree-leaf grids) vs the single global grid.
-DownsampleResult downsample_points(const StoragePtr &in, float cellsize, bool octree_split, int dev, cudaStream_t s);
+StoragePtr downsample_points(const StoragePtr &in, float cellsize, bool octree_split, int dev, cudaStream_t s);
 // The same downsample of pts[0..n), written to dst (room for n points) instead of a new cloud: the voxels come out exactly as
 // downsample_points gives them for a cloud of these n points.  Returns their number and the input's bounding box.
 struct DownsampleRange {
-    bool failed = false;
-    std::string error;
     size_t count = 0;
     bool has_bounds = false; // false when n == 0
     float bounds_min[3] = {0, 0, 0}, bounds_max[3] = {0, 0, 0};
@@ -69,8 +64,10 @@ DownsampleRange downsample_range(const cwipc_point *pts, size_t n, float cellsiz
 // over several GPUs is replayed part by part, the state travelling from rank to rank).  A state that starts a replay is
 // all zero.
 void octree_replay(const cwipc_point *in, size_t n, float cellsize, cwipc_cuda_octree_state &state, float bounds[6], int dev, cudaStream_t s);
-DownsampleResult downsample_points_planned(const StoragePtr &in, float cellsize, bool octree_split, const cwipc_cuda_octree_state &state, const float bounds[6], int dev,
-                                           cudaStream_t s);
+// downsample_points of one part of such a cloud, with the octree state and the bounding box of the whole cloud; an empty
+// part gives an empty cloud in either mode.
+StoragePtr downsample_points_planned(const StoragePtr &in, float cellsize, bool octree_split, const cwipc_cuda_octree_state &state, const float bounds[6], int dev,
+                                     cudaStream_t s);
 // global bounding box of in[0..n), n > 0 (synchronises the stream)
 void global_bbox(const cwipc_point *in, size_t n, float gmin[3], float gmax[3], int dev, cudaStream_t s);
 // diagnostic: sort keys (without the index bits) per input point, to host

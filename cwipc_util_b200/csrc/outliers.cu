@@ -1261,19 +1261,6 @@ __global__ void __launch_bounds__(ST_THREADS) stats_threshold_tile_kernel(const 
     *threshold_out = mean + stddev_mul * sqrt(variance);
 }
 
-int bit_length(uint64_t v) {
-    int b = 0;
-    while (v) {
-        b++;
-        v >>= 1;
-    }
-    return b;
-}
-
-unsigned stream_grid(size_t n, int dev) {
-    return (unsigned)std::max<size_t>(1, std::min(div_up(n, 256), (size_t)sm_count(dev) * 8));
-}
-
 // Test hooks of the kNN index (results never depend on them): CWIPC_CUDA_KNN_PITCH scales the pitch relative to the
 // expected k-neighbour radius, the others move work between the main pass, the second scan and the tree search.
 float env_float(const char *name, float dflt, float lo, float hi) {

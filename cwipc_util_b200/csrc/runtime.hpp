@@ -12,6 +12,7 @@
 #pragma once
 
 #include <cuda_runtime.h>
+#include <algorithm>
 #include <atomic>
 #include <cstddef>
 #include <cstdint>
@@ -203,5 +204,16 @@ void profile_reset();
 std::string profile_report_json();
 
 inline size_t div_up(size_t a, size_t b) { return (a + b - 1) / b; }
+// number of significant bits of v (0 for 0)
+inline int bit_length(uint64_t v) {
+    int b = 0;
+    while (v) {
+        b++;
+        v >>= 1;
+    }
+    return b;
+}
+// grid of a grid-stride kernel of 256 threads over n items: at most 8 blocks per SM
+inline unsigned stream_grid(size_t n, int dev) { return (unsigned)std::max<size_t>(1, std::min(div_up(n, 256), (size_t)sm_count(dev) * 8)); }
 
 } // namespace cwcu

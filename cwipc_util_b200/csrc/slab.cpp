@@ -198,12 +198,6 @@ size_t crop_x(const cwipc_point *in, size_t n, float lo, float hi, Scratch &out,
     return compact_points(in, n, out.as<cwipc_point>(), p, dev, s);
 }
 
-StoragePtr empty_storage(int dev, cudaStream_t s) {
-    auto st = std::make_shared<Storage>(dev, 0, s);
-    st->mark_ready();
-    return st;
-}
-
 // ---- downsample ----------------------------------------------------------------------------------------------------
 StoragePtr slab_downsample_storage(const StoragePtr &in, float voxelsize, float pc_cellsize, cwipc_cuda_comm *c, float *cellsize_out, int dev, cudaStream_t s) {
     const int G = c->size, r = c->rank;
@@ -230,7 +224,11 @@ StoragePtr slab_downsample_storage(const StoragePtr &in, float voxelsize, float 
         }
     }
     *cellsize_out = cs;
-    if (!any) return empty_storage(dev, s); // every part is empty: no leaves, an empty cloud (single-grid mode: the caller reports the reference's error)
+    if (!any) { // every part is empty: no leaves, an empty cloud (single-grid mode: the caller reports the reference's error)
+        auto empty = std::make_shared<Storage>(dev, 0, s);
+        empty->mark_ready();
+        return empty;
+    }
 
     // 2. octree box replay, rank by rank (the box grows with the points IN ORDER).  The box doubles every time it grows, so it
     //    usually contains the whole cloud's bounding box after the first part or two: rank r replays its part and
@@ -294,13 +292,10 @@ StoragePtr slab_downsample_storage(const StoragePtr &in, float voxelsize, float 
         if (incoming.total) CWCU_CHECK(cudaMemcpyAsync(mine->d_pts + keep_count, incoming.buf.p, incoming.total * sizeof(cwipc_point), cudaMemcpyDeviceToDevice, s));
         mine->mark_ready();
     }
-    if (mine->count == 0) return empty_storage(dev, s);
 
-    // 4. the local reduction, with the whole cloud's octree box and bounding box
+    // 4. the local reduction, with the whole cloud's octree box and bounding box (an empty part gives an empty cloud)
     const float bounds[6] = {gmin[0], gmin[1], gmin[2], gmax[0], gmax[1], gmax[2]};
-    DownsampleResult res = downsample_points_planned(mine, cs, octree, state, bounds, dev, s);
-    if (res.failed || !res.out) throw CudaError{cudaErrorUnknown, res.error.empty() ? std::string("downsample failed") : res.error};
-    return res.out;
+    return downsample_points_planned(mine, cs, octree, state, bounds, dev, s);
 }
 
 // ---- outlier removal of one group -----------------------------------------------------------------------------------
