@@ -35,6 +35,7 @@
 
 #include "device_utils.cuh"
 #include "kernels.hpp"
+#include "pointcloud.hpp"
 #include "radix_sort.hpp"
 
 namespace cwcu {
@@ -1658,11 +1659,7 @@ DownsampleRange downsample_range(const cwipc_point *pts, size_t n, float cellsiz
 // Partitioned clouds: the octree box and the bounding box of the WHOLE cloud are supplied by the caller.  An empty part
 // contributes nothing, in either mode.
 StoragePtr downsample_points_planned(const StoragePtr &in, float cellsize, bool octree_split, const cwipc_cuda_octree_state &state, const float bounds[6], int dev, cudaStream_t s) {
-    if (in->count == 0) {
-        auto out = std::make_shared<Storage>(dev, 0, s);
-        out->mark_ready();
-        return out;
-    }
+    if (in->count == 0) return new_storage(dev, 0, s, [](Storage &) -> size_t { return 0; });
     if (octree_split && !state.valid) throw CudaError{cudaErrorInvalidValue, "planned downsample needs the octree state of the whole cloud"};
     return downsample_to_cloud(in, cellsize, octree_split, &state, bounds, dev, s);
 }

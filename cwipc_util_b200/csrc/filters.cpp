@@ -35,27 +35,11 @@ VoxelSize voxel_size(cwipc_pointcloud *pc, float voxelsize) {
     return {octree_split, own >= cellsize ? own : cellsize};
 }
 
-// a subset of a cloud lies inside any box that contains the cloud
-void inherit_bounds(Storage &out, const Storage &in) {
-    if (!in.has_bounds) return;
-    out.has_bounds = true;
-    memcpy(out.bounds_min, in.bounds_min, sizeof(out.bounds_min));
-    memcpy(out.bounds_max, in.bounds_max, sizeof(out.bounds_max));
-}
-
 const float *bounds_of(const Storage &in, float box[6]) {
     if (!in.has_bounds) return nullptr;
     memcpy(box, in.bounds_min, 3 * sizeof(float));
     memcpy(box + 3, in.bounds_max, 3 * sizeof(float));
     return box;
-}
-
-StoragePtr compact_to_new(const StoragePtr &in, const Predicate &pred, int dev, cudaStream_t s) {
-    auto out = std::make_shared<Storage>(dev, in->count, s);
-    out->count = compact_points(in->d_pts, in->count, out->d_pts, pred, dev, s);
-    inherit_bounds(*out, *in);
-    out->mark_ready();
-    return out;
 }
 
 // cwipc_cuda_transform's arguments checked, and the matrix slot of every tile value: slot[v] = i for tiles[i] == v, else the
@@ -88,58 +72,42 @@ extern "C" {
 cwipc_pointcloud *cwipc_tilefilter(cwipc_pointcloud *pc, int tile) {
     return unary_filter("cwipc_tilefilter", pc, [&](const StoragePtr &in, int dev, cudaStream_t s) -> StoragePtr {
         if (tile == 0) return in; // keeps every point: storage is immutable, so share it
-        if (tile < 0 || tile > 255) {
-            // `tile == pt.a` with an 8-bit pt.a can never hold: empty result
-            auto out = std::make_shared<Storage>(dev, 0, s);
-            out->mark_ready();
-            return out;
-        }
-        Predicate p;
-        p.kind = PredKind::TileEquals;
-        p.tile = tile;
-        return compact_to_new(in, p, dev, s);
+        if (tile < 0 || tile > 255) return new_storage(dev, 0, s, [](Storage &) -> size_t { return 0; }); // `tile == pt.a` with an 8-bit pt.a can never hold
+        return new_storage(dev, in->count, s, [&](Storage &out) { return compact_points(in->d_pts, in->count, out.d_pts, tile_equals(tile), dev, s); }, in.get());
     });
 }
 
 // (tile & mask) != 0, the variant python/cwipc/registration/util.py:98-112 builds in numpy
 cwipc_pointcloud *cwipc_cuda_tilefilter_masked(cwipc_pointcloud *pc, int mask) {
     return unary_filter("cwipc_tilefilter_masked", pc, [&](const StoragePtr &in, int dev, cudaStream_t s) -> StoragePtr {
-        Predicate p;
-        p.kind = PredKind::TileMask;
-        p.tile = mask & 0xff;
-        return compact_to_new(in, p, dev, s);
+        return new_storage(dev, in->count, s, [&](Storage &out) { return compact_points(in->d_pts, in->count, out.d_pts, tile_mask(mask & 0xff), dev, s); }, in.get());
     });
 }
 
 // ref: src/cwipc_filters.cpp:333-360
 cwipc_pointcloud *cwipc_crop(cwipc_pointcloud *pc, float bbox[6]) {
     return unary_filter("cwipc_crop", pc, [&](const StoragePtr &in, int dev, cudaStream_t s) -> StoragePtr {
-        Predicate p;
-        p.kind = PredKind::CropBox;
-        memcpy(p.box, bbox, sizeof(p.box));
-        return compact_to_new(in, p, dev, s);
+        return new_storage(dev, in->count, s, [&](Storage &out) { return compact_points(in->d_pts, in->count, out.d_pts, crop_box(bbox), dev, s); }, in.get());
     });
 }
 
 // ref: src/cwipc_filters.cpp:308-331
 cwipc_pointcloud *cwipc_tilemap(cwipc_pointcloud *pc, uint8_t map[256]) {
     return unary_filter("cwipc_tilemap", pc, [&](const StoragePtr &in, int dev, cudaStream_t s) -> StoragePtr {
-        auto out = std::make_shared<Storage>(dev, in->count, s);
-        out->count = in->count;
-        tilemap_points(in->d_pts, in->count, out->d_pts, map, s);
-        out->mark_ready();
-        return out;
+        return new_storage(dev, in->count, s, [&](Storage &out) {
+            tilemap_points(in->d_pts, in->count, out.d_pts, map, s);
+            return in->count;
+        });
     });
 }
 
 // ref: src/cwipc_filters.cpp:362-386
 cwipc_pointcloud *cwipc_colormap(cwipc_pointcloud *pc, uint32_t clearBits, uint32_t setBits) {
     return unary_filter("cwipc_colormap", pc, [&](const StoragePtr &in, int dev, cudaStream_t s) -> StoragePtr {
-        auto out = std::make_shared<Storage>(dev, in->count, s);
-        out->count = in->count;
-        colormap_points(in->d_pts, in->count, out->d_pts, clearBits, setBits, s);
-        out->mark_ready();
-        return out;
+        return new_storage(dev, in->count, s, [&](Storage &out) {
+            colormap_points(in->d_pts, in->count, out.d_pts, clearBits, setBits, s);
+            return in->count;
+        });
     });
 }
 
@@ -150,11 +118,10 @@ cwipc_pointcloud *cwipc_cuda_transform(cwipc_pointcloud *pc, const double *matri
     return unary_filter("cwipc_cuda_transform", pc, [&](const StoragePtr &in, int dev, cudaStream_t s) -> StoragePtr {
         uint16_t slot[256];
         transform_slots(matrices, tiles, n, slot);
-        auto out = std::make_shared<Storage>(dev, in->count, s);
-        out->count = in->count;
-        transform_points(in->d_pts, in->count, out->d_pts, matrices, slot, n, dev, s);
-        out->mark_ready();
-        return out;
+        return new_storage(dev, in->count, s, [&](Storage &out) {
+            transform_points(in->d_pts, in->count, out.d_pts, matrices, slot, n, dev, s);
+            return in->count;
+        });
     });
 }
 
@@ -165,15 +132,15 @@ cwipc_pointcloud *cwipc_join(cwipc_pointcloud *pc1, cwipc_pointcloud *pc2) {
         StoragePtr b = storage_of(pc2, "cwipc_join");
         if (!b) return nullptr;
         ReadLease lease_b(*b, s);
-        auto out = std::make_shared<Storage>(dev, a->count + b->count, s);
-        out->count = a->count + b->count;
-        if (a->count) CWCU_CHECK(cudaMemcpyAsync(out->d_pts, a->d_pts, a->count * sizeof(cwipc_point), cudaMemcpyDeviceToDevice, s));
-        if (b->count) {
-            // a cloud on another device: an explicit peer copy (memory of a private pool is not reachable through UVA alone)
-            if (b->dev != dev) CWCU_CHECK(cudaMemcpyPeerAsync(out->d_pts + a->count, dev, b->d_pts, b->dev, b->count * sizeof(cwipc_point), s));
-            else CWCU_CHECK(cudaMemcpyAsync(out->d_pts + a->count, b->d_pts, b->count * sizeof(cwipc_point), cudaMemcpyDeviceToDevice, s));
-        }
-        out->mark_ready();
+        StoragePtr out = new_storage(dev, a->count + b->count, s, [&](Storage &o) {
+            if (a->count) CWCU_CHECK(cudaMemcpyAsync(o.d_pts, a->d_pts, a->count * sizeof(cwipc_point), cudaMemcpyDeviceToDevice, s));
+            if (b->count) {
+                // a cloud on another device: an explicit peer copy (memory of a private pool is not reachable through UVA alone)
+                if (b->dev != dev) CWCU_CHECK(cudaMemcpyPeerAsync(o.d_pts + a->count, dev, b->d_pts, b->dev, b->count * sizeof(cwipc_point), s));
+                else CWCU_CHECK(cudaMemcpyAsync(o.d_pts + a->count, b->d_pts, b->count * sizeof(cwipc_point), cudaMemcpyDeviceToDevice, s));
+            }
+            return a->count + b->count;
+        });
         return new_result(out, std::min(pc1->timestamp(), pc2->timestamp()), std::min(pc1->cellsize(), pc2->cellsize()));
     });
 }
@@ -224,29 +191,29 @@ cwipc_pointcloud *cwipc_cuda_downsample_pertile(cwipc_pointcloud *pc, float voxe
             split_by_tile(in->d_pts, n, split, nsplit, grouped.as<cwipc_point>(), dev, s);
             // a group keeps at most all of its points: room for the sum of the group sizes
             const bool has_zero = split.size() < tiles.size();
-            out = std::make_shared<Storage>(dev, has_zero ? n + nsplit : n, s);
-            size_t total = 0, offset = 0;
-            bool first = true;
-            for (size_t i = 0; i < tiles.size(); i++) {
-                const cwipc_point *src = in->d_pts;
-                size_t cnt = n;
-                if (tiles[i] != 0) {
-                    src = grouped.as<cwipc_point>() + offset;
-                    cnt = counts[i];
-                    offset += cnt;
+            out = new_storage(dev, has_zero ? n + nsplit : n, s, [&](Storage &o) {
+                size_t total = 0, offset = 0;
+                bool first = true;
+                for (size_t i = 0; i < tiles.size(); i++) {
+                    const cwipc_point *src = in->d_pts;
+                    size_t cnt = n;
+                    if (tiles[i] != 0) {
+                        src = grouped.as<cwipc_point>() + offset;
+                        cnt = counts[i];
+                        offset += cnt;
+                    }
+                    const DownsampleRange r = in_group(tiles[i], [&] { return downsample_range(src, cnt, vs.cellsize, vs.octree_split, o.d_pts + total, dev, s); });
+                    total += r.count;
+                    // a box that holds every group's centroids
+                    for (int a = 0; a < 3; a++) {
+                        o.bounds_min[a] = first ? r.bounds_min[a] : std::min(o.bounds_min[a], r.bounds_min[a]);
+                        o.bounds_max[a] = first ? r.bounds_max[a] : std::max(o.bounds_max[a], r.bounds_max[a]);
+                    }
+                    first = false;
                 }
-                const DownsampleRange r = in_group(tiles[i], [&] { return downsample_range(src, cnt, vs.cellsize, vs.octree_split, out->d_pts + total, dev, s); });
-                total += r.count;
-                // a box that holds every group's centroids
-                for (int a = 0; a < 3; a++) {
-                    out->bounds_min[a] = first ? r.bounds_min[a] : std::min(out->bounds_min[a], r.bounds_min[a]);
-                    out->bounds_max[a] = first ? r.bounds_max[a] : std::max(out->bounds_max[a], r.bounds_max[a]);
-                }
-                first = false;
-            }
-            out->count = total;
-            out->has_bounds = true;
-            out->mark_ready();
+                o.has_bounds = true;
+                return total;
+            });
         }
         return new_result(out, pc->timestamp(), vs.cellsize);
     });
@@ -260,44 +227,24 @@ cwipc_pointcloud *cwipc_remove_outliers(cwipc_pointcloud *pc, int kNeighbors, fl
         const size_t n = in->count;
         float box[6];
         const float *bounds = bounds_of(*in, box);
-        if (!perTile) {
-            auto out = std::make_shared<Storage>(dev, n, s);
-            out->count = remove_outliers_points(in->d_pts, n, out->d_pts, kNeighbors, stddevMulThresh, spacing, bounds, dev, s);
-            inherit_bounds(*out, *in);
-            out->mark_ready();
-            return out;
-        }
+        if (!perTile)
+            return new_storage(dev, n, s, [&](Storage &out) { return remove_outliers_points(in->d_pts, n, out.d_pts, kNeighbors, stddevMulThresh, spacing, bounds, dev, s); }, in.get());
         std::vector<int> tiles = tiles_in_first_appearance_order(in->d_pts, n, s);
         const bool has_zero = std::find(tiles.begin(), tiles.end(), 0) != tiles.end();
-        auto out = std::make_shared<Storage>(dev, has_zero ? 2 * n : n, s);
         static const bool sequential = getenv("CWIPC_CUDA_SOR_PER_TILE") && !strcmp(getenv("CWIPC_CUDA_SOR_PER_TILE"), "sequential"); // tests only
-        if (!has_zero && kNeighbors >= 1 && n > (size_t)kNeighbors && !sequential) {
-            // every group at once: one search index with the tile rank as a band of cells (outliers.cu)
-            out->count = remove_outliers_per_tile(in->d_pts, n, out->d_pts, tiles, kNeighbors, stddevMulThresh, spacing, bounds, dev, s);
-            inherit_bounds(*out, *in);
-            out->mark_ready();
-            return out;
-        }
-        // tile 0 among the values (the whole cloud is a group of its own, src/cwipc_filters.cpp:281-306) or fewer points
-        // than neighbours: group after group
-        Scratch group(n * sizeof(cwipc_point), s);
-        size_t total = 0;
-        for (int tile : tiles) {
-            const cwipc_point *src = in->d_pts;
-            size_t cnt = n;
-            if (tile != 0) {
-                Predicate p;
-                p.kind = PredKind::TileEquals;
-                p.tile = tile;
-                cnt = compact_points(in->d_pts, n, group.as<cwipc_point>(), p, dev, s);
-                src = group.as<cwipc_point>();
+        return new_storage(dev, has_zero ? 2 * n : n, s, [&](Storage &out) -> size_t {
+            if (!has_zero && kNeighbors >= 1 && n > (size_t)kNeighbors && !sequential) {
+                // every group at once: one search index with the tile rank as a band of cells (outliers.cu)
+                return remove_outliers_per_tile(in->d_pts, n, out.d_pts, tiles, kNeighbors, stddevMulThresh, spacing, bounds, dev, s);
             }
-            total += remove_outliers_points(src, cnt, out->d_pts + total, kNeighbors, stddevMulThresh, spacing, bounds, dev, s);
-        }
-        out->count = total;
-        inherit_bounds(*out, *in);
-        out->mark_ready();
-        return out;
+            // tile 0 among the values (the whole cloud is a group of its own, src/cwipc_filters.cpp:281-306) or fewer points
+            // than neighbours: group after group
+            size_t total = 0;
+            for_each_tile_group(in->d_pts, n, tiles, dev, s, [&](const cwipc_point *src, size_t cnt) {
+                total += remove_outliers_points(src, cnt, out.d_pts + total, kNeighbors, stddevMulThresh, spacing, bounds, dev, s);
+            });
+            return total;
+        }, in.get());
     });
 }
 
@@ -317,7 +264,8 @@ int cwipc_cuda_knn_mean_distances(cwipc_pointcloud *pc, int kNeighbors, float *d
 }
 
 // ---- partitioned clouds: building blocks for a cloud spread over several GPUs as x-slabs ---------------
-// The collective steps (who sends what to whom) are the caller's; see cwipc_util_b200/slab.py.
+// The library runs the whole protocol itself in slab.cpp (cwipc_cuda_slab_*).  These are its steps one call at a time, for
+// callers that move the data between the parts by their own means (cwipc_util_b200/slab.py) and for the tests.
 
 int cwipc_cuda_octree_replay(cwipc_pointcloud *pc, float cellsize, struct cwipc_cuda_octree_state *state, float bounds[6]) {
     if (state == nullptr || bounds == nullptr) return -1;
@@ -338,14 +286,11 @@ cwipc_pointcloud *cwipc_cuda_downsample_planned(cwipc_pointcloud *pc, float voxe
 
 cwipc_pointcloud *cwipc_cuda_from_device_points(const void *dev_points, int npoint, uint64_t timestamp) {
     if (npoint < 0 || (npoint > 0 && dev_points == nullptr)) return nullptr;
-    return guarded<cwipc_pointcloud *>("cwipc_cuda_from_device_points", nullptr, [&]() -> cwipc_pointcloud * {
-        const int dev = current_device();
-        DeviceGuard g(dev);
-        cudaStream_t s = thread_stream(dev);
-        auto out = std::make_shared<Storage>(dev, (size_t)npoint, s);
-        out->count = (size_t)npoint;
-        if (npoint) CWCU_CHECK(cudaMemcpyAsync(out->d_pts, dev_points, (size_t)npoint * sizeof(cwipc_point), cudaMemcpyDefault, s));
-        out->mark_ready();
+    return device_entry<cwipc_pointcloud *>("cwipc_cuda_from_device_points", nullptr, current_device(), [&](int dev, cudaStream_t s) -> cwipc_pointcloud * {
+        StoragePtr out = new_storage(dev, (size_t)npoint, s, [&](Storage &o) {
+            if (npoint) CWCU_CHECK(cudaMemcpyAsync(o.d_pts, dev_points, (size_t)npoint * sizeof(cwipc_point), cudaMemcpyDefault, s));
+            return (size_t)npoint;
+        });
         stream_sync(s); // the caller may reuse its buffer on return
         return new DevicePointcloud(out, timestamp, 0.f);
     });
@@ -398,17 +343,9 @@ cwipc_cuda_distances *cwipc_cuda_knn_query_open(cwipc_pointcloud *pc, int kNeigh
         h->mean = persistent_scratch((size_t)nquery * sizeof(float), s);
         h->open_idx = persistent_scratch((size_t)nquery * sizeof(uint32_t), s);
         h->kth = persistent_scratch((size_t)nquery * sizeof(float), s);
-        if (in->count > (size_t)kNeighbors) {
-            Scratch d(in->count * sizeof(float), s), kth(in->count * sizeof(float), s);
-            float box[6];
-            knn_mean_distances(in->d_pts, in->count, kNeighbors, pc->cellsize(), bounds_of(*in, box), d.as<float>(), dev, s, kth.as<float>(), (size_t)nquery);
-            CWCU_CHECK(cudaMemcpyAsync(h->mean.p, d.p, (size_t)nquery * sizeof(float), cudaMemcpyDeviceToDevice, s));
-            CWCU_CHECK(cudaMemcpyAsync(h->kth.p, kth.p, (size_t)nquery * sizeof(float), cudaMemcpyDeviceToDevice, s));
-            h->nopen = mark_open_queries(in->d_pts, kth.as<float>(), (size_t)nquery, x_lo, x_hi, h->open_idx.as<uint32_t>(), dev, s);
-        } else { // fewer points than neighbours here: every query is open, nothing is known about its neighbourhood
-            CWCU_CHECK(cudaMemsetAsync(h->kth.p, 0x7f, (size_t)nquery * sizeof(float), s)); // 0x7f7f7f7f: a huge finite float
-            h->nopen = mark_open_queries(in->d_pts, nullptr, (size_t)nquery, x_lo, x_hi, h->open_idx.as<uint32_t>(), dev, s);
-        }
+        float box[6];
+        h->nopen = knn_open_queries(in->d_pts, in->count, (size_t)nquery, kNeighbors, pc->cellsize(), bounds_of(*in, box), x_lo, x_hi, h->mean.as<float>(), h->kth.as<float>(),
+                                    h->open_idx.as<uint32_t>(), dev, s);
         *nopen = (int)h->nopen;
         return h.release();
     });
@@ -436,10 +373,8 @@ int cwipc_cuda_distances_open(cwipc_cuda_distances *h, cwipc_pointcloud *pc, uin
 // mean[idx[i]] = values[i] for the open queries (values in the order cwipc_cuda_distances_open returned them)
 int cwipc_cuda_distances_patch(cwipc_cuda_distances *h, const float *values, int n) {
     if (h == nullptr || n < 0 || (size_t)n != h->nopen || (n > 0 && values == nullptr)) return -1;
-    return guarded<int>("cwipc_cuda_distances_patch", -1, [&]() -> int {
-        if (n == 0) return 0;
-        DeviceGuard g(h->dev);
-        cudaStream_t s = thread_stream(h->dev);
+    if (n == 0) return 0;
+    return device_entry<int>("cwipc_cuda_distances_patch", -1, h->dev, [&](int, cudaStream_t s) -> int {
         Scratch v((size_t)n * sizeof(float), s);
         CWCU_CHECK(cudaMemcpyAsync(v.p, values, (size_t)n * sizeof(float), cudaMemcpyHostToDevice, s));
         scatter_floats(v.as<float>(), h->open_idx.as<uint32_t>(), (size_t)n, h->mean.as<float>(), s);
@@ -450,9 +385,8 @@ int cwipc_cuda_distances_patch(cwipc_cuda_distances *h, const float *values, int
 
 int cwipc_cuda_distances_stats(cwipc_cuda_distances *h, double sums[2]) {
     if (h == nullptr || sums == nullptr) return -1;
-    return guarded<int>("cwipc_cuda_distances_stats", -1, [&]() -> int {
-        DeviceGuard g(h->dev);
-        distance_stats(h->mean.as<float>(), h->n, sums, thread_stream(h->dev));
+    return device_entry<int>("cwipc_cuda_distances_stats", -1, h->dev, [&](int, cudaStream_t s) -> int {
+        distance_stats(h->mean.as<float>(), h->n, sums, s);
         return 0;
     });
 }
@@ -461,11 +395,8 @@ cwipc_pointcloud *cwipc_cuda_distances_filter(cwipc_pointcloud *pc, cwipc_cuda_d
     if (h == nullptr) return nullptr;
     return unary_filter("cwipc_cuda_distances_filter", pc, [&](const StoragePtr &in, int dev, cudaStream_t s) -> StoragePtr {
         if (h->n != in->count) throw CudaError{cudaErrorInvalidValue, "one distance per point is required"};
-        Predicate p;
-        p.kind = PredKind::DistanceAtMost;
-        p.dist = h->mean.as<float>();
-        p.threshold = threshold;
-        return compact_to_new(in, p, dev, s);
+        return new_storage(dev, in->count, s, [&](Storage &out) { return compact_points(in->d_pts, in->count, out.d_pts, distance_at_most(h->mean.as<float>(), threshold), dev, s); },
+                           in.get());
     });
 }
 
@@ -496,11 +427,8 @@ int cwipc_cuda_knn_lists(cwipc_pointcloud *pc, const struct cwipc_point *queries
 
 int cwipc_cuda_knn_merge_lists(const float *lists, int nlists, int nq, int kNeighbors, float *mean, float *kth2) {
     if (nq < 0 || nlists < 1 || (nq > 0 && (lists == nullptr || mean == nullptr))) return -1;
-    return guarded<int>("cwipc_cuda_knn_merge_lists", -1, [&]() -> int {
-        if (nq == 0) return 0;
-        const int dev = current_device();
-        DeviceGuard g(dev);
-        cudaStream_t s = thread_stream(dev);
+    if (nq == 0) return 0;
+    return device_entry<int>("cwipc_cuda_knn_merge_lists", -1, current_device(), [&](int, cudaStream_t s) -> int {
         const size_t kk = (size_t)kNeighbors + 1, total = (size_t)nlists * nq * kk;
         Scratch l(total * sizeof(float), s), m((size_t)nq * sizeof(float), s), kt((size_t)nq * sizeof(float), s);
         CWCU_CHECK(cudaMemcpyAsync(l.p, lists, total * sizeof(float), cudaMemcpyHostToDevice, s));
@@ -514,10 +442,7 @@ int cwipc_cuda_knn_merge_lists(const float *lists, int nlists, int nq, int kNeig
 
 int cwipc_cuda_distance_stats(const float *dist, size_t ndist, double sums[2]) {
     if (sums == nullptr || (ndist > 0 && dist == nullptr)) return -1;
-    return guarded<int>("cwipc_cuda_distance_stats", -1, [&]() -> int {
-        const int dev = current_device();
-        DeviceGuard g(dev);
-        cudaStream_t s = thread_stream(dev);
+    return device_entry<int>("cwipc_cuda_distance_stats", -1, current_device(), [&](int, cudaStream_t s) -> int {
         Scratch d(ndist * sizeof(float), s);
         if (ndist) CWCU_CHECK(cudaMemcpyAsync(d.p, dist, ndist * sizeof(float), cudaMemcpyHostToDevice, s));
         distance_stats(d.as<float>(), ndist, sums, s);
@@ -532,22 +457,16 @@ cwipc_pointcloud *cwipc_cuda_filter_by_distance(cwipc_pointcloud *pc, const floa
         if (ndist != in->count || (ndist > 0 && dist == nullptr)) throw CudaError{cudaErrorInvalidValue, "one distance per point is required"};
         Scratch d(ndist * sizeof(float), s);
         if (ndist) CWCU_CHECK(cudaMemcpyAsync(d.p, dist, ndist * sizeof(float), cudaMemcpyHostToDevice, s));
-        Predicate p;
-        p.kind = PredKind::DistanceAtMost;
-        p.dist = d.as<float>();
-        p.threshold = threshold;
-        return compact_to_new(in, p, dev, s);
+        return new_storage(dev, in->count, s, [&](Storage &out) { return compact_points(in->d_pts, in->count, out.d_pts, distance_at_most(d.as<float>(), threshold), dev, s); },
+                           in.get());
     });
 }
 
 // Diagnostic: the library's stable LSD radix sort on bits [begin_bit, end_bit) of host words, in place.
 int cwipc_cuda_sort_u64(uint64_t *words, size_t n, int begin_bit, int end_bit) {
     if (n > 0 && words == nullptr) return -1;
-    return guarded<int>("cwipc_cuda_sort_u64", -1, [&]() -> int {
-        if (n == 0) return 0;
-        const int dev = current_device();
-        DeviceGuard g(dev);
-        cudaStream_t s = thread_stream(dev);
+    if (n == 0) return 0;
+    return device_entry<int>("cwipc_cuda_sort_u64", -1, current_device(), [&](int dev, cudaStream_t s) -> int {
         Scratch a(n * sizeof(uint64_t), s), b(n * sizeof(uint64_t), s);
         CWCU_CHECK(cudaMemcpyAsync(a.p, words, n * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
         const uint64_t *sorted = radix_sort_u64(a.as<uint64_t>(), b.as<uint64_t>(), n, begin_bit, end_bit, dev, s);

@@ -2,6 +2,8 @@
 // stream; functions that return a count synchronise that stream once to read it back.
 #pragma once
 
+#include <cmath>
+
 #include "runtime.hpp"
 
 namespace cwcu {
@@ -18,8 +20,31 @@ struct Predicate {
     const double *threshold_dev = nullptr; // when not null the threshold is read from device memory instead
 };
 
+inline Predicate tile_equals(int tile) { return {PredKind::TileEquals, tile}; }
+inline Predicate tile_mask(int mask) { return {PredKind::TileMask, mask}; }
+inline Predicate crop_box(const float box[6]) { return {PredKind::CropBox, 0, {box[0], box[1], box[2], box[3], box[4], box[5]}}; }
+// lo <= x < hi, any y and z
+inline Predicate x_range(float lo, float hi) { return {PredKind::CropBox, 0, {lo, hi, -INFINITY, INFINITY, -INFINITY, INFINITY}}; }
+inline Predicate distance_at_most(const float *dist, double threshold) { return {PredKind::DistanceAtMost, 0, {}, dist, threshold}; }
+inline Predicate distance_at_most(const float *dist, const double *threshold_dev) { return {PredKind::DistanceAtMost, 0, {}, dist, 0.0, threshold_dev}; }
+
 // Stable compaction of in[0..n) by `pred` into out (capacity >= n).  Returns the number kept.
 size_t compact_points(const cwipc_point *in, size_t n, cwipc_point *out, const Predicate &pred, int dev, cudaStream_t s);
+
+// body(src, cnt) for every value of `tiles`, in that order: tile 0 is the whole of in[0..n), any other tile its points
+// (input order) compacted into one scratch block that the groups reuse.  n == 0 gives every tile the empty input.
+template <class Body>
+void for_each_tile_group(const cwipc_point *in, size_t n, const std::vector<int> &tiles, int dev, cudaStream_t s, Body &&body) {
+    Scratch group(n * sizeof(cwipc_point), s);
+    for (int tile : tiles) {
+        if (tile == 0 || n == 0) {
+            body(in, n);
+        } else {
+            const size_t cnt = compact_points(in, n, group.as<cwipc_point>(), tile_equals(tile), dev, s);
+            body(group.as<cwipc_point>(), cnt);
+        }
+    }
+}
 
 // One link of a chain of compactions into the same `out`: keeps the points of `tile` with !(dist[i] > *threshold_dev),
 // writing from position *d_base (device word; 0 when null) and leaving base + kept in *d_total.  No read-back; n > 0.
@@ -102,6 +127,13 @@ double outlier_threshold(double sum, double sq, double n, float stddev_mul);
 // Slab protocol: indices i < nquery whose (k+1)-th neighbour sphere (kth2[i], squared) is not strictly inside the covered
 // interval (x_lo, x_hi); kth2 == nullptr marks every query.  Returns their number (synchronises the stream).
 size_t mark_open_queries(const cwipc_point *pts, const float *kth2, size_t nquery, float x_lo, float x_hi, uint32_t *open_idx, int dev, cudaStream_t s);
+// Slab protocol, the queries of one part: the first nquery of pts[0..ncomb) (the part's own points; the rest is its halo)
+// against all ncomb.  d_mean / d_kth2 (nquery each) receive every query's mean distance and (k+1)-th smallest squared
+// distance, open_idx the queries marked open by mark_open_queries.  With ncomb <= k nothing is known about any
+// neighbourhood: d_mean is left alone, d_kth2 is 0x7f7f7f7f (a huge finite float) and every query is open.  Returns the
+// number of open queries (synchronises the stream).  0 < nquery <= ncomb.
+size_t knn_open_queries(const cwipc_point *pts, size_t ncomb, size_t nquery, int k, float hint_spacing, const float *bounds, float x_lo, float x_hi, float *d_mean, float *d_kth2,
+                        uint32_t *open_idx, int dev, cudaStream_t s);
 void gather_points(const cwipc_point *pts, const uint32_t *idx, size_t n, cwipc_point *out, cudaStream_t s);
 // the same with the indices in the low 32 bits of 64-bit words
 void gather_points(const cwipc_point *pts, const uint64_t *words, size_t n, cwipc_point *out, cudaStream_t s);

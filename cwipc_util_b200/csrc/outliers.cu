@@ -1766,6 +1766,19 @@ size_t mark_open_queries(const cwipc_point *pts, const float *kth2, size_t nquer
     return *h;
 }
 
+size_t knn_open_queries(const cwipc_point *pts, size_t ncomb, size_t nquery, int k, float hint_spacing, const float *bounds, float x_lo, float x_hi, float *d_mean, float *d_kth2,
+                        uint32_t *open_idx, int dev, cudaStream_t s) {
+    if (ncomb <= (size_t)k) {
+        CWCU_CHECK(cudaMemsetAsync(d_kth2, 0x7f, nquery * sizeof(float), s));
+        return mark_open_queries(pts, nullptr, nquery, x_lo, x_hi, open_idx, dev, s);
+    }
+    Scratch d(ncomb * sizeof(float), s), kth2(ncomb * sizeof(float), s);
+    knn_mean_distances(pts, ncomb, k, hint_spacing, bounds, d.as<float>(), dev, s, kth2.as<float>(), nquery);
+    CWCU_CHECK(cudaMemcpyAsync(d_mean, d.p, nquery * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    CWCU_CHECK(cudaMemcpyAsync(d_kth2, kth2.p, nquery * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    return mark_open_queries(pts, kth2.as<float>(), nquery, x_lo, x_hi, open_idx, dev, s);
+}
+
 void gather_points(const cwipc_point *pts, const uint32_t *idx, size_t n, cwipc_point *out, cudaStream_t s) {
     if (n == 0) return;
     launch("gather_points_kernel", s, 36 * n, [&] { gather_points_kernel<<<(unsigned)div_up(n, 256), 256, 0, s>>>(pts, idx, (uint32_t)n, out); });
@@ -1812,11 +1825,7 @@ size_t remove_outliers_points(const cwipc_point *in, size_t n, cwipc_point *out,
     launch("stats_kernel", s, 4 * (size_t)n, [&] {
         stats_threshold_kernel<<<ST_BLOCKS, ST_THREADS, 0, s>>>(dist.as<float>(), (uint32_t)n, partial.as<double>(), counter, (double)stddev_mul, d_thr);
     });
-    Predicate p;
-    p.kind = PredKind::DistanceAtMost;
-    p.dist = dist.as<float>();
-    p.threshold_dev = d_thr;
-    return compact_points(in, n, out, p, dev, s);
+    return compact_points(in, n, out, distance_at_most(dist.as<float>(), d_thr), dev, s);
 }
 
 size_t remove_outliers_per_tile(const cwipc_point *in, size_t n, cwipc_point *out, const std::vector<int> &tiles, int k, float stddev_mul, float hint_spacing, const float *bounds,

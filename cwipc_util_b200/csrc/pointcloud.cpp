@@ -54,13 +54,13 @@ DevicePointcloud *DevicePointcloud::from_host(const cwipc_point *points, size_t 
     if (device_count() <= 0) throw CudaError{cudaErrorNoDevice, "libcwipc_util_cuda needs a CUDA device and found none (there is no CPU fallback)"};
     cudaStream_t s = thread_stream(dev);
     DeviceGuard g(dev);
-    auto store = std::make_shared<Storage>(dev, npoint, s);
-    store->count = npoint;
     // Pageable source memory has been read completely when copy_from_host returns (it travels through the calling
     // thread's page-locked ring); page-locked memory is read by the DMA engine later, so wait unless the caller opted out.
     bool pinned = false;
-    if (npoint) pinned = copy_from_host(store->d_pts, points, npoint * sizeof(cwipc_point), s);
-    store->mark_ready();
+    StoragePtr store = new_storage(dev, npoint, s, [&](Storage &out) {
+        if (npoint) pinned = copy_from_host(out.d_pts, points, npoint * sizeof(cwipc_point), s);
+        return npoint;
+    });
     if (sync && npoint && pinned) stream_sync(s);
     return new DevicePointcloud(store, timestamp, 0.f);
 }
@@ -178,10 +178,10 @@ StoragePtr storage_of(cwipc_pointcloud *pc, const char *who) {
         const int dev = current_device();
         cudaStream_t s = thread_stream(dev);
         DeviceGuard g(dev);
-        auto store = std::make_shared<Storage>(dev, n, s);
-        store->count = n;
-        if (n) (void)copy_from_host(store->d_pts, host.data(), bytes, s);
-        store->mark_ready();
+        StoragePtr store = new_storage(dev, n, s, [&](Storage &out) {
+            if (n) (void)copy_from_host(out.d_pts, host.data(), bytes, s);
+            return n;
+        });
         stream_sync(s);
         return store;
     });

@@ -99,6 +99,33 @@ R read_entry(const char *who, cwipc_pointcloud *pc, R fallback, Body &&body) {
     });
 }
 
+// The shape of an entry point that reads no cloud: `body(dev, stream)` runs with `dev` current and the calling thread's
+// stream there; any exception -> an ERROR log naming `who` and `fallback`.
+template <class R, class Body>
+R device_entry(const char *who, R fallback, int dev, Body &&body) {
+    return guarded<R>(who, fallback, [&]() -> R {
+        DeviceGuard g(dev);
+        return body(dev, thread_stream(dev));
+    });
+}
+
+// A new storage of `capacity` points on `dev` whose home is `s`: `fill(out)` queues the work that writes out.d_pts and
+// returns the number of points.  `subset_of`, when not null, is a cloud that holds every result point: its box, if it has
+// one, is the result's too, so that the kNN grid of a following filter need not measure one.  The storage is marked ready
+// last, so that readers on other streams wait for the fill.
+template <class Fill>
+StoragePtr new_storage(int dev, size_t capacity, cudaStream_t s, Fill &&fill, const Storage *subset_of = nullptr) {
+    auto out = std::make_shared<Storage>(dev, capacity, s);
+    out->count = fill(*out);
+    if (subset_of && subset_of->has_bounds) {
+        out->has_bounds = true;
+        std::copy(subset_of->bounds_min, subset_of->bounds_min + 3, out->bounds_min);
+        std::copy(subset_of->bounds_max, subset_of->bounds_max + 3, out->bounds_max);
+    }
+    out->mark_ready();
+    return out;
+}
+
 // A filter result: a new cloud holding `out`, with the given timestamp and cellsize (cellsize < 0: estimated from the
 // points, as cwipc_pointcloud::_set_cellsize does).
 inline cwipc_pointcloud *new_result(StoragePtr out, uint64_t timestamp, float cellsize) {

@@ -189,13 +189,7 @@ float column_threshold(double v, float inv) {
 size_t crop_x(const cwipc_point *in, size_t n, float lo, float hi, Scratch &out, int dev, cudaStream_t s) {
     out = Scratch(n * sizeof(cwipc_point), s);
     if (n == 0) return 0;
-    Predicate p;
-    p.kind = PredKind::CropBox;
-    p.box[0] = lo;
-    p.box[1] = hi;
-    p.box[2] = p.box[4] = -INFINITY;
-    p.box[3] = p.box[5] = INFINITY;
-    return compact_points(in, n, out.as<cwipc_point>(), p, dev, s);
+    return compact_points(in, n, out.as<cwipc_point>(), x_range(lo, hi), dev, s);
 }
 
 // ---- downsample ----------------------------------------------------------------------------------------------------
@@ -224,11 +218,8 @@ StoragePtr slab_downsample_storage(const StoragePtr &in, float voxelsize, float 
         }
     }
     *cellsize_out = cs;
-    if (!any) { // every part is empty: no leaves, an empty cloud (single-grid mode: the caller reports the reference's error)
-        auto empty = std::make_shared<Storage>(dev, 0, s);
-        empty->mark_ready();
-        return empty;
-    }
+    // every part is empty: no leaves, an empty cloud (single-grid mode: the caller reports the reference's error)
+    if (!any) return new_storage(dev, 0, s, [](Storage &) -> size_t { return 0; });
 
     // 2. octree box replay, rank by rank (the box grows with the points IN ORDER).  The box doubles every time it grows, so it
     //    usually contains the whole cloud's bounding box after the first part or two: rank r replays its part and
@@ -286,11 +277,11 @@ StoragePtr slab_downsample_storage(const StoragePtr &in, float voxelsize, float 
     if (incoming.total == 0 && keep_ptr == in->d_pts) {
         mine = in;
     } else {
-        mine = std::make_shared<Storage>(dev, keep_count + incoming.total, s);
-        mine->count = keep_count + incoming.total;
-        if (keep_count) CWCU_CHECK(cudaMemcpyAsync(mine->d_pts, keep_ptr, keep_count * sizeof(cwipc_point), cudaMemcpyDeviceToDevice, s));
-        if (incoming.total) CWCU_CHECK(cudaMemcpyAsync(mine->d_pts + keep_count, incoming.buf.p, incoming.total * sizeof(cwipc_point), cudaMemcpyDeviceToDevice, s));
-        mine->mark_ready();
+        mine = new_storage(dev, keep_count + incoming.total, s, [&](Storage &o) {
+            if (keep_count) CWCU_CHECK(cudaMemcpyAsync(o.d_pts, keep_ptr, keep_count * sizeof(cwipc_point), cudaMemcpyDeviceToDevice, s));
+            if (incoming.total) CWCU_CHECK(cudaMemcpyAsync(o.d_pts + keep_count, incoming.buf.p, incoming.total * sizeof(cwipc_point), cudaMemcpyDeviceToDevice, s));
+            return keep_count + incoming.total;
+        });
     }
 
     // 4. the local reduction, with the whole cloud's octree box and bounding box (an empty part gives an empty cloud)
@@ -369,19 +360,8 @@ size_t slab_sor_group(const cwipc_point *pts, size_t n, cwipc_point *out, int k,
     }
     const float lo_lim = left ? (float)(xlo[r] - H) : -INFINITY, hi_lim = right ? (float)(xhi[r] + H) : INFINITY;
     const int kk = k + 1;
-    Scratch dist(std::max<size_t>(n, 1) * sizeof(float), s), kth(std::max<size_t>(ncomb, 1) * sizeof(float), s), open_idx(std::max<size_t>(n, 1) * sizeof(uint32_t), s);
-    size_t nopen = 0;
-    if (n) {
-        if (ncomb > (size_t)k) {
-            Scratch dall(ncomb * sizeof(float), s);
-            knn_mean_distances(combined, ncomb, k, (float)cs, nullptr, dall.as<float>(), dev, s, kth.as<float>(), n);
-            CWCU_CHECK(cudaMemcpyAsync(dist.p, dall.p, n * sizeof(float), cudaMemcpyDeviceToDevice, s));
-            nopen = mark_open_queries(combined, kth.as<float>(), n, lo_lim, hi_lim, open_idx.as<uint32_t>(), dev, s);
-        } else { // fewer points here than neighbours: every query is open, nothing is known about its neighbourhood
-            CWCU_CHECK(cudaMemsetAsync(kth.p, 0x7f, n * sizeof(float), s)); // 0x7f7f7f7f: a huge finite float
-            nopen = mark_open_queries(combined, nullptr, n, lo_lim, hi_lim, open_idx.as<uint32_t>(), dev, s);
-        }
-    }
+    Scratch dist(std::max<size_t>(n, 1) * sizeof(float), s), kth(std::max<size_t>(n, 1) * sizeof(float), s), open_idx(std::max<size_t>(n, 1) * sizeof(uint32_t), s);
+    const size_t nopen = n ? knn_open_queries(combined, ncomb, n, k, (float)cs, nullptr, lo_lim, hi_lim, dist.as<float>(), kth.as<float>(), open_idx.as<uint32_t>(), dev, s) : 0;
 
     // 4. open queries: all-gathered (points + bounds), answered by every rank from its own points, lists returned to the owners
     double my_open = (double)nopen;
@@ -440,11 +420,7 @@ size_t slab_sor_group(const cwipc_point *pts, size_t n, cwipc_point *out, int k,
     sums[2] = (double)n;
     allreduce_doubles(c, sums, 3, s);
     if (n == 0) return 0;
-    Predicate p;
-    p.kind = PredKind::DistanceAtMost;
-    p.dist = dist.as<float>();
-    p.threshold = outlier_threshold(sums[0], sums[1], sums[2], mul);
-    return compact_points(pts, n, out, p, dev, s);
+    return compact_points(pts, n, out, distance_at_most(dist.as<float>(), outlier_threshold(sums[0], sums[1], sums[2], mul)), dev, s);
 }
 
 // what every collective entry point needs of its communicator, for a cloud on `dev`
@@ -531,46 +507,30 @@ cwipc_pointcloud *cwipc_cuda_slab_remove_outliers(cwipc_pointcloud *pc, int kNei
         const size_t n = in->count;
         const float spacing = pc->cellsize();
         if (kNeighbors > 511) throw CudaError{cudaErrorInvalidValue, "remove_outliers: kNeighbors > 511 is not supported by libcwipc_util_cuda"};
-        StoragePtr out;
-        if (!perTile) {
-            out = std::make_shared<Storage>(dev, n, s);
-            out->count = slab_sor_group(in->d_pts, n, out->d_pts, kNeighbors, stddevMulThresh, spacing, halo, comm, dev, s);
-        } else {
-            // distinct tile values in first-appearance order of the whole cloud: the ranks' own lists, concatenated in rank order
-            std::vector<int> local = n ? tiles_in_first_appearance_order(in->d_pts, n, s) : std::vector<int>();
-            std::vector<double> row(257, -1.0);
-            row[0] = (double)local.size();
-            for (size_t i = 0; i < local.size(); i++) row[1 + i] = (double)local[i];
-            const std::vector<double> all = allgather_doubles(comm, row.data(), 257, s);
-            std::vector<int> tiles;
-            bool seen[256] = {false};
-            for (int q = 0; q < comm->size; q++)
-                for (int i = 0; i < (int)all[(size_t)q * 257]; i++) {
-                    const int t = (int)all[(size_t)q * 257 + 1 + i];
-                    if (!seen[t & 255]) {
-                        seen[t & 255] = true;
-                        tiles.push_back(t);
-                    }
+        auto sor = [&](const cwipc_point *src, size_t cnt, cwipc_point *dst) { return slab_sor_group(src, cnt, dst, kNeighbors, stddevMulThresh, spacing, halo, comm, dev, s); };
+        if (!perTile) return new_result(new_storage(dev, n, s, [&](Storage &out) { return sor(in->d_pts, n, out.d_pts); }), pc->timestamp(), pc->cellsize());
+        // distinct tile values in first-appearance order of the whole cloud: the ranks' own lists, concatenated in rank order
+        std::vector<int> local = n ? tiles_in_first_appearance_order(in->d_pts, n, s) : std::vector<int>();
+        std::vector<double> row(257, -1.0);
+        row[0] = (double)local.size();
+        for (size_t i = 0; i < local.size(); i++) row[1 + i] = (double)local[i];
+        const std::vector<double> all = allgather_doubles(comm, row.data(), 257, s);
+        std::vector<int> tiles;
+        bool seen[256] = {false};
+        for (int q = 0; q < comm->size; q++)
+            for (int i = 0; i < (int)all[(size_t)q * 257]; i++) {
+                const int t = (int)all[(size_t)q * 257 + 1 + i];
+                if (!seen[t & 255]) {
+                    seen[t & 255] = true;
+                    tiles.push_back(t);
                 }
-            const bool has_zero = seen[0];
-            out = std::make_shared<Storage>(dev, has_zero ? 2 * n : n, s);
-            Scratch group(std::max<size_t>(n, 1) * sizeof(cwipc_point), s);
-            size_t total = 0;
-            for (int tile : tiles) {
-                const cwipc_point *src = in->d_pts;
-                size_t cnt = n;
-                if (tile != 0 && n) {
-                    Predicate p;
-                    p.kind = PredKind::TileEquals;
-                    p.tile = tile;
-                    cnt = compact_points(in->d_pts, n, group.as<cwipc_point>(), p, dev, s);
-                    src = group.as<cwipc_point>();
-                }
-                total += slab_sor_group(src, cnt, out->d_pts + total, kNeighbors, stddevMulThresh, spacing, halo, comm, dev, s);
             }
-            out->count = total;
-        }
-        out->mark_ready();
+        const bool has_zero = seen[0];
+        StoragePtr out = new_storage(dev, has_zero ? 2 * n : n, s, [&](Storage &o) {
+            size_t total = 0;
+            for_each_tile_group(in->d_pts, n, tiles, dev, s, [&](const cwipc_point *src, size_t cnt) { total += sor(src, cnt, o.d_pts + total); });
+            return total;
+        });
         return new_result(out, pc->timestamp(), pc->cellsize());
     });
 }

@@ -142,18 +142,16 @@ private:
             const float pi = 3.14159265358979f;
             const float dh = 2.0f / m_side, da = 2 * pi / m_side;
             const bool eyes_lit = std::fmod(m_angle, pi / 2) > 0.08;
-            auto store = std::make_shared<Storage>(dev, n, s);
-            store->count = n;
-            {
+            StoragePtr store = new_storage(dev, n, s, [&](Storage &out) {
                 Scratch rad(m_side * sizeof(float), s), sn(m_side * sizeof(double), s), cs(m_side * sizeof(double), s);
                 if (m_side) {
                     CWCU_CHECK(cudaMemcpyAsync(rad.p, m_radius.data(), m_side * sizeof(float), cudaMemcpyHostToDevice, s));
                     CWCU_CHECK(cudaMemcpyAsync(sn.p, m_sin.data(), m_side * sizeof(double), cudaMemcpyHostToDevice, s));
                     CWCU_CHECK(cudaMemcpyAsync(cs.p, m_cos.data(), m_side * sizeof(double), cudaMemcpyHostToDevice, s));
-                    synthetic_points(store->d_pts, m_side, dh, da, rad.as<float>(), sn.as<double>(), cs.as<double>(), m_angle, eyes_lit, s);
+                    synthetic_points(out.d_pts, m_side, dh, da, rad.as<float>(), sn.as<double>(), cs.as<double>(), m_angle, eyes_lit, s);
                 }
-            }
-            store->mark_ready();
+                return n;
+            });
             auto *pc = new DevicePointcloud(store, timestamp, 0.f);
             pc->set_exact_size(true); // the reference builds this cloud with cwipc_from_points (:127)
             return pc;
