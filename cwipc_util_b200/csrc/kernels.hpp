@@ -139,20 +139,30 @@ void gather_points(const cwipc_point *pts, const uint32_t *idx, size_t n, cwipc_
 void gather_points(const cwipc_point *pts, const uint64_t *words, size_t n, cwipc_point *out, cudaStream_t s);
 void scatter_floats(const float *values, const uint32_t *idx, size_t n, float *out, cudaStream_t s);
 
-// cwipc_cuda_icp's correspondences: the search index of a target cloud (built once, k = 1), and the evaluation of a motion of
-// a source cloud against it.  sums, in double, relative to origin() (the centre of the target's box), over the pairs
-// (p' = motion * p, its nearest target point q) with float d2 <= limit, ties to the smaller target index:
-//   [0] count, [1] sum d2, [2..4] sum p', [5..7] sum q, [8..16] sum p'_a q_b (row-major a, b),
-//   [17] with check_finite: the number of points of either cloud with a non-finite coordinate (else 0).
+// cwipc_cuda_icp's correspondences: the search index of a target cloud (built once), and the evaluation of a motion of a
+// source cloud against it.  The pairs are (p' = motion * p, its nearest target point q) with float d2 <= limit, ties to the
+// smaller target index.  Their sums, in double, relative to origin() (the centre of the target's box):
+//   point-to-point (ICP_NSUMS): [0] count, [1] sum d2, [2..4] sum p', [5..7] sum q, [8..16] sum p'_a q_b (row-major a, b),
+//     [17] with check_finite: the number of points of either cloud with a non-finite coordinate (else 0);
+//   point-to-plane (ICP_PLANE_NSUMS), with n the target normal of q, r = (p' - q) . n and J = [p' x n, n]: [0] count,
+//     [1] sum d2, [2..22] sum J_a J_b (a <= b, row-major), [23..28] sum J_a r, [29] the non-finite count as above.
 // One search kernel, one reduction kernel and one read-back per evaluation; the same bits on every run.
 constexpr int ICP_NSUMS = 18;
+constexpr int ICP_PLANE_NSUMS = 30;
+constexpr int ICP_MAX_NN = 32; // a normal's neighbourhood fits one warp, one (d2, index) key per lane
 class IcpMatcher {
 public:
-    // nt > 0; bounds (min xyz, max xyz, nullable): a box known to hold every target point
+    // point-to-point: the index with k = 1.  nt > 0; bounds (min xyz, max xyz, nullable): a box known to hold every target point
     IcpMatcher(const cwipc_point *target, size_t nt, float hint_spacing, const float *bounds, int dev, cudaStream_t s);
+    // point-to-plane: the index with k = normal_max_nn (3..32), then the unit normal of every target point from its
+    // normal_max_nn nearest points within normal_radius (cwipc_cuda_estimate_normals in include/cwipc_util_cuda.h)
+    IcpMatcher(const cwipc_point *target, size_t nt, float hint_spacing, const float *bounds, int dev, cudaStream_t s, double normal_radius, int normal_max_nn);
     ~IcpMatcher();
     const double *origin() const;
-    void evaluate(const cwipc_point *source, size_t ns, const double motion[16], float limit, bool check_finite, double sums[ICP_NSUMS]);
+    int nsums() const; // ICP_NSUMS or ICP_PLANE_NSUMS
+    void evaluate(const cwipc_point *source, size_t ns, const double motion[16], float limit, bool check_finite, double *sums);
+    // point-to-plane only: the normals, 3 floats per target point in its order; false when a target point has a non-finite coordinate
+    bool normals_to_host(float *out);
 
 private:
     struct Impl;

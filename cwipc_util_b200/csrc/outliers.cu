@@ -1463,29 +1463,19 @@ struct IcpParams {
     uint32_t check;    // also count the non-finite coordinates of both clouds (first evaluation of a call)
 };
 
-// The nearest target point to q with d2 <= limit, as the key (d2 bits << 32) | (index in the target's input order), or ~0 when
-// there is none: the smallest key is the smallest d2 and, among equal ones, the smallest index.  Called by all 32 lanes with
-// the same q; the result is the same in every lane.  The search is dfs_knn's for one neighbour: depth-first through the table
-// pyramid, the four nearest open nodes per step (8 lanes per node), nodes of at most leaf_points points scanned.  It starts at
-// the <= 2x2x2 nodes of the lowest level that cover every cell within sqrt(limit) of q, and a node is dropped when its box is
-// farther than min(limit, best d2 so far).  So a query with no target point within the bound only visits the nodes that touch
-// its ball, never a scan of the cells around it.  Nodes at exactly the best d2 are kept: an equally near point with a smaller
-// index must still be seen.
-__device__ __forceinline__ uint64_t icp_nearest(const Point16 q, float limit, float slack, const Point16 *__restrict__ spts16, const uint64_t *__restrict__ sorted,
-                                                const GridParams &gp, const uint2 *__restrict__ table, uint32_t leaf_points, FarNode *stack) {
+// Depth-first search of the table pyramid around q, the search of icp_nearest and icp_neighbours, called by all 32 lanes
+// with the same q.  It is dfs_knn's search: the four nearest open nodes per step (8 lanes per node), nodes of at most
+// leaf_points points scanned.  It starts at the <= 2x2x2 nodes of the lowest level that cover every cell within sqrt(limit)
+// of q, and a node is dropped when its box is farther than tau, the caller's pruning bound (<= limit, the same in every
+// lane).  So a query with no target point within the bound only visits the nodes that touch its ball, never a scan of the
+// cells around it.  Nodes at exactly tau are kept: an equally near point with a smaller index must still be seen.
+// consider(c, valid) is called by every lane at once, with a position c of the cell-ordered target on the lanes where valid
+// is true; refresh() (all lanes) follows each batch and may lower tau.  Every target point is offered at most once.
+template <class Consider, class Refresh>
+__device__ __forceinline__ void pyramid_search(const Point16 q, float limit, float slack, const GridParams &gp, const uint2 *__restrict__ table, uint32_t leaf_points,
+                                               FarNode *stack, const float &tau, Consider &&consider, Refresh &&refresh) {
     const unsigned lane = lane_id();
-    const uint64_t idxmask = (1ull << gp.idxbits) - 1ull;
-    uint64_t best = ~0ull; // this lane's best key
-    float tau = limit;     // pruning bound, the same in every lane
     int sp = 0;
-    auto consider = [&](uint32_t c) { // position c of the cell-ordered target
-        const float d2 = dist2(q, spts16[c]);
-        if (d2 <= limit && __float_as_uint(d2) <= (uint32_t)(best >> 32)) best = min(best, ((uint64_t)__float_as_uint(d2) << 32) | (sorted[c] & idxmask));
-    };
-    auto refresh = [&] {
-        const uint32_t hi = __reduce_min_sync(FULL_MASK, (uint32_t)(best >> 32)); // non-negative floats order like their bits
-        if (hi != 0xffffffffu) tau = __uint_as_float(hi);
-    };
     // Lanes that `want` their node (level cl, (chx, chy, chz)) push it when it holds points and its box is within tau; the
     // pushed nodes are ranked by (distance, lane), the nearest on top.
     auto push_nodes = [&](bool want, int cl, uint32_t chx, uint32_t chy, uint32_t chz) {
@@ -1550,7 +1540,7 @@ __device__ __forceinline__ uint64_t icp_nearest(const Point16 q, float limit, fl
         __syncwarp();
         if (__all_sync(FULL_MASK, !have || node.pe - node.pb <= 8u)) { // sparse neighbourhood: every node taken is scanned at once
             const uint32_t c = node.pb + (lane & 7u);
-            if (have && c < node.pe) consider(c);
+            consider(c, have && c < node.pe);
             refresh();
             continue;
         }
@@ -1562,16 +1552,73 @@ __device__ __forceinline__ uint64_t icp_nearest(const Point16 q, float limit, fl
             const uint32_t pb = __shfl_sync(FULL_MASK, node.pb, src), pe = __shfl_sync(FULL_MASK, node.pe, src);
             if (__shfl_sync(FULL_MASK, node.mind2, src) * 0.9999f > tau) continue; // (the bound may have dropped since the vote)
             for (uint32_t base = pb; base < pe; base += 32)
-                if (base + lane < pe) consider(base + lane);
+                consider(base + lane, base + lane < pe);
             refresh();
         }
         const bool expand = have && !is_leaf && !(node.mind2 * 0.9999f > tau);
         push_nodes(expand, node_level - 1, 2u * (node.xy & 0xffffu) + ((lane >> 2) & 1u), 2u * (node.xy >> 16) + ((lane >> 1) & 1u), 2u * (node.zl & 0xffffu) + (lane & 1u));
         __syncwarp();
     }
+}
+
+// The nearest target point to q with d2 <= limit, as the key (d2 bits << 32) | (index in the target's input order), or ~0 when
+// there is none: the smallest key is the smallest d2 and, among equal ones, the smallest index.  Called by all 32 lanes with
+// the same q; the result is the same in every lane.  The pruning bound is min(limit, best d2 so far).
+__device__ __forceinline__ uint64_t icp_nearest(const Point16 q, float limit, float slack, const Point16 *__restrict__ spts16, const uint64_t *__restrict__ sorted,
+                                                const GridParams &gp, const uint2 *__restrict__ table, uint32_t leaf_points, FarNode *stack) {
+    const uint64_t idxmask = (1ull << gp.idxbits) - 1ull;
+    uint64_t best = ~0ull; // this lane's best key
+    float tau = limit;     // pruning bound, the same in every lane
+    pyramid_search(
+        q, limit, slack, gp, table, leaf_points, stack, tau,
+        [&](uint32_t c, bool valid) { // position c of the cell-ordered target
+            if (valid) {
+                const float d2 = dist2(q, spts16[c]);
+                if (d2 <= limit && __float_as_uint(d2) <= (uint32_t)(best >> 32)) best = min(best, ((uint64_t)__float_as_uint(d2) << 32) | (sorted[c] & idxmask));
+            }
+        },
+        [&] {
+            const uint32_t hi = __reduce_min_sync(FULL_MASK, (uint32_t)(best >> 32)); // non-negative floats order like their bits
+            if (hi != 0xffffffffu) tau = __uint_as_float(hi);
+        });
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) best = min(best, (uint64_t)__shfl_xor_sync(FULL_MASK, (unsigned long long)best, o));
     return best;
+}
+
+// The kk (1..32) smallest keys (d2 bits << 32) | (index in the target's input order) of the target points with d2 <= limit,
+// one per lane: lane j holds the j-th smallest, ~0 where there are fewer.  The set does not depend on the order in which the
+// points are met, so it is the same on every run.  The pruning bound is min(limit, the kk-th d2 so far) once kk are held.
+__device__ __forceinline__ uint64_t icp_neighbours(const Point16 q, float limit, float slack, int kk, const Point16 *__restrict__ spts16, const uint64_t *__restrict__ sorted,
+                                                   const GridParams &gp, const uint2 *__restrict__ table, uint32_t leaf_points, FarNode *stack) {
+    const int lane = (int)lane_id();
+    const uint64_t idxmask = (1ull << gp.idxbits) - 1ull;
+    uint64_t mine = ~0ull; // this lane's place in the ascending list
+    uint64_t kth = ~0ull;  // the list's last place (kk - 1), the same in every lane
+    float tau = limit;
+    pyramid_search(
+        q, limit, slack, gp, table, leaf_points, stack, tau,
+        [&](uint32_t c, bool valid) {
+            uint64_t key = ~0ull;
+            if (valid) {
+                const float d2 = dist2(q, spts16[c]);
+                if (d2 <= limit) key = ((uint64_t)__float_as_uint(d2) << 32) | (sorted[c] & idxmask);
+            }
+            // insert the lanes' keys that beat the list one at a time: place pos = how many listed keys are smaller
+            for (unsigned todo = __ballot_sync(FULL_MASK, key < kth); todo; todo &= todo - 1u) {
+                const uint64_t x = __shfl_sync(FULL_MASK, (unsigned long long)key, __ffs(todo) - 1);
+                if (!(x < kth)) continue;
+                const int pos = __popc(__ballot_sync(FULL_MASK, mine < x));
+                const uint64_t up = __shfl_up_sync(FULL_MASK, (unsigned long long)mine, 1);
+                if (lane == pos) mine = x;
+                else if (lane > pos && lane < kk) mine = up;
+                kth = __shfl_sync(FULL_MASK, (unsigned long long)mine, kk - 1);
+            }
+        },
+        [&] {
+            if (kth != ~0ull) tau = __uint_as_float((uint32_t)(kth >> 32));
+        });
+    return mine;
 }
 
 __device__ __forceinline__ bool finite_point(const Point16 &p) { return isfinite(p.x) && isfinite(p.y) && isfinite(p.z); }
@@ -1627,6 +1674,180 @@ __global__ void __launch_bounds__(ICP_NSUMS * 32) icp_reduce_kernel(const double
     const unsigned lane = lane_id(), j = threadIdx.x >> 5;
     double s = 0.0;
     for (uint32_t w = lane; w < nwarps; w += 32) s += partial[(size_t)w * ICP_NSUMS + j];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(FULL_MASK, s, o);
+    if (lane == 0) out[j] = s;
+}
+
+// ---- point-to-plane ICP (cwipc_cuda_icp_point_to_plane, cwipc_cuda_estimate_normals) ----------------------------------------
+// One cyclic Jacobi rotation of the symmetric 3x3 A that zeroes A[P][Q], accumulated in the columns of V.
+template <int P, int Q>
+__device__ __forceinline__ void jacobi3_rotate(double (&A)[3][3], double (&V)[3][3]) {
+    if (A[P][Q] == 0.0) return;
+    const double theta = (A[Q][Q] - A[P][P]) / (2.0 * A[P][Q]);
+    const double t = (theta >= 0.0 ? 1.0 : -1.0) / (fabs(theta) + sqrt(theta * theta + 1.0));
+    const double c = 1.0 / sqrt(t * t + 1.0), s = t * c;
+#pragma unroll
+    for (int k = 0; k < 3; k++) {
+        const double a = A[k][P], b = A[k][Q];
+        A[k][P] = c * a - s * b;
+        A[k][Q] = s * a + c * b;
+    }
+#pragma unroll
+    for (int k = 0; k < 3; k++) {
+        const double a = A[P][k], b = A[Q][k];
+        A[P][k] = c * a - s * b;
+        A[Q][k] = s * a + c * b;
+    }
+#pragma unroll
+    for (int k = 0; k < 3; k++) {
+        const double a = V[k][P], b = V[k][Q];
+        V[k][P] = c * a - s * b;
+        V[k][Q] = s * a + c * b;
+    }
+}
+
+// The unit eigenvector of the smallest eigenvalue of the symmetric 3x3 A, by cyclic Jacobi rotations in double (the same
+// rules as icp.cpp's horn_rotation: an off-diagonal entry below the rounding of both diagonal entries is dropped).
+__device__ __forceinline__ float3 smallest_eigenvector(double (&A)[3][3]) {
+    double V[3][3] = {{1.0, 0.0, 0.0}, {0.0, 1.0, 0.0}, {0.0, 0.0, 1.0}};
+    for (int sweep = 0; sweep < 50 && !(A[0][1] == 0.0 && A[0][2] == 0.0 && A[1][2] == 0.0); sweep++) {
+        if (sweep > 3) {
+#pragma unroll
+            for (int p = 0; p < 2; p++)
+#pragma unroll
+                for (int q = p + 1; q < 3; q++) {
+                    const double g = 100.0 * fabs(A[p][q]);
+                    if (fabs(A[p][p]) + g == fabs(A[p][p]) && fabs(A[q][q]) + g == fabs(A[q][q])) A[p][q] = A[q][p] = 0.0;
+                }
+        }
+        jacobi3_rotate<0, 1>(A, V);
+        jacobi3_rotate<0, 2>(A, V);
+        jacobi3_rotate<1, 2>(A, V);
+    }
+    const int m = A[0][0] <= A[1][1] ? (A[0][0] <= A[2][2] ? 0 : 2) : (A[1][1] <= A[2][2] ? 1 : 2);
+    const double x = m == 0 ? V[0][0] : (m == 1 ? V[0][1] : V[0][2]);
+    const double y = m == 0 ? V[1][0] : (m == 1 ? V[1][1] : V[1][2]);
+    const double z = m == 0 ? V[2][0] : (m == 1 ? V[2][1] : V[2][2]);
+    const double inv = 1.0 / sqrt(x * x + y * y + z * z);
+    return make_float3((float)(x * inv), (float)(y * inv), (float)(z * inv));
+}
+
+// One warp per point of the cloud, in cell order (grid-stride): its neighbourhood is the kk smallest keys (d2, index) of the
+// cloud's points with d2 <= limit (itself included), found by icp_neighbours.  The mean and then the covariance relative to
+// it are summed in double over the lanes in a fixed butterfly order; the normal is the unit eigenvector of the covariance's
+// smallest eigenvalue.  normals[i] (input order) = (nx, ny, nz, 0); (0, 0, 0, 0) for fewer than 3 neighbours or a zero
+// covariance; (0, 0, 0, 1) for a point with a non-finite coordinate.
+__global__ void __launch_bounds__(ICP_THREADS) icp_normals_kernel(const cwipc_point *__restrict__ pts, uint32_t n, const cwipc_point *__restrict__ spts,
+                                                                  const uint64_t *__restrict__ sorted, const __grid_constant__ GridParams gp, const uint2 *__restrict__ table,
+                                                                  uint32_t leaf_points, float limit, float slack, int kk, float4 *__restrict__ normals) {
+    __shared__ __align__(16) FarNode s_stack[ICP_WARPS][KF_STACK];
+    const unsigned lane = lane_id(), warp = threadIdx.x >> 5;
+    const uint32_t gwarp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, warps_total = (gridDim.x * blockDim.x) >> 5;
+    const Point16 *spts16 = reinterpret_cast<const Point16 *>(spts);
+    const uint64_t idxmask = (1ull << gp.idxbits) - 1ull;
+    for (uint32_t c = gwarp; c < n; c += warps_total) {
+        const Point16 q = spts16[c];
+        const uint32_t self = (uint32_t)(sorted[c] & idxmask);
+        float4 out = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (!finite_point(q)) {
+            out.w = 1.f;
+        } else {
+            const uint64_t key = icp_neighbours(q, limit, slack, kk, spts16, sorted, gp, table, leaf_points, s_stack[warp]);
+            const bool have = key != ~0ull;
+            const int cnt = __popc(__ballot_sync(FULL_MASK, have));
+            if (cnt >= 3) {
+                double p[3] = {0.0, 0.0, 0.0};
+                if (have) {
+                    const Point16 t = ld_point(pts, (uint32_t)(key & idxmask));
+                    p[0] = t.x, p[1] = t.y, p[2] = t.z;
+                }
+                double mean[3];
+#pragma unroll
+                for (int a = 0; a < 3; a++) mean[a] = warp_sum(p[a]) / (double)cnt;
+#pragma unroll
+                for (int a = 0; a < 3; a++) p[a] = have ? p[a] - mean[a] : 0.0;
+                double A[3][3];
+#pragma unroll
+                for (int a = 0; a < 3; a++)
+#pragma unroll
+                    for (int b = a; b < 3; b++) A[a][b] = A[b][a] = warp_sum(p[a] * p[b]);
+                if (!(A[0][0] == 0.0 && A[1][1] == 0.0 && A[2][2] == 0.0)) { // (a zero diagonal is a zero covariance)
+                    const float3 v = smallest_eigenvector(A);
+                    out.x = v.x, out.y = v.y, out.z = v.z;
+                }
+            }
+        }
+        if (lane == 0) normals[self] = out;
+    }
+}
+
+__device__ __forceinline__ double pick6(const double (&v)[6], int i) {
+    return i == 0 ? v[0] : (i == 1 ? v[1] : (i == 2 ? v[2] : (i == 3 ? v[3] : (i == 4 ? v[4] : v[5]))));
+}
+
+// icp_match_kernel's correspondences (the same search, bound and tie rule) with the point-to-plane sums: for a pair (p', q)
+// with target normal n, r = (p' - q) . n and J = [p' x n, n], p' relative to ip.origin, all in double.  Lane j adds up term
+// j of ICP_PLANE_NSUMS over the warp's correspondences in the warp's query order: count, sum d2, the 21 entries J_a J_b with
+// a <= b (row-major), the 6 entries J_a r; term 29 is the non-finite count of both clouds when ip.check is set.  The warp
+// stores them in partial[warp][ICP_PLANE_NSUMS]; icp_plane_reduce_kernel adds them up in warp order.
+__global__ void __launch_bounds__(ICP_THREADS) icp_plane_match_kernel(const cwipc_point *__restrict__ src, uint32_t ns, const cwipc_point *__restrict__ tgt, uint32_t nt,
+                                                                      const cwipc_point *__restrict__ spts, const uint64_t *__restrict__ sorted, const __grid_constant__ GridParams gp,
+                                                                      const uint2 *__restrict__ table, uint32_t leaf_points, const __grid_constant__ IcpParams ip,
+                                                                      const float4 *__restrict__ normals, double *__restrict__ partial) {
+    __shared__ __align__(16) FarNode s_stack[ICP_WARPS][KF_STACK];
+    const unsigned lane = lane_id(), warp = threadIdx.x >> 5;
+    const uint32_t gwarp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, warps_total = (gridDim.x * blockDim.x) >> 5;
+    const Point16 *spts16 = reinterpret_cast<const Point16 *>(spts);
+    // the (a, b) of this lane's term: J_a J_b for lanes 2..22, J_a r for lanes 23..28
+    int ja = 0, jb = 0;
+    if (lane >= 2 && lane < 23) {
+        int t = (int)lane - 2;
+        while (t >= 6 - ja) t -= 6 - ja++;
+        jb = ja + t;
+    } else if (lane >= 23 && lane < 29) {
+        ja = (int)lane - 23;
+    }
+    double acc = 0.0;
+    for (uint32_t qi = gwarp; qi < ns; qi += warps_total) {
+        const Point16 p = ld_point(src, qi);
+        Point16 q;
+        q.x = affine_row(ip.m, p.x, p.y, p.z);
+        q.y = affine_row(ip.m + 4, p.x, p.y, p.z);
+        q.z = affine_row(ip.m + 8, p.x, p.y, p.z);
+        q.rgbt = 0u;
+        if (!finite_point(q)) continue; // (a non-finite input point, counted below; or a float overflow of the motion)
+        const uint64_t key = icp_nearest(q, ip.limit, ip.slack, spts16, sorted, gp, table, leaf_points, s_stack[warp]);
+        if (key == ~0ull) continue;
+        const Point16 t = ld_point(tgt, (uint32_t)key);
+        const float4 nf = normals[(uint32_t)key];
+        const double nv[3] = {(double)nf.x, (double)nf.y, (double)nf.z};
+        const double pr[3] = {(double)q.x - ip.origin[0], (double)q.y - ip.origin[1], (double)q.z - ip.origin[2]};
+        const double qr[3] = {(double)t.x - ip.origin[0], (double)t.y - ip.origin[1], (double)t.z - ip.origin[2]};
+        const double r = ((pr[0] - qr[0]) * nv[0] + (pr[1] - qr[1]) * nv[1]) + (pr[2] - qr[2]) * nv[2];
+        const double J[6] = {pr[1] * nv[2] - pr[2] * nv[1], pr[2] * nv[0] - pr[0] * nv[2], pr[0] * nv[1] - pr[1] * nv[0], nv[0], nv[1], nv[2]};
+        double term = 0.0;
+        if (lane == 0) term = 1.0;
+        else if (lane == 1) term = (double)__uint_as_float((uint32_t)(key >> 32));
+        else if (lane < 23) term = pick6(J, ja) * pick6(J, jb);
+        else if (lane < 29) term = pick6(J, ja) * r;
+        acc += term;
+    }
+    if (ip.check) {
+        uint32_t bad = 0;
+        for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < ns; i += gridDim.x * blockDim.x) bad += finite_point(ld_point_stream(src, i)) ? 0u : 1u;
+        for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < nt; i += gridDim.x * blockDim.x) bad += finite_point(ld_point_stream(tgt, i)) ? 0u : 1u;
+        bad = warp_sum(bad);
+        if (lane == ICP_PLANE_NSUMS - 1) acc = (double)bad;
+    }
+    if (lane < ICP_PLANE_NSUMS) partial[(size_t)gwarp * ICP_PLANE_NSUMS + lane] = acc;
+}
+
+// icp_reduce_kernel's fixed order for the ICP_PLANE_NSUMS sums of icp_plane_match_kernel.
+__global__ void __launch_bounds__(ICP_PLANE_NSUMS * 32) icp_plane_reduce_kernel(const double *__restrict__ partial, uint32_t nwarps, double *__restrict__ out) {
+    const unsigned lane = lane_id(), j = threadIdx.x >> 5;
+    double s = 0.0;
+    for (uint32_t w = lane; w < nwarps; w += 32) s += partial[(size_t)w * ICP_PLANE_NSUMS + j];
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(FULL_MASK, s, o);
     if (lane == 0) out[j] = s;
@@ -1873,58 +2094,93 @@ struct IcpMatcher::Impl {
     int dev;
     cudaStream_t s;
     uint32_t max_warps;
-    Scratch partial; // [max_warps + 1][ICP_NSUMS]: the warps' sums, then the totals
+    Scratch partial; // [max_warps + 1][nsums]: the warps' sums, then the totals
+    Scratch normals; // point-to-plane: float4 per target point, input order (icp_normals_kernel)
+
+    Impl(const cwipc_point *target, size_t nt, float hint_spacing, const float *bounds, int k, int nsums, int dev, cudaStream_t s) : target(target), nt(nt), dev(dev), s(s) {
+        float box[6];
+        if (bounds) {
+            memcpy(box, bounds, sizeof(box));
+        } else {
+            global_bbox(target, nt, box, box + 3, dev, s);
+            for (int a = 0; a < 6; a++)
+                if (!std::isfinite(box[a])) throw CudaError{cudaErrorInvalidValue, "the target contains non-finite coordinates"};
+        }
+        float maxabs = 0.f;
+        for (int a = 0; a < 3; a++) {
+            origin[a] = 0.5 * ((double)box[a] + (double)box[3 + a]);
+            maxabs = std::max(maxabs, std::max(std::fabs(box[a]), std::fabs(box[3 + a])));
+        }
+        build_index(ix, target, nt, k, hint_spacing, box, dev, s);
+        // a node's box corners are rounded to float like the points themselves: allow a few units in the last place of the
+        // largest coordinate besides the 0.01 pitch of cell_u's rounding
+        slack = std::max(0.01f * ix.gp.h, 8.f * std::ldexp(maxabs, -23));
+        max_warps = (uint32_t)sm_count(dev) * ICP_BLOCKS_PER_SM * ICP_WARPS;
+        partial = Scratch(((size_t)max_warps + 1) * nsums * sizeof(double), s);
+    }
+    unsigned grid(size_t n) const { return (unsigned)std::max<size_t>(1, std::min(div_up(n, (size_t)ICP_WARPS), (size_t)sm_count(dev) * ICP_BLOCKS_PER_SM)); }
 };
 
-IcpMatcher::IcpMatcher(const cwipc_point *target, size_t nt, float hint_spacing, const float *bounds, int dev, cudaStream_t s) : m(new Impl) {
-    m->target = target;
-    m->nt = nt;
-    m->dev = dev;
-    m->s = s;
-    float box[6];
-    if (bounds) {
-        memcpy(box, bounds, sizeof(box));
-    } else {
-        global_bbox(target, nt, box, box + 3, dev, s);
-        for (int a = 0; a < 6; a++)
-            if (!std::isfinite(box[a])) throw CudaError{cudaErrorInvalidValue, "the target contains non-finite coordinates"};
-    }
-    float maxabs = 0.f;
-    for (int a = 0; a < 3; a++) {
-        m->origin[a] = 0.5 * ((double)box[a] + (double)box[3 + a]);
-        maxabs = std::max(maxabs, std::max(std::fabs(box[a]), std::fabs(box[3 + a])));
-    }
-    build_index(m->ix, target, nt, 1, hint_spacing, box, dev, s);
-    // a node's box corners are rounded to float like the points themselves: allow a few units in the last place of the
-    // largest coordinate besides the 0.01 pitch of cell_u's rounding
-    m->slack = std::max(0.01f * m->ix.gp.h, 8.f * std::ldexp(maxabs, -23));
-    m->max_warps = (uint32_t)sm_count(dev) * ICP_BLOCKS_PER_SM * ICP_WARPS;
-    m->partial = Scratch(((size_t)m->max_warps + 1) * ICP_NSUMS * sizeof(double), s);
+IcpMatcher::IcpMatcher(const cwipc_point *target, size_t nt, float hint_spacing, const float *bounds, int dev, cudaStream_t s)
+    : m(new Impl(target, nt, hint_spacing, bounds, 1, ICP_NSUMS, dev, s)) {}
+
+IcpMatcher::IcpMatcher(const cwipc_point *target, size_t nt, float hint_spacing, const float *bounds, int dev, cudaStream_t s, double normal_radius, int normal_max_nn)
+    : m(new Impl(target, nt, hint_spacing, bounds, normal_max_nn, ICP_PLANE_NSUMS, dev, s)) {
+    m->normals = Scratch(nt * sizeof(float4), s);
+    const float limit = (float)(normal_radius * normal_radius);
+    launch("icp_normals_kernel", s, 16 * nt, [&] {
+        icp_normals_kernel<<<m->grid(nt), ICP_THREADS, 0, s>>>(target, (uint32_t)nt, m->ix.spts.as<cwipc_point>(), m->ix.sorted, m->ix.gp, m->ix.table.as<uint2>(), FAR_LEAF_POINTS, limit,
+                                                            m->slack, normal_max_nn, m->normals.as<float4>());
+    });
 }
 
 IcpMatcher::~IcpMatcher() = default;
 
 const double *IcpMatcher::origin() const { return m->origin; }
 
-void IcpMatcher::evaluate(const cwipc_point *source, size_t ns, const double motion[16], float limit, bool check_finite, double sums[ICP_NSUMS]) {
+int IcpMatcher::nsums() const { return m->normals.p ? ICP_PLANE_NSUMS : ICP_NSUMS; }
+
+void IcpMatcher::evaluate(const cwipc_point *source, size_t ns, const double motion[16], float limit, bool check_finite, double *sums) {
     IcpParams ip;
     memcpy(ip.m, motion, sizeof(ip.m));
     memcpy(ip.origin, m->origin, sizeof(ip.origin));
     ip.limit = limit;
     ip.slack = m->slack;
     ip.check = check_finite ? 1u : 0u;
-    const unsigned grid = (unsigned)std::max<size_t>(1, std::min(div_up(ns, (size_t)ICP_WARPS), (size_t)sm_count(m->dev) * ICP_BLOCKS_PER_SM));
+    const unsigned grid = m->grid(ns);
     const uint32_t nwarps = grid * ICP_WARPS;
-    double *partial = m->partial.as<double>(), *d_out = partial + (size_t)m->max_warps * ICP_NSUMS;
-    launch("icp_match_kernel", m->s, 16 * ns, [&] {
-        icp_match_kernel<<<grid, ICP_THREADS, 0, m->s>>>(source, (uint32_t)ns, m->target, (uint32_t)m->nt, m->ix.spts.as<cwipc_point>(), m->ix.sorted, m->ix.gp, m->ix.table.as<uint2>(),
-                                                        FAR_LEAF_POINTS, ip, partial);
-    });
-    launch("icp_reduce_kernel", m->s, 8 * (size_t)nwarps * ICP_NSUMS, [&] { icp_reduce_kernel<<<1, ICP_NSUMS * 32, 0, m->s>>>(partial, nwarps, d_out); });
-    double *h = static_cast<double *>(thread_pinned(ICP_NSUMS * sizeof(double)));
-    CWCU_CHECK(cudaMemcpyAsync(h, d_out, ICP_NSUMS * sizeof(double), cudaMemcpyDeviceToHost, m->s));
+    const int nsum = nsums();
+    double *partial = m->partial.as<double>(), *d_out = partial + (size_t)m->max_warps * nsum;
+    if (!m->normals.p) {
+        launch("icp_match_kernel", m->s, 16 * ns, [&] {
+            icp_match_kernel<<<grid, ICP_THREADS, 0, m->s>>>(source, (uint32_t)ns, m->target, (uint32_t)m->nt, m->ix.spts.as<cwipc_point>(), m->ix.sorted, m->ix.gp, m->ix.table.as<uint2>(),
+                                                            FAR_LEAF_POINTS, ip, partial);
+        });
+        launch("icp_reduce_kernel", m->s, 8 * (size_t)nwarps * ICP_NSUMS, [&] { icp_reduce_kernel<<<1, ICP_NSUMS * 32, 0, m->s>>>(partial, nwarps, d_out); });
+    } else {
+        launch("icp_plane_match_kernel", m->s, 16 * ns, [&] {
+            icp_plane_match_kernel<<<grid, ICP_THREADS, 0, m->s>>>(source, (uint32_t)ns, m->target, (uint32_t)m->nt, m->ix.spts.as<cwipc_point>(), m->ix.sorted, m->ix.gp,
+                                                                  m->ix.table.as<uint2>(), FAR_LEAF_POINTS, ip, m->normals.as<float4>(), partial);
+        });
+        launch("icp_plane_reduce_kernel", m->s, 8 * (size_t)nwarps * ICP_PLANE_NSUMS,
+               [&] { icp_plane_reduce_kernel<<<1, ICP_PLANE_NSUMS * 32, 0, m->s>>>(partial, nwarps, d_out); });
+    }
+    double *h = static_cast<double *>(thread_pinned(nsum * sizeof(double)));
+    CWCU_CHECK(cudaMemcpyAsync(h, d_out, nsum * sizeof(double), cudaMemcpyDeviceToHost, m->s));
     stream_sync(m->s);
-    memcpy(sums, h, ICP_NSUMS * sizeof(double));
+    memcpy(sums, h, nsum * sizeof(double));
+}
+
+bool IcpMatcher::normals_to_host(float *out) {
+    float4 *h = static_cast<float4 *>(thread_pinned(m->nt * sizeof(float4)));
+    CWCU_CHECK(cudaMemcpyAsync(h, m->normals.p, m->nt * sizeof(float4), cudaMemcpyDeviceToHost, m->s));
+    stream_sync(m->s);
+    bool finite = true;
+    for (size_t i = 0; i < m->nt; i++) {
+        out[3 * i] = h[i].x, out[3 * i + 1] = h[i].y, out[3 * i + 2] = h[i].z;
+        finite = finite && h[i].w == 0.f;
+    }
+    return finite;
 }
 
 } // namespace cwcu

@@ -371,6 +371,43 @@ struct cwipc_cuda_icp_result {
 };
 _CWIPC_UTIL_EXPORT int cwipc_cuda_icp(cwipc_pointcloud *source, cwipc_pointcloud *target, const double init[16], double max_correspondence_distance, int max_iterations,
                                       double relative_fitness, double relative_rmse, struct cwipc_cuda_icp_result *result);
+/* Unit normal of every point, estimated from its neighbourhood (open3d estimate_normals with
+ * KDTreeSearchParamHybrid(radius, max_nn)); copied to normals[3 * count], in the cloud's order.  Returns count or -1.
+ *   Neighbourhood of point i: at most max_nn points of the same cloud, i itself included: those with the smallest keys
+ *   (d2, index) among the points with d2 <= (float)(radius^2), the square taken in double.  d2 = ((dx*dx + dy*dy) + dz*dz)
+ *   with every operation rounded to float, as in cwipc_cuda_icp; of equal d2 the smaller index in the cloud's order wins.
+ *   Normal: the covariance of the neighbourhood, in double and relative to its mean (two passes, so that clouds far from
+ *   the origin stay accurate); the unit eigenvector of its smallest eigenvalue, found in double and rounded to float.  Its
+ *   sign is not specified (point-to-plane ICP uses only n n^T and r . n).  The normal is (0, 0, 0) when the neighbourhood
+ *   has fewer than 3 points or when the covariance is zero (all neighbours coincide); open3d writes (0, 0, 1) there.
+ *   Results are bit-identical from run to run.  3 <= max_nn <= 32 (one warp holds the list, one key per lane).
+ *   Errors: radius not finite or not > 0, max_nn outside [3, 32], normals == NULL, nfloats < 3 * count, or non-finite
+ *   coordinates give -1 and one ERROR log naming cwipc_cuda_estimate_normals; the cloud stays usable.  NULL pc: -1,
+ *   silently, before any argument check.  An empty cloud returns 0.
+ *   Cost: one search index and one normal kernel over the cloud, one copy to the host. */
+_CWIPC_UTIL_EXPORT int cwipc_cuda_estimate_normals(cwipc_pointcloud *pc, double radius, int max_nn, float *normals, size_t nfloats);
+/* Point-to-plane ICP of `source` against `target` (open3d registration_icp with TransformationEstimationPointToPlane),
+ * the target's normals as cwipc_cuda_estimate_normals(target, normal_radius, normal_max_nn).
+ *   Evaluation is exactly cwipc_cuda_icp's: the same correspondences, tie rule, fitness and inlier_rmse (the Euclidean
+ *   rmse, as in open3d, not the point-to-plane residual).  So with max_iterations = 0 both calls return the same
+ *   correspondences, fitness and inlier_rmse, bit for bit.
+ *   Update: for every correspondence (p', q) with target normal n, r = (p' - q) . n and J = [p' x n, n], both in double and
+ *   relative to the centre of the target's box.  x = (alpha, beta, gamma, tx, ty, tz) is the minimum-norm least-squares
+ *   solution of (sum J J^T) x = -sum J r, from a symmetric eigen-decomposition in double that drops the eigenvalues
+ *   <= 1e-12 times the largest; a zero system (every pair has a zero normal) gives x = 0.  So on a plane the motions the
+ *   data cannot see (sliding along it, turning about its normal) stay 0, not NaN.  open3d solves with LDLT instead.
+ *   dT = [Rz(gamma) Ry(beta) Rx(alpha), t] (open3d's TransformVector6dToMatrix4d) about the box centre, shifted back to
+ *   the cloud's coordinates, and T <- dT * T.  The loop, the stopping rule, the stop with fewer than 3 correspondences,
+ *   the application of T to the ORIGINAL source points, the result and the empty-cloud rules are cwipc_cuda_icp's.
+ *   Errors: those of cwipc_cuda_icp, and normal_radius not finite or not > 0 or normal_max_nn outside [3, 32]: -1 and one
+ *   ERROR log naming cwipc_cuda_icp_point_to_plane; the inputs stay usable.  NULL source or target: -1, silently, before
+ *   any argument check.
+ *   Cost: one search index (pitched for normal_max_nn neighbours) and one normal kernel over the target per call, then per
+ *   iteration one search kernel, one reduction kernel and one read-back of 30 numbers.  Results are bit-identical from
+ *   run to run and under concurrent callers. */
+_CWIPC_UTIL_EXPORT int cwipc_cuda_icp_point_to_plane(cwipc_pointcloud *source, cwipc_pointcloud *target, const double init[16], double max_correspondence_distance,
+                                                     int max_iterations, double relative_fitness, double relative_rmse, double normal_radius, int normal_max_nn,
+                                                     struct cwipc_cuda_icp_result *result);
 /* Per-point mean k-neighbour distance of cwipc_remove_outliers' first pass, copied to host
  * (dist[count]); returns count or -1.  Diagnostic hook used by the parity tests. */
 _CWIPC_UTIL_EXPORT int cwipc_cuda_knn_mean_distances(cwipc_pointcloud *pc, int kNeighbors, float *dist, size_t ndist);

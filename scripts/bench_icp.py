@@ -13,7 +13,12 @@ library's launch profile (CUDA events) in a separate call; `ref_s` the reference
 The recovered matrices must agree: rotation within 1e-6 and the motion of the camera's centre within 1e-5 m.  The
 card's name and power limit are read, never set.
 
-    python scripts/bench_icp.py [--reps 5]
+--point-to-plane times cwipc_icp_point_to_plane on the same rows instead (normals from KDTreeSearchParamHybrid(normal_radius,
+30), normal_radius = 0.01 on the raw frame and 0.02 after the downsample), against tests/icp_plane_reference.py.
+`index_ms` then also holds icp_normals_kernel (reported on its own as `normals_ms`), and `per_iter_ms` is
+icp_plane_match_kernel + icp_plane_reduce_kernel.
+
+    python scripts/bench_icp.py [--reps 5] [--point-to-plane]
 """
 import argparse
 import ctypes
@@ -34,6 +39,8 @@ sys.dont_write_bytecode = True
 INDEX_KERNELS = ("bbox_octree_kernel", "knn_keygen_kernel", "radix_cluster_kernel", "radix_fused_kernel", "radix_hist_kernel", "radix_onesweep_kernel",
                  "radix_scan_kernel", "knn_layout_kernel")
 EVAL_KERNELS = ("icp_match_kernel", "icp_reduce_kernel")
+PLANE_EVAL_KERNELS = ("icp_plane_match_kernel", "icp_plane_reduce_kernel")
+NORMAL_RADIUS = {"raw 1 M": 0.01, "downsample_pertile(0.005)": 0.02}
 
 
 def card():
@@ -59,10 +66,14 @@ def pose(seed, centre):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--reps", type=int, default=5)
+    ap.add_argument("--point-to-plane", action="store_true", help="time cwipc_icp_point_to_plane instead of cwipc_icp")
     args = ap.parse_args()
     import cwipc_util_b200 as cw
     from cwipc_util_b200 import synthetic
     import icp_reference as ref
+    import icp_plane_reference as pref
+    plane = args.point_to_plane
+    eval_kernels = PLANE_EVAL_KERNELS if plane else EVAL_KERNELS
     lib = cw.util.cwipc_util_dll_load()
     if cw.cuda_device_count() <= 0:
         raise SystemExit("bench_icp.py: no CUDA device")
@@ -78,7 +89,7 @@ def main():
         lib.cwipc_cuda_profile_report(buf, need)
         return out, json.loads(buf.value.decode())
 
-    res = {"card": card(), "reps": args.reps, "rows": []}
+    res = {"card": card(), "reps": args.reps, "estimation": "point-to-plane" if plane else "point-to-point", "rows": []}
     print(json.dumps(res["card"]), file=sys.stderr)
     raw = cw.cwipc_from_numpy_array(synthetic.camera_cloud(1000000, seed=1), 1)
     for size, pc in (("raw 1 M", raw), ("downsample_pertile(0.005)", cw.cwipc_downsample_pertile(raw, 0.005))):
@@ -88,7 +99,10 @@ def main():
             P = pose(100 + tile, centre)
             src = cw.cwipc_transform(cam, P)
             tgt = cw.cwipc_tilefilter_masked(pc, ~tile & 0xff)
-            call = lambda: cw.cwipc_icp(src, tgt, 0.05, max_iterations=30)
+            if plane:
+                call = lambda: cw.cwipc_icp_point_to_plane(src, tgt, 0.05, NORMAL_RADIUS[size], max_iterations=30)
+            else:
+                call = lambda: cw.cwipc_icp(src, tgt, 0.05, max_iterations=30)
             call()  # warm-up
             walls = []
             for _ in range(args.reps):
@@ -97,12 +111,19 @@ def main():
                 r = call()
                 walls.append((time.perf_counter() - t0) * 1e3)
             r, prof = profiled(call)
-            index_ms = sum(prof[k]["total_ms"] for k in INDEX_KERNELS if k in prof)
-            evals = prof["icp_match_kernel"]["launches"]
-            per_iter = sum(prof[k]["total_ms"] for k in EVAL_KERNELS) / evals
+            normals_ms = prof["icp_normals_kernel"]["total_ms"] if plane else 0.0
+            index_ms = sum(prof[k]["total_ms"] for k in INDEX_KERNELS if k in prof) + normals_ms
+            evals = prof[eval_kernels[0]]["launches"]
+            per_iter = sum(prof[k]["total_ms"] for k in eval_kernels) / evals
             S, T = ref.xyz32(src.get_numpy_array()), ref.xyz32(tgt.get_numpy_array())
             t0 = time.perf_counter()
-            want = ref.icp(S, T, 0.05, max_iterations=30)
+            if plane:
+                # the library takes the centre of the box the target carries: its own on the raw frame, the whole frame's
+                # after cwipc_downsample_pertile (which hands the input's box on)
+                origin = pref.box_centre(T if pc is raw else ref.xyz32(raw.get_numpy_array()))
+                want = pref.icp_point_to_plane(S, T, 0.05, NORMAL_RADIUS[size], max_iterations=30, origin=origin)
+            else:
+                want = ref.icp(S, T, 0.05, max_iterations=30)
             ref_s = time.perf_counter() - t0
             d = r.matrix - want.matrix
             agree = bool(np.abs(d[:3, :3]).max() < 1e-6 and np.abs(d[:3, :3] @ centre + d[:3, 3]).max() < 1e-5)
@@ -110,7 +131,7 @@ def main():
             row = {"size": size, "camera": tile, "source_points": cam.count(), "target_points": tgt.count(), "iterations": r.iterations,
                    "fitness": round(r.fitness, 6), "inlier_rmse": r.inlier_rmse, "call_ms": round(float(np.median(walls)), 3),
                    "call_range_ms": [round(min(walls), 3), round(max(walls), 3)], "index_ms": round(index_ms, 3), "per_iter_ms": round(per_iter, 3),
-                   "evaluations": evals, "ref_s": round(ref_s, 2), "ref_iterations": want.iterations, "matrices_agree": agree,
+                   "evaluations": evals, **({"normals_ms": round(normals_ms, 3)} if plane else {}), "ref_s": round(ref_s, 2), "ref_iterations": want.iterations, "matrices_agree": agree,
                    "residual_deg": float(np.degrees(np.arccos(np.clip((np.trace(E[:3, :3]) - 1) / 2, -1, 1)))),
                    "residual_centre_m": float(np.linalg.norm(E[:3, :3] @ centre + E[:3, 3] - centre))}
             res["rows"].append(row)
