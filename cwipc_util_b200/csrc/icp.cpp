@@ -1,8 +1,8 @@
-// icp.cpp -- cwipc_cuda_icp and cwipc_cuda_icp_point_to_plane: ICP of one device-resident cloud against another, the fine
-// step of multi-camera registration (python/cwipc/registration/: open3d's registration_icp with
-// TransformationEstimationPointToPoint or PointToPlane), and cwipc_cuda_estimate_normals.  The correspondences and their
-// sums come from the target's search index in outliers.cu (IcpMatcher); the host solves the motion from those 18 or 30
-// numbers per iteration and runs the loop.
+// icp.cpp -- cwipc_cuda_icp, cwipc_cuda_icp_point_to_plane and cwipc_cuda_icp_colored: ICP of one device-resident cloud
+// against another, the fine step of multi-camera registration (python/cwipc/registration/: open3d's registration_icp with
+// TransformationEstimationPointToPoint or PointToPlane, and registration_colored_icp), with cwipc_cuda_estimate_normals and
+// cwipc_cuda_estimate_color_gradients.  The correspondences and their sums come from the target's search index in
+// outliers.cu (IcpMatcher); the host solves the motion from those 18 or 30 numbers per iteration and runs the loop.
 #include <cmath>
 #include <cstring>
 
@@ -187,13 +187,21 @@ void check_normal_args(double radius, int max_nn) {
     if (max_nn < 3 || max_nn > ICP_MAX_NN) bad("the normal max_nn must be in [3, " + std::to_string(ICP_MAX_NN) + "]");
 }
 
+void check_gradient_args(double radius, int max_nn) {
+    if (!(std::isfinite(radius) && radius > 0.0)) bad("the gradient radius must be finite and > 0");
+    if (max_nn < 4 || max_nn > ICP_MAX_NN) bad("the gradient max_nn must be in [4, " + std::to_string(ICP_MAX_NN) + "]");
+}
+
 struct PlaneOptions {
     double normal_radius;
     int normal_max_nn;
+    bool colored;            // colored ICP: also the target's colour gradients and the photometric rows
+    double lambda_geometric; // colored only
 };
 
-// The loop of open3d's RegistrationICP, shared by both entry points: point-to-point when plane is null, else point-to-plane
-// with the target's normals.  The estimation's solve is the one difference.
+// The loop of open3d's RegistrationICP, shared by the three entry points: point-to-point when plane is null, else
+// point-to-plane with the target's normals, or colored ICP with its normals and colour gradients.  The estimation's solve
+// is the one difference between point-to-point and the other two, which share plane_motion.
 int icp_entry(const char *who, cwipc_pointcloud *source, cwipc_pointcloud *target, const double init[16], double max_correspondence_distance, int max_iterations,
               double relative_fitness, double relative_rmse, const PlaneOptions *plane, struct cwipc_cuda_icp_result *result) {
     if (target == nullptr) return -1;
@@ -203,6 +211,8 @@ int icp_entry(const char *who, cwipc_pointcloud *source, cwipc_pointcloud *targe
         if (!(std::isfinite(relative_fitness) && relative_fitness >= 0.0 && std::isfinite(relative_rmse) && relative_rmse >= 0.0))
             bad("relative_fitness and relative_rmse must be finite and >= 0");
         if (plane) check_normal_args(plane->normal_radius, plane->normal_max_nn);
+        if (plane && plane->colored && !(std::isfinite(plane->lambda_geometric) && plane->lambda_geometric >= 0.0 && plane->lambda_geometric <= 1.0))
+            bad("lambda_geometric must be finite and in [0, 1]");
         double T[16] = {1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1};
         if (init) {
             for (int k = 0; k < 16; k++)
@@ -226,8 +236,11 @@ int icp_entry(const char *who, cwipc_pointcloud *source, cwipc_pointcloud *targe
                 memcpy(box + 3, tgt->bounds_max, 3 * sizeof(float));
             }
             const float *bounds = tgt->has_bounds ? box : nullptr;
-            IcpMatcher matcher = plane ? IcpMatcher(tgt->d_pts, tgt->count, target->cellsize(), bounds, dev, s, plane->normal_radius, plane->normal_max_nn)
-                                       : IcpMatcher(tgt->d_pts, tgt->count, target->cellsize(), bounds, dev, s);
+            // colored: open3d's RegistrationColoredICP takes the gradients of the 30 nearest points within 2 d
+            IcpMatcher matcher = !plane ? IcpMatcher(tgt->d_pts, tgt->count, target->cellsize(), bounds, dev, s)
+                                 : !plane->colored ? IcpMatcher(tgt->d_pts, tgt->count, target->cellsize(), bounds, dev, s, plane->normal_radius, plane->normal_max_nn)
+                                                   : IcpMatcher(tgt->d_pts, tgt->count, target->cellsize(), bounds, dev, s, plane->normal_radius, plane->normal_max_nn,
+                                                                2.0 * max_correspondence_distance, 30, plane->lambda_geometric);
             const float limit = (float)(max_correspondence_distance * max_correspondence_distance);
             double sums[ICP_PLANE_NSUMS];
             matcher.evaluate(src->d_pts, ns, T, limit, true, sums);
@@ -268,8 +281,35 @@ int cwipc_cuda_icp(cwipc_pointcloud *source, cwipc_pointcloud *target, const dou
 // The same loop with point-to-plane estimation against the target's normals (see include/cwipc_util_cuda.h).
 int cwipc_cuda_icp_point_to_plane(cwipc_pointcloud *source, cwipc_pointcloud *target, const double init[16], double max_correspondence_distance, int max_iterations,
                                   double relative_fitness, double relative_rmse, double normal_radius, int normal_max_nn, struct cwipc_cuda_icp_result *result) {
-    const PlaneOptions plane{normal_radius, normal_max_nn};
+    const PlaneOptions plane{normal_radius, normal_max_nn, false, 1.0};
     return icp_entry("cwipc_cuda_icp_point_to_plane", source, target, init, max_correspondence_distance, max_iterations, relative_fitness, relative_rmse, &plane, result);
+}
+
+// The same loop with colored ICP's estimation against the target's normals and colour gradients (see include/cwipc_util_cuda.h).
+int cwipc_cuda_icp_colored(cwipc_pointcloud *source, cwipc_pointcloud *target, const double init[16], double max_correspondence_distance, int max_iterations,
+                           double relative_fitness, double relative_rmse, double normal_radius, int normal_max_nn, double lambda_geometric,
+                           struct cwipc_cuda_icp_result *result) {
+    const PlaneOptions colored{normal_radius, normal_max_nn, true, lambda_geometric};
+    return icp_entry("cwipc_cuda_icp_colored", source, target, init, max_correspondence_distance, max_iterations, relative_fitness, relative_rmse, &colored, result);
+}
+
+int cwipc_cuda_estimate_color_gradients(cwipc_pointcloud *pc, double normal_radius, int normal_max_nn, double radius, int max_nn, float *gradients, size_t nfloats) {
+    return read_entry<int>("cwipc_cuda_estimate_color_gradients", pc, -1, [&](const StoragePtr &in, int dev, cudaStream_t s) -> int {
+        check_normal_args(normal_radius, normal_max_nn);
+        check_gradient_args(radius, max_nn);
+        if (gradients == nullptr) bad("gradients must not be NULL");
+        if (nfloats < 3 * in->count) bad("gradients holds " + std::to_string(nfloats) + " floats, " + std::to_string(3 * in->count) + " are needed");
+        if (in->count == 0) return 0;
+        float box[6];
+        if (in->has_bounds) {
+            memcpy(box, in->bounds_min, 3 * sizeof(float));
+            memcpy(box + 3, in->bounds_max, 3 * sizeof(float));
+        }
+        // (the weight only matters to evaluate, which the hook does not call)
+        IcpMatcher matcher(in->d_pts, in->count, pc->cellsize(), in->has_bounds ? box : nullptr, dev, s, normal_radius, normal_max_nn, radius, max_nn, 1.0);
+        if (!matcher.gradients_to_host(gradients)) bad("the cloud contains non-finite coordinates");
+        return (int)in->count;
+    });
 }
 
 int cwipc_cuda_estimate_normals(cwipc_pointcloud *pc, double radius, int max_nn, float *normals, size_t nfloats) {

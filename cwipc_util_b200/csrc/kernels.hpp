@@ -145,7 +145,9 @@ void scatter_floats(const float *values, const uint32_t *idx, size_t n, float *o
 //   point-to-point (ICP_NSUMS): [0] count, [1] sum d2, [2..4] sum p', [5..7] sum q, [8..16] sum p'_a q_b (row-major a, b),
 //     [17] with check_finite: the number of points of either cloud with a non-finite coordinate (else 0);
 //   point-to-plane (ICP_PLANE_NSUMS), with n the target normal of q, r = (p' - q) . n and J = [p' x n, n]: [0] count,
-//     [1] sum d2, [2..22] sum J_a J_b (a <= b, row-major), [23..28] sum J_a r, [29] the non-finite count as above.
+//     [1] sum d2, [2..22] sum J_a J_b (a <= b, row-major), [23..28] sum J_a r, [29] the non-finite count as above;
+//   colored (ICP_PLANE_NSUMS, the same layout): J J^T and J r summed over the geometric and the photometric row of every
+//     pair (cwipc_cuda_icp_colored in include/cwipc_util_cuda.h).
 // One search kernel, one reduction kernel and one read-back per evaluation; the same bits on every run.
 constexpr int ICP_NSUMS = 18;
 constexpr int ICP_PLANE_NSUMS = 30;
@@ -157,12 +159,20 @@ public:
     // point-to-plane: the index with k = normal_max_nn (3..32), then the unit normal of every target point from its
     // normal_max_nn nearest points within normal_radius (cwipc_cuda_estimate_normals in include/cwipc_util_cuda.h)
     IcpMatcher(const cwipc_point *target, size_t nt, float hint_spacing, const float *bounds, int dev, cudaStream_t s, double normal_radius, int normal_max_nn);
+    // colored: point-to-plane's index and normals, then the colour gradient of every target point from its gradient_max_nn
+    // (4..32) nearest points within gradient_radius (cwipc_cuda_estimate_color_gradients in include/cwipc_util_cuda.h).
+    // evaluate weighs the geometric row by sqrt(lambda_geometric) and the photometric row by sqrt(1 - lambda_geometric).
+    IcpMatcher(const cwipc_point *target, size_t nt, float hint_spacing, const float *bounds, int dev, cudaStream_t s, double normal_radius, int normal_max_nn,
+               double gradient_radius, int gradient_max_nn, double lambda_geometric);
     ~IcpMatcher();
     const double *origin() const;
     int nsums() const; // ICP_NSUMS or ICP_PLANE_NSUMS
     void evaluate(const cwipc_point *source, size_t ns, const double motion[16], float limit, bool check_finite, double *sums);
-    // point-to-plane only: the normals, 3 floats per target point in its order; false when a target point has a non-finite coordinate
+    // point-to-plane and colored: the normals, 3 floats per target point in its order; false when a target point has a
+    // non-finite coordinate
     bool normals_to_host(float *out);
+    // colored only: the gradients, 3 floats per target point in its order; false as above
+    bool gradients_to_host(float *out);
 
 private:
     struct Impl;

@@ -1707,10 +1707,13 @@ __device__ __forceinline__ void jacobi3_rotate(double (&A)[3][3], double (&V)[3]
     }
 }
 
-// The unit eigenvector of the smallest eigenvalue of the symmetric 3x3 A, by cyclic Jacobi rotations in double (the same
-// rules as icp.cpp's horn_rotation: an off-diagonal entry below the rounding of both diagonal entries is dropped).
-__device__ __forceinline__ float3 smallest_eigenvector(double (&A)[3][3]) {
-    double V[3][3] = {{1.0, 0.0, 0.0}, {0.0, 1.0, 0.0}, {0.0, 0.0, 1.0}};
+// The eigen-decomposition of the symmetric 3x3 A by cyclic Jacobi rotations in double (the same rules as icp.cpp's
+// horn_rotation: an off-diagonal entry below the rounding of both diagonal entries is dropped): A ends diagonal, holding
+// the eigenvalues, and column k of V is the unit eigenvector of A[k][k].
+__device__ __forceinline__ void jacobi3_eigen(double (&A)[3][3], double (&V)[3][3]) {
+    V[0][0] = 1.0, V[0][1] = 0.0, V[0][2] = 0.0;
+    V[1][0] = 0.0, V[1][1] = 1.0, V[1][2] = 0.0;
+    V[2][0] = 0.0, V[2][1] = 0.0, V[2][2] = 1.0;
     for (int sweep = 0; sweep < 50 && !(A[0][1] == 0.0 && A[0][2] == 0.0 && A[1][2] == 0.0); sweep++) {
         if (sweep > 3) {
 #pragma unroll
@@ -1725,6 +1728,12 @@ __device__ __forceinline__ float3 smallest_eigenvector(double (&A)[3][3]) {
         jacobi3_rotate<0, 2>(A, V);
         jacobi3_rotate<1, 2>(A, V);
     }
+}
+
+// The unit eigenvector of the smallest eigenvalue of the symmetric 3x3 A.
+__device__ __forceinline__ float3 smallest_eigenvector(double (&A)[3][3]) {
+    double V[3][3];
+    jacobi3_eigen(A, V);
     const int m = A[0][0] <= A[1][1] ? (A[0][0] <= A[2][2] ? 0 : 2) : (A[1][1] <= A[2][2] ? 1 : 2);
     const double x = m == 0 ? V[0][0] : (m == 1 ? V[0][1] : V[0][2]);
     const double y = m == 0 ? V[1][0] : (m == 1 ? V[1][1] : V[1][2]);
@@ -1782,19 +1791,86 @@ __global__ void __launch_bounds__(ICP_THREADS) icp_normals_kernel(const cwipc_po
     }
 }
 
+// ---- colored ICP (cwipc_cuda_icp_colored, cwipc_cuda_estimate_color_gradients) ----------------------------------------------
+// The intensity of a point: ((double)r + g + b) / 765, an exact integer sum and one division.
+__device__ __forceinline__ double pt_intensity(const Point16 &p) { return (double)(pt_r(p) + pt_g(p) + pt_b(p)) / 765.0; }
+
+// One warp per point of the cloud, in cell order (grid-stride), after icp_normals_kernel: the colour gradient g of point i
+// (open3d's InitializePointCloudForColoredICP).  Its neighbourhood is the kk smallest keys (d2, index) of the cloud's points
+// with d2 <= limit (itself included), found by icp_neighbours, and n = normals[i].  Every neighbour j gives the row
+// A_j = d_j - (d_j . n) n with d_j = v_j - v_i and b_j = I_j - I_i; one more row (nn - 1) n with b = 0 keeps g in the tangent
+// plane.  The 6 entries of A^T A and the 3 of A^T b are summed in double over the lanes in a fixed butterfly order; g is the
+// minimum-norm solution of (A^T A) g = A^T b from jacobi3_eigen, the eigenvalues <= 1e-12 times the largest dropped.
+// gradients[i] (input order) = (gx, gy, gz, 0); (0, 0, 0, 0) for fewer than 4 neighbours or a zero normal; (0, 0, 0, 1) for
+// a point with a non-finite coordinate.
+__global__ void __launch_bounds__(ICP_THREADS) icp_gradients_kernel(const cwipc_point *__restrict__ pts, uint32_t n, const cwipc_point *__restrict__ spts,
+                                                                    const uint64_t *__restrict__ sorted, const __grid_constant__ GridParams gp, const uint2 *__restrict__ table,
+                                                                    uint32_t leaf_points, float limit, float slack, int kk, const float4 *__restrict__ normals,
+                                                                    float4 *__restrict__ gradients) {
+    __shared__ __align__(16) FarNode s_stack[ICP_WARPS][KF_STACK];
+    const unsigned lane = lane_id(), warp = threadIdx.x >> 5;
+    const uint32_t gwarp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, warps_total = (gridDim.x * blockDim.x) >> 5;
+    const Point16 *spts16 = reinterpret_cast<const Point16 *>(spts);
+    const uint64_t idxmask = (1ull << gp.idxbits) - 1ull;
+    for (uint32_t c = gwarp; c < n; c += warps_total) {
+        const Point16 q = spts16[c]; // (the cell-ordered copy holds the colour too)
+        const uint32_t self = (uint32_t)(sorted[c] & idxmask);
+        float4 out = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (!finite_point(q)) {
+            out.w = 1.f;
+        } else {
+            const float4 nf = normals[self];
+            const uint64_t key = icp_neighbours(q, limit, slack, kk, spts16, sorted, gp, table, leaf_points, s_stack[warp]);
+            const bool have = key != ~0ull;
+            const int cnt = __popc(__ballot_sync(FULL_MASK, have));
+            if (cnt >= 4 && !(nf.x == 0.f && nf.y == 0.f && nf.z == 0.f)) {
+                const double nv[3] = {(double)nf.x, (double)nf.y, (double)nf.z};
+                double row[3] = {0.0, 0.0, 0.0}, b = 0.0;
+                if (have) {
+                    const Point16 t = ld_point(pts, (uint32_t)(key & idxmask));
+                    const double d[3] = {(double)t.x - (double)q.x, (double)t.y - (double)q.y, (double)t.z - (double)q.z};
+                    const double dn = (d[0] * nv[0] + d[1] * nv[1]) + d[2] * nv[2];
+#pragma unroll
+                    for (int a = 0; a < 3; a++) row[a] = d[a] - dn * nv[a];
+                    b = pt_intensity(t) - pt_intensity(q);
+                }
+                const double w = (double)(cnt - 1);
+                const double cr[3] = {w * nv[0], w * nv[1], w * nv[2]};
+                double A[3][3], rhs[3];
+#pragma unroll
+                for (int a = 0; a < 3; a++) {
+#pragma unroll
+                    for (int c2 = a; c2 < 3; c2++) A[a][c2] = A[c2][a] = warp_sum(row[a] * row[c2]) + cr[a] * cr[c2];
+                    rhs[a] = warp_sum(row[a] * b);
+                }
+                double V[3][3];
+                jacobi3_eigen(A, V);
+                const double top = fmax(fmax(A[0][0], A[1][1]), A[2][2]);
+                double g[3] = {0.0, 0.0, 0.0};
+#pragma unroll
+                for (int e = 0; e < 3; e++) {
+                    if (!(A[e][e] > 1e-12 * top)) continue;
+                    const double vb = (V[0][e] * rhs[0] + V[1][e] * rhs[1]) + V[2][e] * rhs[2];
+#pragma unroll
+                    for (int k = 0; k < 3; k++) g[k] += V[k][e] * (vb / A[e][e]);
+                }
+                out.x = (float)g[0], out.y = (float)g[1], out.z = (float)g[2];
+            }
+        }
+        if (lane == 0) gradients[self] = out;
+    }
+}
+
 __device__ __forceinline__ double pick6(const double (&v)[6], int i) {
     return i == 0 ? v[0] : (i == 1 ? v[1] : (i == 2 ? v[2] : (i == 3 ? v[3] : (i == 4 ? v[4] : v[5]))));
 }
 
-// icp_match_kernel's correspondences (the same search, bound and tie rule) with the point-to-plane sums: for a pair (p', q)
-// with target normal n, r = (p' - q) . n and J = [p' x n, n], p' relative to ip.origin, all in double.  Lane j adds up term
-// j of ICP_PLANE_NSUMS over the warp's correspondences in the warp's query order: count, sum d2, the 21 entries J_a J_b with
-// a <= b (row-major), the 6 entries J_a r; term 29 is the non-finite count of both clouds when ip.check is set.  The warp
-// stores them in partial[warp][ICP_PLANE_NSUMS]; icp_plane_reduce_kernel adds them up in warp order.
-__global__ void __launch_bounds__(ICP_THREADS) icp_plane_match_kernel(const cwipc_point *__restrict__ src, uint32_t ns, const cwipc_point *__restrict__ tgt, uint32_t nt,
-                                                                      const cwipc_point *__restrict__ spts, const uint64_t *__restrict__ sorted, const __grid_constant__ GridParams gp,
-                                                                      const uint2 *__restrict__ table, uint32_t leaf_points, const __grid_constant__ IcpParams ip,
-                                                                      const float4 *__restrict__ normals, double *__restrict__ partial) {
+// The body of icp_plane_match_kernel and icp_colored_match_kernel.  COLORED scales the point-to-plane row by sg and, when
+// sp != 0, adds the photometric row of the pair to the same 30 sums (see icp_colored_match_kernel).
+template <bool COLORED>
+__device__ __forceinline__ void plane_match(const cwipc_point *__restrict__ src, uint32_t ns, const cwipc_point *__restrict__ tgt, uint32_t nt, const cwipc_point *__restrict__ spts,
+                                            const uint64_t *__restrict__ sorted, const GridParams &gp, const uint2 *__restrict__ table, uint32_t leaf_points, const IcpParams &ip,
+                                            const float4 *__restrict__ normals, const float4 *__restrict__ gradients, double sg, double sp, double *__restrict__ partial) {
     __shared__ __align__(16) FarNode s_stack[ICP_WARPS][KF_STACK];
     const unsigned lane = lane_id(), warp = threadIdx.x >> 5;
     const uint32_t gwarp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, warps_total = (gridDim.x * blockDim.x) >> 5;
@@ -1826,12 +1902,35 @@ __global__ void __launch_bounds__(ICP_THREADS) icp_plane_match_kernel(const cwip
         const double qr[3] = {(double)t.x - ip.origin[0], (double)t.y - ip.origin[1], (double)t.z - ip.origin[2]};
         const double r = ((pr[0] - qr[0]) * nv[0] + (pr[1] - qr[1]) * nv[1]) + (pr[2] - qr[2]) * nv[2];
         const double J[6] = {pr[1] * nv[2] - pr[2] * nv[1], pr[2] * nv[0] - pr[0] * nv[2], pr[0] * nv[1] - pr[1] * nv[0], nv[0], nv[1], nv[2]};
-        double term = 0.0;
-        if (lane == 0) term = 1.0;
-        else if (lane == 1) term = (double)__uint_as_float((uint32_t)(key >> 32));
-        else if (lane < 23) term = pick6(J, ja) * pick6(J, jb);
-        else if (lane < 29) term = pick6(J, ja) * r;
-        acc += term;
+        if (!COLORED) {
+            double term = 0.0;
+            if (lane == 0) term = 1.0;
+            else if (lane == 1) term = (double)__uint_as_float((uint32_t)(key >> 32));
+            else if (lane < 23) term = pick6(J, ja) * pick6(J, jb);
+            else if (lane < 29) term = pick6(J, ja) * r;
+            acc += term;
+        } else {
+            const double JG[6] = {sg * J[0], sg * J[1], sg * J[2], sg * J[3], sg * J[4], sg * J[5]}, rG = sg * r;
+            double JI[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0}, rI = 0.0;
+            const bool photo = sp != 0.0;
+            if (photo) {
+                const float4 gf = gradients[(uint32_t)key];
+                const double g[3] = {(double)gf.x, (double)gf.y, (double)gf.z};
+                const double proj[3] = {(pr[0] - qr[0]) - r * nv[0], (pr[1] - qr[1]) - r * nv[1], (pr[2] - qr[2]) - r * nv[2]}; // p_proj - q
+                const double i0 = ((g[0] * proj[0] + g[1] * proj[1]) + g[2] * proj[2]) + pt_intensity(t);
+                const double gn = (g[0] * nv[0] + g[1] * nv[1]) + g[2] * nv[2];
+                const double d[3] = {-(g[0] - gn * nv[0]), -(g[1] - gn * nv[1]), -(g[2] - gn * nv[2])};
+                JI[0] = sp * (pr[1] * d[2] - pr[2] * d[1]), JI[1] = sp * (pr[2] * d[0] - pr[0] * d[2]), JI[2] = sp * (pr[0] * d[1] - pr[1] * d[0]);
+                JI[3] = sp * d[0], JI[4] = sp * d[1], JI[5] = sp * d[2];
+                rI = sp * (pt_intensity(p) - i0);
+            }
+            double term = 0.0;
+            if (lane == 0) term = 1.0;
+            else if (lane == 1) term = (double)__uint_as_float((uint32_t)(key >> 32));
+            else if (lane < 23) term = photo ? pick6(JG, ja) * pick6(JG, jb) + pick6(JI, ja) * pick6(JI, jb) : pick6(JG, ja) * pick6(JG, jb);
+            else if (lane < 29) term = photo ? pick6(JG, ja) * rG + pick6(JI, ja) * rI : pick6(JG, ja) * rG;
+            acc += term;
+        }
     }
     if (ip.check) {
         uint32_t bad = 0;
@@ -1841,6 +1940,33 @@ __global__ void __launch_bounds__(ICP_THREADS) icp_plane_match_kernel(const cwip
         if (lane == ICP_PLANE_NSUMS - 1) acc = (double)bad;
     }
     if (lane < ICP_PLANE_NSUMS) partial[(size_t)gwarp * ICP_PLANE_NSUMS + lane] = acc;
+}
+
+// icp_match_kernel's correspondences (the same search, bound and tie rule) with the point-to-plane sums: for a pair (p', q)
+// with target normal n, r = (p' - q) . n and J = [p' x n, n], p' relative to ip.origin, all in double.  Lane j adds up term
+// j of ICP_PLANE_NSUMS over the warp's correspondences in the warp's query order: count, sum d2, the 21 entries J_a J_b with
+// a <= b (row-major), the 6 entries J_a r; term 29 is the non-finite count of both clouds when ip.check is set.  The warp
+// stores them in partial[warp][ICP_PLANE_NSUMS]; icp_plane_reduce_kernel adds them up in warp order.
+__global__ void __launch_bounds__(ICP_THREADS) icp_plane_match_kernel(const cwipc_point *__restrict__ src, uint32_t ns, const cwipc_point *__restrict__ tgt, uint32_t nt,
+                                                                      const cwipc_point *__restrict__ spts, const uint64_t *__restrict__ sorted, const __grid_constant__ GridParams gp,
+                                                                      const uint2 *__restrict__ table, uint32_t leaf_points, const __grid_constant__ IcpParams ip,
+                                                                      const float4 *__restrict__ normals, double *__restrict__ partial) {
+    plane_match<false>(src, ns, tgt, nt, spts, sorted, gp, table, leaf_points, ip, normals, nullptr, 1.0, 0.0, partial);
+}
+
+// icp_plane_match_kernel with the colored-ICP sums (Park, Zhou and Koltun, ICCV 2017; open3d's
+// TransformationEstimationForColoredICP): for a pair (p', q) with target normal n, target gradient g = gradients[q] and
+// intensities I_s (source point) and I_t (target point), the geometric row J_G = sg [p' x n, n], r_G = sg (p' - q) . n and
+// the photometric row J_I = sp [p' x d, d], r_I = sp (I_s - I_0) with p_proj = p' - ((p' - q) . n) n,
+// I_0 = g . (p_proj - q) + I_t and d = -(g - (g . n) n).  Lanes 2..28 add J_G J_G^T + J_I J_I^T and J_G r_G + J_I r_I in
+// icp_plane_match_kernel's layout, so icp_plane_reduce_kernel adds them up.  sp == 0 (lambda_geometric = 1) skips the
+// photometric row, and with sg == 1 the sums are icp_plane_match_kernel's bit for bit.
+__global__ void __launch_bounds__(ICP_THREADS) icp_colored_match_kernel(const cwipc_point *__restrict__ src, uint32_t ns, const cwipc_point *__restrict__ tgt, uint32_t nt,
+                                                                        const cwipc_point *__restrict__ spts, const uint64_t *__restrict__ sorted, const __grid_constant__ GridParams gp,
+                                                                        const uint2 *__restrict__ table, uint32_t leaf_points, const __grid_constant__ IcpParams ip,
+                                                                        const float4 *__restrict__ normals, const float4 *__restrict__ gradients, double sg, double sp,
+                                                                        double *__restrict__ partial) {
+    plane_match<true>(src, ns, tgt, nt, spts, sorted, gp, table, leaf_points, ip, normals, gradients, sg, sp, partial);
 }
 
 // icp_reduce_kernel's fixed order for the ICP_PLANE_NSUMS sums of icp_plane_match_kernel.
@@ -2096,6 +2222,8 @@ struct IcpMatcher::Impl {
     uint32_t max_warps;
     Scratch partial; // [max_warps + 1][nsums]: the warps' sums, then the totals
     Scratch normals; // point-to-plane: float4 per target point, input order (icp_normals_kernel)
+    Scratch gradients; // colored: float4 per target point, input order (icp_gradients_kernel)
+    double sg = 1.0, sp = 0.0; // colored: the weights of the geometric and the photometric row
 
     Impl(const cwipc_point *target, size_t nt, float hint_spacing, const float *bounds, int k, int nsums, int dev, cudaStream_t s) : target(target), nt(nt), dev(dev), s(s) {
         float box[6];
@@ -2134,6 +2262,19 @@ IcpMatcher::IcpMatcher(const cwipc_point *target, size_t nt, float hint_spacing,
     });
 }
 
+IcpMatcher::IcpMatcher(const cwipc_point *target, size_t nt, float hint_spacing, const float *bounds, int dev, cudaStream_t s, double normal_radius, int normal_max_nn,
+                       double gradient_radius, int gradient_max_nn, double lambda_geometric)
+    : IcpMatcher(target, nt, hint_spacing, bounds, dev, s, normal_radius, normal_max_nn) {
+    m->gradients = Scratch(nt * sizeof(float4), s);
+    m->sg = std::sqrt(lambda_geometric);
+    m->sp = std::sqrt(1.0 - lambda_geometric);
+    const float limit = (float)(gradient_radius * gradient_radius);
+    launch("icp_gradients_kernel", s, 16 * nt, [&] {
+        icp_gradients_kernel<<<m->grid(nt), ICP_THREADS, 0, s>>>(target, (uint32_t)nt, m->ix.spts.as<cwipc_point>(), m->ix.sorted, m->ix.gp, m->ix.table.as<uint2>(), FAR_LEAF_POINTS,
+                                                              limit, m->slack, gradient_max_nn, m->normals.as<float4>(), m->gradients.as<float4>());
+    });
+}
+
 IcpMatcher::~IcpMatcher() = default;
 
 const double *IcpMatcher::origin() const { return m->origin; }
@@ -2158,10 +2299,18 @@ void IcpMatcher::evaluate(const cwipc_point *source, size_t ns, const double mot
         });
         launch("icp_reduce_kernel", m->s, 8 * (size_t)nwarps * ICP_NSUMS, [&] { icp_reduce_kernel<<<1, ICP_NSUMS * 32, 0, m->s>>>(partial, nwarps, d_out); });
     } else {
-        launch("icp_plane_match_kernel", m->s, 16 * ns, [&] {
-            icp_plane_match_kernel<<<grid, ICP_THREADS, 0, m->s>>>(source, (uint32_t)ns, m->target, (uint32_t)m->nt, m->ix.spts.as<cwipc_point>(), m->ix.sorted, m->ix.gp,
-                                                                  m->ix.table.as<uint2>(), FAR_LEAF_POINTS, ip, m->normals.as<float4>(), partial);
-        });
+        if (!m->gradients.p) {
+            launch("icp_plane_match_kernel", m->s, 16 * ns, [&] {
+                icp_plane_match_kernel<<<grid, ICP_THREADS, 0, m->s>>>(source, (uint32_t)ns, m->target, (uint32_t)m->nt, m->ix.spts.as<cwipc_point>(), m->ix.sorted, m->ix.gp,
+                                                                      m->ix.table.as<uint2>(), FAR_LEAF_POINTS, ip, m->normals.as<float4>(), partial);
+            });
+        } else {
+            launch("icp_colored_match_kernel", m->s, 16 * ns, [&] {
+                icp_colored_match_kernel<<<grid, ICP_THREADS, 0, m->s>>>(source, (uint32_t)ns, m->target, (uint32_t)m->nt, m->ix.spts.as<cwipc_point>(), m->ix.sorted, m->ix.gp,
+                                                                        m->ix.table.as<uint2>(), FAR_LEAF_POINTS, ip, m->normals.as<float4>(), m->gradients.as<float4>(), m->sg,
+                                                                        m->sp, partial);
+            });
+        }
         launch("icp_plane_reduce_kernel", m->s, 8 * (size_t)nwarps * ICP_PLANE_NSUMS,
                [&] { icp_plane_reduce_kernel<<<1, ICP_PLANE_NSUMS * 32, 0, m->s>>>(partial, nwarps, d_out); });
     }
@@ -2171,16 +2320,23 @@ void IcpMatcher::evaluate(const cwipc_point *source, size_t ns, const double mot
     memcpy(sums, h, nsum * sizeof(double));
 }
 
-bool IcpMatcher::normals_to_host(float *out) {
-    float4 *h = static_cast<float4 *>(thread_pinned(m->nt * sizeof(float4)));
-    CWCU_CHECK(cudaMemcpyAsync(h, m->normals.p, m->nt * sizeof(float4), cudaMemcpyDeviceToHost, m->s));
-    stream_sync(m->s);
+namespace {
+// xyz of n float4 (w: 0, or 1 for a point with a non-finite coordinate) to out[3 n]; false when a w is not 0
+bool float4_xyz_to_host(const void *d, size_t n, float *out, cudaStream_t s) {
+    float4 *h = static_cast<float4 *>(thread_pinned(n * sizeof(float4)));
+    CWCU_CHECK(cudaMemcpyAsync(h, d, n * sizeof(float4), cudaMemcpyDeviceToHost, s));
+    stream_sync(s);
     bool finite = true;
-    for (size_t i = 0; i < m->nt; i++) {
+    for (size_t i = 0; i < n; i++) {
         out[3 * i] = h[i].x, out[3 * i + 1] = h[i].y, out[3 * i + 2] = h[i].z;
         finite = finite && h[i].w == 0.f;
     }
     return finite;
 }
+} // namespace
+
+bool IcpMatcher::normals_to_host(float *out) { return float4_xyz_to_host(m->normals.p, m->nt, out, m->s); }
+
+bool IcpMatcher::gradients_to_host(float *out) { return float4_xyz_to_host(m->gradients.p, m->nt, out, m->s); }
 
 } // namespace cwcu

@@ -28,6 +28,7 @@ __all__ = [
     "cwipc_downsample", "cwipc_remove_outliers", "cwipc_tilefilter", "cwipc_tilemap", "cwipc_colormap", "cwipc_crop",
     "cwipc_join", "cwipc_join_multi", "cwipc_tilefilter_masked", "cwipc_downsample_pertile", "cwipc_transform",
     "cwipc_icp", "cwipc_icp_result", "cwipc_icp_point_to_plane", "cwipc_estimate_normals",
+    "cwipc_icp_colored", "cwipc_estimate_color_gradients",
     "cuda_device_count", "cuda_set_device", "cuda_synchronize", "cuda_kernel_launches",
 ]
 
@@ -158,6 +159,10 @@ def cwipc_util_dll_load(libname: Optional[str] = None) -> ctypes.CDLL:
         "cwipc_cuda_icp_point_to_plane": ([cwipc_pointcloud_p, cwipc_pointcloud_p, ctypes.c_void_p, ctypes.c_double, ctypes.c_int, ctypes.c_double, ctypes.c_double,
                                            ctypes.c_double, ctypes.c_int, ctypes.POINTER(cwipc_cuda_icp_result)], ctypes.c_int),
         "cwipc_cuda_estimate_normals": ([cwipc_pointcloud_p, ctypes.c_double, ctypes.c_int, ctypes.c_void_p, ctypes.c_size_t], ctypes.c_int),
+        "cwipc_cuda_icp_colored": ([cwipc_pointcloud_p, cwipc_pointcloud_p, ctypes.c_void_p, ctypes.c_double, ctypes.c_int, ctypes.c_double, ctypes.c_double,
+                                    ctypes.c_double, ctypes.c_int, ctypes.c_double, ctypes.POINTER(cwipc_cuda_icp_result)], ctypes.c_int),
+        "cwipc_cuda_estimate_color_gradients": ([cwipc_pointcloud_p, ctypes.c_double, ctypes.c_int, ctypes.c_double, ctypes.c_int, ctypes.c_void_p, ctypes.c_size_t],
+                                                ctypes.c_int),
         "cwipc_tilemap": ([cwipc_pointcloud_p, ctypes.c_char_p], cwipc_pointcloud_p),
         "cwipc_colormap": ([cwipc_pointcloud_p, ctypes.c_uint32, ctypes.c_uint32], cwipc_pointcloud_p),
         "cwipc_crop": ([cwipc_pointcloud_p, ctypes.POINTER(ctypes.c_float)], cwipc_pointcloud_p),
@@ -559,6 +564,44 @@ def cwipc_estimate_normals(pc: cwipc_pointcloud_wrapper, radius: float, max_nn: 
     rv = cwipc_util_dll_load().cwipc_cuda_estimate_normals(pc.as_cwipc_p(), float(radius), int(max_nn), out.ctypes.data, out.size)
     if rv < 0:
         raise CwipcError("cwipc_cuda_estimate_normals failed (the ERROR log says why)")
+    return out
+
+
+def cwipc_icp_colored(source: cwipc_pointcloud_wrapper, target: cwipc_pointcloud_wrapper, max_correspondence_distance: float, normal_radius: float,
+                      init: Any = None, max_iterations: int = 30, relative_fitness: float = 1e-6, relative_rmse: float = 1e-6,
+                      normal_max_nn: int = 30, lambda_geometric: float = 0.968) -> cwipc_icp_result:
+    """Colored ICP of `source` against `target` on the device (cwipc_cuda_icp_colored in include/cwipc_util_cuda.h):
+    open3d's estimate_normals(target, KDTreeSearchParamHybrid(normal_radius, normal_max_nn)) followed by
+    registration_colored_icp(source, target, max_correspondence_distance, init,
+    TransformationEstimationForColoredICP(lambda_geometric), ICPConvergenceCriteria(relative_fitness, relative_rmse,
+    max_iterations)).  The evaluation is cwipc_icp's; lambda_geometric = 1 is cwipc_icp_point_to_plane bit for bit.  init: a
+    (4, 4) array-like, None for the identity; another shape raises ValueError before the library is called.  A failure of
+    the library raises CwipcError."""
+    m = None
+    if init is not None:
+        m = numpy.ascontiguousarray(init, dtype=numpy.float64)
+        if m.shape != (4, 4):
+            raise ValueError(f"cwipc_icp_colored: init must have shape (4, 4), not {m.shape}")
+    res = cwipc_cuda_icp_result()
+    rv = cwipc_util_dll_load().cwipc_cuda_icp_colored(source.as_cwipc_p(), target.as_cwipc_p(), None if m is None else m.ctypes.data,
+                                                      float(max_correspondence_distance), int(max_iterations), float(relative_fitness), float(relative_rmse),
+                                                      float(normal_radius), int(normal_max_nn), float(lambda_geometric), ctypes.byref(res))
+    if rv != 0:
+        raise CwipcError("cwipc_cuda_icp_colored failed (the ERROR log says why)")
+    return cwipc_icp_result(numpy.array(res.matrix, numpy.float64).reshape(4, 4), res.fitness, res.inlier_rmse, res.iterations, res.correspondences)
+
+
+def cwipc_estimate_color_gradients(pc: cwipc_pointcloud_wrapper, normal_radius: float, radius: float, normal_max_nn: int = 30, max_nn: int = 30) -> numpy.ndarray:
+    """The colour gradient of every point of `pc` as an (n, 3) float32 array in the cloud's order
+    (cwipc_cuda_estimate_color_gradients in include/cwipc_util_cuda.h; open3d's InitializePointCloudForColoredICP with
+    KDTreeSearchParamHybrid(radius, max_nn), after estimate_normals with KDTreeSearchParamHybrid(normal_radius,
+    normal_max_nn)).  Intensity is (r + g + b) / 765; a point with fewer than 4 neighbours or a zero normal gets (0, 0, 0).
+    A failure of the library (an invalid argument, non-finite coordinates) raises CwipcError."""
+    out = numpy.zeros((max(pc.count(), 0), 3), numpy.float32)
+    rv = cwipc_util_dll_load().cwipc_cuda_estimate_color_gradients(pc.as_cwipc_p(), float(normal_radius), int(normal_max_nn), float(radius), int(max_nn),
+                                                                   out.ctypes.data, out.size)
+    if rv < 0:
+        raise CwipcError("cwipc_cuda_estimate_color_gradients failed (the ERROR log says why)")
     return out
 
 

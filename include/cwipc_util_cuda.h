@@ -408,6 +408,53 @@ _CWIPC_UTIL_EXPORT int cwipc_cuda_estimate_normals(cwipc_pointcloud *pc, double 
 _CWIPC_UTIL_EXPORT int cwipc_cuda_icp_point_to_plane(cwipc_pointcloud *source, cwipc_pointcloud *target, const double init[16], double max_correspondence_distance,
                                                      int max_iterations, double relative_fitness, double relative_rmse, double normal_radius, int normal_max_nn,
                                                      struct cwipc_cuda_icp_result *result);
+/* Colour gradient of every point (open3d's InitializePointCloudForColoredICP), copied to gradients[3 * count], in the
+ * cloud's order.  Returns count or -1.
+ *   Intensity of a point: I = ((double)r + g + b) / 765, an exact integer sum and one division (open3d takes the mean of
+ *   its [0, 1] colours, which differs only in rounding).  The tile byte is not a colour.
+ *   Normal n of point i: exactly cwipc_cuda_estimate_normals(pc, normal_radius, normal_max_nn), from the same kernel.
+ *   Neighbourhood of point i: the max_nn smallest keys (d2, index) within radius, i itself included, by
+ *   cwipc_cuda_estimate_normals' rule; nn is its size.  Every neighbour j gives the row A_j = d_j - (d_j . n) n with
+ *   d_j = v_j - v_i (open3d's (v_j - (d_j . n) n) - v_i, taken relative to v_i) and b_j = I_j - I_i; one more row
+ *   A = (nn - 1) n, b = 0, keeps g in the tangent plane.  open3d skips the first neighbour instead of i; a neighbour that
+ *   coincides with i gives a zero row either way, so the sums are the same.  g is the minimum-norm solution of
+ *   (A^T A) g = A^T b, from a symmetric eigen-decomposition in double that drops the eigenvalues <= 1e-12 times the largest
+ *   (the rule of cwipc_cuda_icp_point_to_plane's step; open3d uses LDLT), rounded to float.  g = (0, 0, 0) when nn < 4 or
+ *   n = (0, 0, 0).  Results are bit-identical from run to run.  4 <= max_nn <= 32 (one warp holds the list).
+ *   Errors: normal_radius or radius not finite or not > 0, normal_max_nn outside [3, 32], max_nn outside [4, 32],
+ *   gradients == NULL, nfloats < 3 * count, or non-finite coordinates give -1 and one ERROR log naming
+ *   cwipc_cuda_estimate_color_gradients; the cloud stays usable.  NULL pc: -1, silently, before any argument check.  An
+ *   empty cloud returns 0.
+ *   Cost: one search index (pitched for normal_max_nn neighbours), one normal kernel and one gradient kernel over the
+ *   cloud, one copy to the host. */
+_CWIPC_UTIL_EXPORT int cwipc_cuda_estimate_color_gradients(cwipc_pointcloud *pc, double normal_radius, int normal_max_nn, double radius, int max_nn, float *gradients,
+                                                           size_t nfloats);
+/* Colored ICP of `source` against `target` (open3d registration_colored_icp with
+ * TransformationEstimationForColoredICP(lambda_geometric); Park, Zhou and Koltun, ICCV 2017): point-to-plane ICP plus a
+ * photometric term that pins the motions the geometry cannot see (a surface of revolution turning about its axis, a wall
+ * sliding along itself).  The target's normals are cwipc_cuda_estimate_normals(target, normal_radius, normal_max_nn) and its
+ * gradients cwipc_cuda_estimate_color_gradients(target, normal_radius, normal_max_nn, 2 * max_correspondence_distance, 30),
+ * the radius and count open3d's RegistrationColoredICP takes.
+ *   Evaluation is exactly cwipc_cuda_icp's: the same correspondences, tie rule, fitness and inlier_rmse.  So with
+ *   max_iterations = 0 both calls return the same correspondences, fitness and inlier_rmse, bit for bit.
+ *   Update: sg = sqrt(lambda_geometric), sp = sqrt(1 - lambda_geometric).  For every correspondence (p', q) with target
+ *   normal n, target gradient g and intensities I_s (of the source point) and I_t (of q), all in double and relative to
+ *   the centre of the target's box: the geometric row J_G = sg [p' x n, n], r_G = sg (p' - q) . n, and the photometric row
+ *   with p_proj = p' - ((p' - q) . n) n, I_0 = g . (p_proj - q) + I_t and d = -(g - (g . n) n): J_I = sp [p' x d, d],
+ *   r_I = sp (I_s - I_0).  x is the minimum-norm least-squares solution of
+ *   (sum J_G J_G^T + J_I J_I^T) x = -sum (J_G r_G + J_I r_I); the solve, dT, the loop, the stopping rule and the result are
+ *   cwipc_cuda_icp_point_to_plane's.  lambda_geometric = 1 skips the photometric row and returns
+ *   cwipc_cuda_icp_point_to_plane's result bit for bit (matrix, fitness, rmse, iterations, correspondences).
+ *   lambda_geometric = 0 is the photometric term alone.
+ *   Errors: those of cwipc_cuda_icp_point_to_plane, and lambda_geometric not finite or outside [0, 1]: -1 and one ERROR log
+ *   naming cwipc_cuda_icp_colored; the inputs stay usable.  NULL source or target: -1, silently, before any argument
+ *   check.  An empty source or target follows cwipc_cuda_icp's rules.
+ *   Cost: one search index (pitched for normal_max_nn neighbours), one normal kernel and one gradient kernel over the
+ *   target per call, then per iteration one search kernel, one reduction kernel and one read-back of 30 numbers.  Results
+ *   are bit-identical from run to run and under concurrent callers. */
+_CWIPC_UTIL_EXPORT int cwipc_cuda_icp_colored(cwipc_pointcloud *source, cwipc_pointcloud *target, const double init[16], double max_correspondence_distance,
+                                              int max_iterations, double relative_fitness, double relative_rmse, double normal_radius, int normal_max_nn,
+                                              double lambda_geometric, struct cwipc_cuda_icp_result *result);
 /* Per-point mean k-neighbour distance of cwipc_remove_outliers' first pass, copied to host
  * (dist[count]); returns count or -1.  Diagnostic hook used by the parity tests. */
 _CWIPC_UTIL_EXPORT int cwipc_cuda_knn_mean_distances(cwipc_pointcloud *pc, int kNeighbors, float *dist, size_t ndist);
